@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA engine)
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU arm (compiled port of the oracle)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + outputs of the last timed step, as DIR/*.npy
 
 Workload (config.workload): BASELINE.json config 3 -- batched bound + equality constrained
 Gaussian-peak curve fits, n=6, m=128, 1 equality + 12 bounds, forward-difference Jacobians,
@@ -40,6 +41,33 @@ def fp64_fma_peak():
     if os.path.exists(p):
         return float(json.load(open(p))["fp64_dfma_tflops"])
     return 40.0
+
+
+def sample_rows(B, k, seed=0):
+    """--dump-outputs: a fixed, seeded sample of k of the B problems of a batch (all of them when B <= k), sorted."""
+    if B <= k:
+        return np.arange(B)
+    return np.sort(np.random.default_rng(seed).choice(B, k, replace=False))
+
+
+def write_outputs(dirname, prefix, arrays, rows=None):
+    """--dump-outputs: the arrays a caller of a timed path receives after its last step, as DIR/<prefix><name>.npy in
+    float64 (the integer outputs are exact in it), so that two builds can be compared output for output.  `rows` keeps
+    those problems of a batched output and is written as <prefix>index.npy."""
+    os.makedirs(dirname, exist_ok=True)
+    if rows is not None:
+        np.save(os.path.join(dirname, prefix + "index.npy"), rows.astype(np.float64))
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        if rows is not None:
+            a = a[rows]
+        np.save(os.path.join(dirname, prefix + name + ".npy"), a.astype(np.float64))
+
+
+def large_outputs(mod):
+    """What solve() hands the caller of one large-regime problem."""
+    return {"x": mod.sol[0], "f": mod.obj_value, "exit_code": mod.exit_code, "status": mod.status_code,
+            "iters": mod.iterations, "nact": mod.nb_active, "active": mod.active[0]}
 
 
 def dist_env():
@@ -276,6 +304,8 @@ def c2_arm(args, torch, dist, E, rank, world, local, dev):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item()) / steps
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, "hs65_", out, sample_rows(B, 1 << 16))
     st = out["status"].cpu().numpy()
     ec = out["exit_code"].cpu().numpy()
     res = {"metric": "batched CNLS solves/s (HS65: n=3, m=3)", "value": world * B / (ms * 1e-3), "unit": "solves/s", "n_gpus": world,
@@ -309,6 +339,8 @@ def c5_arm(args, torch, E, dev, local):
         its += int(mod.iterations[0])
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, "large5_", large_outputs(mod))
     st1 = mod.stats()
     dst = {k: st1[k] - st0[k] for k in st1 if k != "rows_pad"}
     nfac = max(dst["factorisations"], 1.0)
@@ -427,6 +459,8 @@ def large_arm(args, torch, dist, E, rank, world, local, dev):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dt = float(t.item())
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, "large_", large_outputs(mod))
     st1 = mod.stats()
     dst = {k: st1[k] - st0[k] for k in st1 if k != "rows_pad"}
     nfac = max(dst["factorisations"], 1.0)
@@ -577,8 +611,15 @@ def main():
     ap.add_argument("--c2-problems", type=int, default=1_000_000, help="HS65 instances per GPU (config 2)")
     ap.add_argument("--c5-steps", type=int, default=2)
     ap.add_argument("--c5-ref-full", action="store_true", help="--impl reference: time the C5 pass at the named size (minutes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of each arm's last timed step as DIR/<name>.npy (float64; batched outputs as a "
+                         "fixed, seeded sample of problems, with their indices in index.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the CUDA engine (--impl ours)")
         reference_arm(args)
         return
 
@@ -648,6 +689,9 @@ def main():
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     elapsed_ms = float(t.item())
+    # rank 0's shard; 2^19 of the 4M problems keep the outputs of every arm under 64 MB
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, "", out, sample_rows(B, 1 << 19))
     ms_per_step = elapsed_ms / args.steps
     value = world * B / (ms_per_step * 1e-3)
 

@@ -18,10 +18,18 @@ os.environ.setdefault("OPENBLAS_NUM_THREADS", "1")
 os.environ.setdefault("OMP_NUM_THREADS", "1")
 import enlsip_jl_b200 as E                                   # noqa: E402
 from oracle import enlsip_oracle as O, problems as P         # noqa: E402
-from make_golden import pack                                 # noqa: E402
+from make_golden import pack as pack_all                     # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 B, START = 10_000, 100_000
+
+
+def pack(results, n, lmax):
+    """make_golden.pack without x_pen: the 10^4-problem histograms never read it, and it would take each C3 fixture over
+    1 MB."""
+    d = pack_all(results, n, lmax)
+    del d["x_pen"]
+    return d
 
 
 def solve_hs65(x0):
