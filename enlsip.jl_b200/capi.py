@@ -39,7 +39,8 @@ EXPORTS = ["enlsipb200_version", "enlsipb200_last_error", "enlsipb200_default_op
            "enlsipb200_large_last_error", "enlsipb200_large_create", "enlsipb200_large_destroy",
            "enlsipb200_large_set_data", "enlsipb200_large_comm_id", "enlsipb200_large_comm_init",
            "enlsipb200_large_solve", "enlsipb200_large_factor", "enlsipb200_large_stats",
-           "enlsipb200_dense_qrcp", "enlsipb200_dense_mulq", "enlsipb200_dense_vecop", "enlsipb200_dense_last_ms"]
+           "enlsipb200_dense_qrcp", "enlsipb200_dense_qr", "enlsipb200_dense_mulq", "enlsipb200_dense_vecop",
+           "enlsipb200_dense_gemv", "enlsipb200_dense_last_ms"]
 
 
 class Options(ctypes.Structure):
@@ -114,8 +115,10 @@ def _bind(L, large=True):
         L.enlsipb200_large_factor.argtypes = [vp, vp, vp, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float)]
         L.enlsipb200_large_stats.argtypes = [vp, vp, ci]
         L.enlsipb200_dense_qrcp.argtypes = [ci, ci, vp, vp, vp, ci]
+        L.enlsipb200_dense_qr.argtypes = [ci, ci, vp, vp, ci]
         L.enlsipb200_dense_mulq.argtypes = [ci, ci, ci, vp, vp, vp, ci]
         L.enlsipb200_dense_vecop.argtypes = [ci, ci, ci, vp, vp, vp, ci]
+        L.enlsipb200_dense_gemv.argtypes = [ci, ci, ci, vp, ci, vp, ctypes.c_double, vp, ctypes.c_double, vp, ci]
         L.enlsipb200_dense_last_ms.restype = ctypes.c_float
     return L
 

@@ -770,37 +770,14 @@ struct LargeHandle : LargeOps, SmallBackend {
         return T;
     }
     void k_reflect(const double* f, int frows, int k, const double* tau, double* v, int transpose) {
-        if (frows <= 0 || k <= 0) return;
-        if (frows <= enl_small::VEC_WARP_MAX) {
-            enl_small::reflect_vec_warp_kernel<<<1, 32, sizeof(double) * (size_t)frows, st>>>(f, frows, k, tau, v, transpose);
-            ++launches;
-            return;
-        }
-        // long vectors: the compact-WY panels in one cooperative kernel (one grid barrier per 32 reflectors)
-        if (double* T = wy_t_of(f, frows, k, tau)) {
-            const int rc = enl_small::reflect_vec_wy(f, frows, k, T, v, transpose, dwpart, qw.ticket + 1, st);
-            if (rc > 0) { launches += rc; return; }
-        }
-        enl_small::reflect_vec_kernel<<<1, 1024, sizeof(double) * (size_t)frows, st>>>(f, frows, k, tau, v, transpose);
-        ++launches;
-    }
-    static int coop_min() {          // smallest triangle solved by the multi-CTA kernels (ENLSIP_TRSV_COOP_MIN overrides)
-        static const int v = [] { const char* e = getenv("ENLSIP_TRSV_COOP_MIN"); return e ? atoi(e) : 320; }();
-        return v;
+        launches += enl_small::reflect_vec(f, frows, k, tau, v, transpose, [&] { return wy_t_of(f, frows, k, tau); }, dwpart,
+                                           qw.ticket + 1, st);
     }
     void k_trsv_upper(const double* f, int ldf, int k, double* x) {
-        if (k <= 0) return;
-        if (k >= coop_min() && enl_small::trsv_coop(f, ldf, k, x, false, qw.ticket + 1, st) > 0) { ++launches; return; }
-        if (k <= enl_small::VEC_WARP_MAX) enl_small::trsv_upper_warp_kernel<<<1, 32, sizeof(double) * (size_t)k, st>>>(f, ldf, k, x);
-        else enl_small::trsv_upper_kernel<<<1, 1024, sizeof(double) * (size_t)k, st>>>(f, ldf, k, x);
-        ++launches;
+        launches += enl_small::trsv_upper(f, ldf, k, x, false, qw.ticket + 1, st);
     }
     void k_trsv_upperT(const double* f, int ldf, int k, double* x) {
-        if (k <= 0) return;
-        if (k >= coop_min() && enl_small::trsv_coop(f, ldf, k, x, true, qw.ticket + 1, st) > 0) { ++launches; return; }
-        if (k <= enl_small::VEC_WARP_MAX) enl_small::trsv_upperT_warp_kernel<<<1, 32, sizeof(double) * (size_t)k, st>>>(f, ldf, k, x);
-        else enl_small::trsv_upperT_kernel<<<1, 1024, sizeof(double) * (size_t)k, st>>>(f, ldf, k, x);
-        ++launches;
+        launches += enl_small::trsv_upper(f, ldf, k, x, true, qw.ticket + 1, st);
     }
     void k_copy_pad(double* dst, const double* src, int k, int len) {
         if (len <= 0) return;
@@ -1194,6 +1171,8 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
         nb = 0; ineq = 0; rho = nullptr;
     } else if (n < TS_B || n % TS_B != 0) {
         return lfail(ENLSIPB200_EINVAL, "n must be a positive multiple of 32");
+    } else if (n > enl_small::VEC_STAGE_MAX) {
+        return lfail(ENLSIPB200_EINVAL, "single-index family: n <= 6144 (x is staged in 48 KB of shared memory)");
     }
     if (m_local < 0 || m_global < m_local || nb < 0 || 4 * nb > n) return lfail(ENLSIPB200_EINVAL, "bad sizes");
     if ((long long)n + m_global < 1000)
@@ -1381,9 +1360,10 @@ int enlsipb200_large_stats(enlsipb200_large hh, double* out, int count) {
     return 0;
 }
 
-// ---- known-answer hooks of enl_small.cuh (tests/test_gpu_kat.py) ----
-int enlsipb200_dense_qrcp(int rows, int cols, double* f, double* tau, int* jpvt, int device) {
-    if (rows < 1 || cols < 1 || !f || !tau || !jpvt) return lfail(ENLSIPB200_EINVAL, "bad arguments");
+// ---- known-answer hooks of enl_small.cuh (tests/test_gpu_kat.py, tests/test_gpu_dense_dispatch.py) ----
+// qrcp_device on a copy of f: dgeqp3 (nopivot = 0, jpvt returned) or dgeqrf (nopivot = 1, jpvt may be NULL)
+static int dense_qr_run(int rows, int cols, double* f, double* tau, int* jpvt, int device, int nopivot) {
+    if (rows < 1 || cols < 1 || !f || !tau || (!jpvt && !nopivot)) return lfail(ENLSIPB200_EINVAL, "bad arguments");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return lfail(ENLSIPB200_ENOGPU, "no CUDA device");
     if (device < 0) LCU(cudaGetDevice(&device));
@@ -1406,7 +1386,7 @@ int enlsipb200_dense_qrcp(int rows, int cols, double* f, double* tau, int* jpvt,
     LCU(cudaStreamCreate(&hs));
     LCU(cudaEventCreate(&ev0)); LCU(cudaEventCreate(&ev1));
     LCU(cudaEventRecord(ev0, hs));
-    enl_small::qrcp_device(df, rows, cols, dtau, dp, S.qw, hs);
+    enl_small::qrcp_device(df, rows, cols, dtau, dp, S.qw, hs, nopivot);
     LCU(cudaEventRecord(ev1, hs));
     cudaError_t es = cudaStreamSynchronize(hs);
     if (es == cudaSuccess) es = cudaGetLastError();
@@ -1416,8 +1396,16 @@ int enlsipb200_dense_qrcp(int rows, int cols, double* f, double* tau, int* jpvt,
     LCU(es);
     LCU(cudaMemcpy(f, df, sizeof(double) * (size_t)rows * cols, cudaMemcpyDeviceToHost));
     LCU(cudaMemcpy(tau, dtau, sizeof(double) * k, cudaMemcpyDeviceToHost));
-    LCU(cudaMemcpy(jpvt, dp, sizeof(int) * cols, cudaMemcpyDeviceToHost));
+    if (jpvt) LCU(cudaMemcpy(jpvt, dp, sizeof(int) * cols, cudaMemcpyDeviceToHost));
     return 0;
+}
+
+int enlsipb200_dense_qrcp(int rows, int cols, double* f, double* tau, int* jpvt, int device) {
+    return dense_qr_run(rows, cols, f, tau, jpvt, device, 0);
+}
+
+int enlsipb200_dense_qr(int rows, int cols, double* f, double* tau, int device) {
+    return dense_qr_run(rows, cols, f, tau, nullptr, device, 1);
 }
 
 float enlsipb200_dense_last_ms(void) { return g_dense_ms; }
@@ -1454,9 +1442,13 @@ int enlsipb200_dense_mulq(int mr, int nq, int k, const double* f, const double* 
 
 // Known-answer hook for the vector kernels of the small stage (tests/test_gpu_kat.py).  kind 0: v <- Q' v, 1: v <- Q v
 // (f: frows x k reflectors in dgeqrf layout, tau [k], v [frows]; compact-WY cooperative kernel);
-// kind 2: v <- UpperTriangular(f[0:k, 0:k]) \ v, 3: v <- UpperTriangular(f[0:k, 0:k])' \ v (f: frows x k, v [k]).
+// kind 2: v <- UpperTriangular(f[0:k, 0:k]) \ v, 3: v <- UpperTriangular(f[0:k, 0:k])' \ v (f: frows x k, v [k];
+// multi-CTA cooperative kernels).  Kinds 4-7: the operations of kinds 0-3 with the kernel chosen by size as the solver
+// chooses it (enl_small::reflect_vec / trsv_upper).
 int enlsipb200_dense_vecop(int kind, int frows, int k, const double* f, const double* tau, double* v, int device) {
-    if (kind < 0 || kind > 3 || frows < 1 || k < 1 || k > frows || !f || !v || (kind < 2 && !tau)) return lfail(ENLSIPB200_EINVAL, "bad arguments");
+    if (kind < 0 || kind > 7 || frows < 1 || k < 1 || k > frows || !f || !v || ((kind & 3) < 2 && !tau)) return lfail(ENLSIPB200_EINVAL, "bad arguments");
+    const bool dispatched = kind >= 4;
+    kind &= 3;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return lfail(ENLSIPB200_ENOGPU, "no CUDA device");
     if (device < 0) LCU(cudaGetDevice(&device));
@@ -1476,7 +1468,17 @@ int enlsipb200_dense_vecop(int kind, int frows, int k, const double* f, const do
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     LCU(cudaEventCreate(&ev0)); LCU(cudaEventCreate(&ev1));
     int rc = 0;
-    if (kind < 2) {
+    if (dispatched) {
+        LCU(cudaEventRecord(ev0, nullptr));
+        if (kind < 2) {
+            auto t_of = [&]() -> const double* {
+                return enl_small::wy_build_t_all(df, frows, k, dtau, dTall, dscr, scr, nullptr) >= 0 ? dTall : nullptr;
+            };
+            rc = enl_small::reflect_vec(df, frows, k, dtau, dv, kind == 0 ? 1 : 0, t_of, dwp, dbar, nullptr);
+        } else {
+            rc = enl_small::trsv_upper(df, frows, k, dv, kind == 3, dbar, nullptr);
+        }
+    } else if (kind < 2) {
         rc = enl_small::wy_build_t_all(df, frows, k, dtau, dTall, dscr, scr, nullptr);
         LCU(cudaEventRecord(ev0, nullptr));
         if (rc >= 0) rc = enl_small::reflect_vec_wy(df, frows, k, dTall, dv, kind == 0 ? 1 : 0, dwp, dbar, nullptr);
@@ -1492,6 +1494,40 @@ int enlsipb200_dense_vecop(int kind, int frows, int k, const double* f, const do
     LCU(es);
     if (rc < 0) return lfail(ENLSIPB200_EINVAL, "shape not supported by the cooperative kernel");
     LCU(cudaMemcpy(v, dv, sizeof(double) * vlen, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+// Known-answer hook for the small stage's gemv (enl_small::gemv_n / gemv_t).  A: rows x cols, column major, lda >= rows.
+// trans 0: y [rows] = alpha A x + beta y0 (x [cols]; y0 [rows] or NULL = 0); trans 1: y [cols] = A' x (x [rows]; alpha,
+// y0 and beta unused: gemv_t forms the plain product).
+int enlsipb200_dense_gemv(int trans, int rows, int cols, const double* A, int lda, const double* x, double alpha,
+                          const double* y0, double beta, double* y, int device) {
+    if ((trans != 0 && trans != 1) || rows < 1 || cols < 1 || lda < rows || !A || !x || !y) return lfail(ENLSIPB200_EINVAL, "bad arguments");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return lfail(ENLSIPB200_ENOGPU, "no CUDA device");
+    if (device < 0) LCU(cudaGetDevice(&device));
+    LCU(cudaSetDevice(device));
+    DenseScratch S;
+    const int xlen = trans ? rows : cols, ylen = trans ? cols : rows;
+    const bool with_y0 = !trans && y0;
+    double *dA = nullptr, *dx = nullptr, *dy0 = nullptr, *dy = nullptr;
+    bool ok = S.get(&dA, (size_t)lda * cols) && S.get(&dx, xlen) && S.get(&dy, ylen) && (!with_y0 || S.get(&dy0, ylen));
+    if (!ok) return lfail(ENLSIPB200_ENOMEM, "cudaMalloc");
+    LCU(cudaMemcpy(dA, A, sizeof(double) * (size_t)lda * cols, cudaMemcpyHostToDevice));
+    LCU(cudaMemcpy(dx, x, sizeof(double) * xlen, cudaMemcpyHostToDevice));
+    if (with_y0) LCU(cudaMemcpy(dy0, y0, sizeof(double) * ylen, cudaMemcpyHostToDevice));
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    LCU(cudaEventCreate(&ev0)); LCU(cudaEventCreate(&ev1));
+    LCU(cudaEventRecord(ev0, nullptr));
+    if (trans) enl_small::gemv_t(dA, lda, rows, cols, dx, dy, nullptr);
+    else enl_small::gemv_n(dA, lda, rows, cols, dx, alpha, dy0, beta, dy, nullptr);
+    LCU(cudaEventRecord(ev1, nullptr));
+    cudaError_t es = cudaDeviceSynchronize();
+    if (es == cudaSuccess) es = cudaGetLastError();
+    cudaEventElapsedTime(&g_dense_ms, ev0, ev1);
+    cudaEventDestroy(ev0); cudaEventDestroy(ev1);
+    LCU(es);
+    LCU(cudaMemcpy(y, dy, sizeof(double) * ylen, cudaMemcpyDeviceToHost));
     return 0;
 }
 

@@ -1006,14 +1006,21 @@ __global__ void __launch_bounds__(1024) qr_p2_pivot_house_kernel(double* __restr
     if (tid == 0) tau[i] = tau_i;
 }
 
-// apply H_i to the trailing columns (one warp per column) + dlaqp2 partial-norm downdate of that column
+// apply H_i to the trailing columns (one warp per column) + dlaqp2 partial-norm downdate of that column.  STAGED: the
+// reflector is first copied to shared memory (len <= VEC_STAGE_MAX); otherwise it is read from column i of f, which this
+// launch does not write.  Both forms add in the same order, so they give the same bits.
+constexpr int VEC_STAGE_MAX = 6144;   // doubles in the 48 KB of dynamic shared memory a launch gets without an opt-in
+template <bool STAGED>
 __global__ void __launch_bounds__(256) qr_p2_apply_kernel(double* __restrict__ f, int rows, int cols, int i, double* vn1,
                                                           double* vn2, const double* __restrict__ tau) {
-    extern __shared__ double vs[];
+    extern __shared__ double vsm[];
     const int len = rows - i - 1;
     const double* v = f + (size_t)i * rows + i + 1;
-    for (int r = threadIdx.x; r < len; r += blockDim.x) vs[r] = v[r];
-    __syncthreads();
+    if (STAGED) {
+        for (int r = threadIdx.x; r < len; r += blockDim.x) vsm[r] = v[r];
+        __syncthreads();
+    }
+    const double* vs = STAGED ? vsm : v;
     const double tau_i = tau[i];
     const int lane = threadIdx.x & 31;
     const int gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
@@ -1412,7 +1419,10 @@ inline int qrcp_device(double* f, int rows, int cols, double* tau, int* jpvt, Qr
             int ncol = cols - i - 1;
             int grid = (ncol + 7) / 8;
             if (grid > 148 * 4) grid = 148 * 4;
-            qr_p2_apply_kernel<<<grid, 256, sizeof(double) * (size_t)(len > 0 ? len : 1), st>>>(f, rows, cols, i, wk.vn1, wk.vn2, tau);
+            if (len <= VEC_STAGE_MAX)
+                qr_p2_apply_kernel<true><<<grid, 256, sizeof(double) * (size_t)(len > 0 ? len : 1), st>>>(f, rows, cols, i, wk.vn1, wk.vn2, tau);
+            else
+                qr_p2_apply_kernel<false><<<grid, 256, 0, st>>>(f, rows, cols, i, wk.vn1, wk.vn2, tau);
             ++launches;
         }
     }
@@ -1967,13 +1977,57 @@ __global__ void __launch_bounds__(1024) trsv_upperT_kernel(const double* __restr
     for (int r = threadIdx.x; r < k; r += blockDim.x) x[r] = xs[r];
 }
 
-// y (rows) = alpha * A (rows x cols, lda) x + beta * y0   (y0 may be nullptr = 0); thread per row, columns streamed
+// ---- the size selection of the vector operations (the solver's small stage and the known-answer hook use these) ----
+// v (frows entries) <- Q' v (transpose = 1) / Q v: one warp up to VEC_WARP_MAX entries, else the compact-WY cooperative
+// kernel with the T factors t_of() returns (nullptr: none), else one CTA.  Returns the launches (t_of()'s not included).
+template <class TOf>
+inline int reflect_vec(const double* f, int frows, int k, const double* tau, double* v, int transpose, TOf&& t_of,
+                       double* wpart, unsigned int* bar, cudaStream_t st) {
+    if (frows <= 0 || k <= 0) return 0;
+    if (frows <= VEC_WARP_MAX) {
+        reflect_vec_warp_kernel<<<1, 32, sizeof(double) * (size_t)frows, st>>>(f, frows, k, tau, v, transpose);
+        return 1;
+    }
+    if (const double* T = t_of()) {
+        const int rc = reflect_vec_wy(f, frows, k, T, v, transpose, wpart, bar, st);
+        if (rc > 0) return rc;
+    }
+    reflect_vec_kernel<<<1, 1024, sizeof(double) * (size_t)frows, st>>>(f, frows, k, tau, v, transpose);
+    return 1;
+}
+inline int trsv_coop_min() {     // smallest triangle solved by the multi-CTA kernels (ENLSIP_TRSV_COOP_MIN overrides)
+    static const int v = [] { const char* e = getenv("ENLSIP_TRSV_COOP_MIN"); return e ? atoi(e) : 320; }();
+    return v;
+}
+// x (k entries) <- R \ x (transposed: R' \ x), R = UpperTriangular(f[0:k, 0:k]): the cooperative kernels from
+// trsv_coop_min() entries, else one warp up to VEC_WARP_MAX, else one CTA.  Returns the number of launches.
+inline int trsv_upper(const double* f, int ldf, int k, double* x, bool transposed, unsigned int* bar, cudaStream_t st) {
+    if (k <= 0) return 0;
+    if (k >= trsv_coop_min() && trsv_coop(f, ldf, k, x, transposed, bar, st) > 0) return 1;
+    const size_t shb = sizeof(double) * (size_t)k;
+    if (k <= VEC_WARP_MAX) {
+        if (transposed) trsv_upperT_warp_kernel<<<1, 32, shb, st>>>(f, ldf, k, x);
+        else trsv_upper_warp_kernel<<<1, 32, shb, st>>>(f, ldf, k, x);
+    } else if (transposed) {
+        trsv_upperT_kernel<<<1, 1024, shb, st>>>(f, ldf, k, x);
+    } else {
+        trsv_upper_kernel<<<1, 1024, shb, st>>>(f, ldf, k, x);
+    }
+    return 1;
+}
+
+// y (rows) = alpha * A (rows x cols, lda) x + beta * y0   (y0 may be nullptr = 0); thread per row, columns streamed.
+// STAGED: x is first copied to shared memory (cols <= VEC_STAGE_MAX), otherwise read from global memory; same sums.
+template <bool STAGED>
 __global__ void __launch_bounds__(256) gemv_n_kernel(const double* __restrict__ A, int lda, int rows, int cols,
                                                      const double* __restrict__ x, double alpha, const double* __restrict__ y0,
                                                      double beta, double* __restrict__ y) {
-    extern __shared__ double xs[];
-    for (int c = threadIdx.x; c < cols; c += blockDim.x) xs[c] = x[c];
-    __syncthreads();
+    extern __shared__ double xsm[];
+    if (STAGED) {
+        for (int c = threadIdx.x; c < cols; c += blockDim.x) xsm[c] = x[c];
+        __syncthreads();
+    }
+    const double* xs = STAGED ? xsm : x;
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= rows) return;
     double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
@@ -2031,7 +2085,9 @@ inline int gemv_n(const double* A, int lda, int rows, int cols, const double* x,
                   double* y, cudaStream_t st) {
     if (rows <= 0) return 0;
     if (rows <= 2048) gemv_n_split_kernel<<<(rows + 31) / 32, 256, 0, st>>>(A, lda, rows, cols, x, alpha, y0, beta, y);
-    else gemv_n_kernel<<<(rows + 255) / 256, 256, sizeof(double) * (size_t)(cols > 0 ? cols : 1), st>>>(A, lda, rows, cols, x, alpha, y0, beta, y);
+    else if (cols <= VEC_STAGE_MAX)
+        gemv_n_kernel<true><<<(rows + 255) / 256, 256, sizeof(double) * (size_t)(cols > 0 ? cols : 1), st>>>(A, lda, rows, cols, x, alpha, y0, beta, y);
+    else gemv_n_kernel<false><<<(rows + 255) / 256, 256, 0, st>>>(A, lda, rows, cols, x, alpha, y0, beta, y);
     return 1;
 }
 inline int gemv_t(const double* A, int lda, int rows, int cols, const double* x, double* y, cudaStream_t st) {

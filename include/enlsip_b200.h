@@ -215,12 +215,21 @@ ENLSIPB200_API int enlsipb200_large_stats(enlsipb200_large h, double* out, int c
  *   enlsipb200_dense_mulq : `J * F_A.Q` of src/enlsip_functions.jl:219: M [mr x nq] <- M * H(0) ... H(k-1), the
  *       reflectors in f [nq x k] / tau [k] (dgeqp3 layout). */
 ENLSIPB200_API int enlsipb200_dense_qrcp(int rows, int cols, double* f, double* tau, int* jpvt, int device);
+/*   enlsipb200_dense_qr : the plain Householder QR (LAPACK dgeqrf, no pivoting) that compresses [J | r] of the general
+ *       large-regime families; f / tau as enlsipb200_dense_qrcp. */
+ENLSIPB200_API int enlsipb200_dense_qr(int rows, int cols, double* f, double* tau, int device);
 ENLSIPB200_API int enlsipb200_dense_mulq(int mr, int nq, int k, const double* f, const double* tau, double* M, int device);
 /*   enlsipb200_dense_vecop : the vector products and triangular solves of src/enlsip_functions.jl:133-152, 484-500 as the
  *       engine runs them for long vectors (cooperative multi-CTA kernels).  kind 0: v [frows] <- Q' v, 1: v <- Q v with
  *       Q = H(0) ... H(k-1) from f [frows x k] / tau [k] (LAPACK dormqr); kind 2: v [k] <- R \ v, 3: v [k] <- R' \ v with
- *       R = the upper triangle of the leading k x k block of f [frows x k] (LAPACK dtrtrs). */
+ *       R = the upper triangle of the leading k x k block of f [frows x k] (LAPACK dtrtrs).  Kinds 4-7: the operations of
+ *       kinds 0-3 with the kernel the engine picks for that size (one warp, cooperative, or one CTA). */
 ENLSIPB200_API int enlsipb200_dense_vecop(int kind, int frows, int k, const double* f, const double* tau, double* v, int device);
+/*   enlsipb200_dense_gemv : the small stage's matrix-vector products.  A [rows x cols], leading dimension lda >= rows.
+ *       trans 0: y [rows] = alpha A x + beta y0 (x [cols]; y0 [rows], NULL = 0); trans 1: y [cols] = A' x (x [rows];
+ *       alpha, y0 and beta unused). */
+ENLSIPB200_API int enlsipb200_dense_gemv(int trans, int rows, int cols, const double* A, int lda, const double* x, double alpha,
+                                         const double* y0, double beta, double* y, int device);
 /* device time (CUDA events around the kernels, transfers excluded) of the last enlsipb200_dense_* call, in ms */
 ENLSIPB200_API float enlsipb200_dense_last_ms(void);
 

@@ -62,6 +62,9 @@ def test_large_api_validation(capi):
     assert b"batched engine" in L.enlsipb200_large_last_error()          # n + m < 1000: Newton regime (EF:2658)
     assert L.enlsipb200_large_create(99, 32, 1000, 1000, 4, 0, rho.ctypes.data, None, None, -1, ctypes.byref(h)) != 0
     assert L.enlsipb200_large_create(capi.FAMILY_SINGLE_INDEX, 32, 2000, 1000, 4, 0, rho.ctypes.data, None, None, -1, ctypes.byref(h)) != 0
+    # the single-index kernels stage x in 48 KB of shared memory: n > 6144 is refused as an argument error (-1, EINVAL)
+    assert L.enlsipb200_large_create(capi.FAMILY_SINGLE_INDEX, 6176, 10000, 10000, 4, 0, rho.ctypes.data, None, None, -1, ctypes.byref(h)) == -1
+    assert b"n <= 6144" in L.enlsipb200_large_last_error()
 
 
 def test_product_does_not_import_oracle():

@@ -36,10 +36,12 @@ __device__ double jac_constraint(int k, int j, int, const double* x, const doubl
 }
 """
 
-# a data-carrying problem without user Jacobians: y_i ~ x0 exp(-x1 t_i) + x2 / (1 + x3 t_i^2)  (n = 4, m = 1200 points),
+# a data-carrying problem without user Jacobians: y_i ~ x0 exp(-x1 t_i) + x2 / (1 + x3 t_i^2)  (n = 4, m points),
 # one inequality (x0 + x2 <= 3), bounds on every parameter (the upper bound of x0 is active at the solution): forward
-# differences throughout
+# differences throughout.  m is compiled into the library.  At m = 1200 the [J | r] QR (1200 x 5) runs in a thread-block
+# cluster; at m = 50 000 it takes the unblocked column loop with reflectors too long for shared memory.
 MIX_M = 1200
+MIX_MS = (MIX_M, 50_000)
 MIX_SRC = r"""
 namespace enl_user {
 template <class X> __device__ double residual(long long i, int, const X& x, const double* t, const double* y) {
@@ -54,11 +56,16 @@ template <class X> __device__ double constraint(int, int, const X& x, const doub
 """
 
 
-def mix_problem(seed=3):
+def mix_family(m=MIX_M):
+    """MIX_SRC compiled for m data points (one library per m)."""
+    import enlsip_jl_b200 as E
+    return E.LargeUserFamily(MIX_SRC, m=m, nb_ineqcons=1, data=("t", "y"), name="mix_user" if m == MIX_M else "mix%d_user" % m)
+
+
+def mix_problem(seed=3, m=MIX_M):
     """numpy restatement of MIX_SRC for the oracle (forward-difference Jacobians)."""
     from oracle import enlsip_oracle as O
     rng = np.random.default_rng(seed)
-    m = MIX_M
     t = np.linspace(0.0, 4.0, m)
     truth = np.array([2.0, 1.3, 0.7, 0.25])
     def model(x):
@@ -75,7 +82,7 @@ def test_large_user_sources_compile():
     """nvcc builds both user families for sm_100a in this container (no GPU needed); the libraries export the large API."""
     import enlsip_jl_b200 as E
     for fam in (E.LargeUserFamily(CR_SRC, m=2 * (1000 - 1), nb_eqcons=998, has_jacobians=True, name="cr1000_user"),
-                E.LargeUserFamily(MIX_SRC, m=MIX_M, nb_ineqcons=1, data=("t", "y"), name="mix_user")):
+                *(mix_family(m) for m in MIX_MS)):
         L = fam.library()
         for sym in ("enlsipb200_large_create", "enlsipb200_large_solve", "enlsipb200_large_set_data", "enlsipb200_large_stats"):
             assert hasattr(L, sym)
@@ -96,14 +103,13 @@ def test_user_chained_rosenbrock_equals_builtin():
     u.close(); b.close()
 
 
-@pytest.mark.gpu
-def test_user_data_family_vs_oracle():
-    """n = 4, m = 1200 (n + m >= 1000), data slots t / y, one inequality + 8 bounds, no user Jacobians (forward
+def check_user_data_family_vs_oracle(m):
+    """n = 4, m data points (n + m >= 1000), data slots t / y, one inequality + 8 bounds, no user Jacobians (forward
     differences): status / iterations / working set as the oracle, f and x to the forward-difference noise floor."""
     import enlsip_jl_b200 as E
     from oracle import enlsip_oracle as O
-    pb, t, y, lo, up = mix_problem()
-    fam = E.LargeUserFamily(MIX_SRC, m=MIX_M, nb_ineqcons=1, data=("t", "y"), name="mix_user")
+    pb, t, y, lo, up = mix_problem(m=m)
+    fam = mix_family(m)
     mod = E.LargeCnlsModel(fam, pb.x0, data={"t": t, "y": y}, x_low=lo, x_upp=up)
     assert mod.jacobian == "forward_diff" and mod.nb_constraints == 9
     E.solve(mod, trace_cap=100)
@@ -114,3 +120,16 @@ def test_user_data_family_vs_oracle():
     assert abs(float(mod.obj_value[0]) - r.f) <= 1e-8 * max(r.f, 1e-300)
     assert np.linalg.norm(mod.sol[0] - r.x) <= 1e-6 * np.linalg.norm(r.x)
     mod.close()
+
+
+@pytest.mark.gpu
+def test_user_data_family_vs_oracle():
+    """m = 1200: [J | r] (1200 x 5) is factored in a thread-block cluster."""
+    check_user_data_family_vs_oracle(MIX_M)
+
+
+@pytest.mark.gpu
+def test_tall_user_data_family_vs_oracle():
+    """m = 50 000: [J | r] (50 000 x 5) is factored by the unblocked column loop, its reflectors too long for shared
+    memory and read from global memory."""
+    check_user_data_family_vs_oracle(MIX_MS[1])
