@@ -334,7 +334,8 @@ __global__ void si_jac_bounds_kernel(const int* __restrict__ idx, int nlo, int n
 struct LargeHandle : LargeOps, SmallBackend {
     int device = 0;
     // ---- SmallBackend state: the small stage's matrices, all column major in HBM ----
-    int tcap = 0, lv = 0;             // capacity of the working set min(l, n); length of the scratch vectors
+    int tcap = 0, lv = 0;             // the working-set buffers hold tcap + 1 rows (min(l, n) + 1 at first, grown on
+                                      // demand up to l); length of the scratch vectors
     double* dArow = nullptr;          // A, row major l x n  (= column-major n x l)
     double *dCA = nullptr, *dCA2 = nullptr;   // C.A, row major t x n (= C.A' column major n x t); spare for row removal
     double *dFA = nullptr, *dtauA = nullptr;  // factors of qr(C.A')   n x t
@@ -355,7 +356,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     int fa_rows = 0, fa_cols = 0, fa_k = 0, fl_rows = 0, fl_cols = 0, fl_k = 0, f2_rows = 0, f2_cols = 0, f2_k = 0;
     bool jq1_valid = false;
     int ca_rows = 0;
-    long long n_dev_qrcp = 0, n_dev_mulq = 0;
+    long long n_dev_qrcp = 0, n_dev_mulq = 0, n_ws_grow = 0;
     double ms_small = 0;              // host wall clock inside the small-stage calls (kernels + waits)
 
     // general row families (enl_large_generic.cuh): gv != nullptr; [J | r] column major in dQ, factored without pivoting
@@ -501,16 +502,12 @@ struct LargeHandle : LargeOps, SmallBackend {
         LCU(cudaMalloc(&dscal, sizeof(double) * 8));
         LCU(cudaHostAlloc(&hst, sizeof(double) * 4 * (size_t)lv, cudaHostAllocDefault));
         LCU(cudaHostAlloc(&hsti, sizeof(int) * 2 * (size_t)lv, cudaHostAllocDefault));
-        const int maxc = (int)mt;    // no factorisation of the solve has more columns than n (< n + 1)
-        qw.cap_cols = maxc;
-        LCU(cudaMalloc(&qw.vn1, sizeof(double) * maxc));
-        LCU(cudaMalloc(&qw.vn2, sizeof(double) * maxc));
-        LCU(cudaMalloc(&qw.F, sizeof(double) * (size_t)maxc * enl_small::QR_NB));
+        // per-column QR scratch: n + 1 columns ([J | r], J2, and qr(C.A') while t <= n + 1); ensure_ws_capacity grows it
+        if (alloc_qr_cols((int)mt) != 0) return lfail(ENLSIPB200_ENOMEM, "cudaMalloc");
         LCU(cudaMalloc(&qw.auxv, sizeof(double) * enl_small::QR_NB));
         LCU(cudaMalloc(&qw.pbest, sizeof(double) * enl_small::QR_MAXPART));
         LCU(cudaMalloc(&qw.psum, sizeof(double) * enl_small::QR_PSUM_LEN));
         LCU(cudaMalloc(&qw.pidx, sizeof(int) * enl_small::QR_PIDX_LEN));
-        LCU(cudaMalloc(&qw.flags, sizeof(int) * maxc));
         LCU(cudaMalloc(&qw.state, sizeof(enl_small::QrState)));
         LCU(cudaMalloc(&qw.ticket, sizeof(unsigned int) * enl_small::QR_TICKET_LEN));
         LCU(cudaMemsetAsync(qw.ticket, 0, sizeof(unsigned int) * enl_small::QR_TICKET_LEN, st));
@@ -536,6 +533,57 @@ struct LargeHandle : LargeOps, SmallBackend {
         }
         LCU(cudaGetLastError());
         return 0;
+    }
+    // QrWork's per-column arrays for `cols` columns (the contents are scratch of one factorisation)
+    int alloc_qr_cols(int cols) {
+        for (double* p : {qw.vn1, qw.vn2, qw.F}) if (p) cudaFree(p);
+        if (qw.flags) cudaFree(qw.flags);
+        qw.vn1 = qw.vn2 = qw.F = nullptr; qw.flags = nullptr; qw.cap_cols = 0;
+        if (cudaMalloc(&qw.vn1, sizeof(double) * cols) != cudaSuccess || cudaMalloc(&qw.vn2, sizeof(double) * cols) != cudaSuccess ||
+            cudaMalloc(&qw.F, sizeof(double) * (size_t)cols * enl_small::QR_NB) != cudaSuccess ||
+            cudaMalloc(&qw.flags, sizeof(int) * cols) != cudaSuccess)
+            return -1;
+        qw.cap_cols = cols;
+        return 0;
+    }
+    // Nothing bounds the working set by n: init_working_set takes every violated row, so t can reach l.  The buffers
+    // sized by t are (re)allocated here, before t rows enter C.A; their contents are rebuilt by gather_active and the
+    // factorisations that follow, so nothing is copied.  The small stage runs identically on every rank, so every rank
+    // grows at the same call.  Starts whose working set stays within min(l, n) + 1 rows never come here.
+    void ensure_ws_capacity(int t) {
+        if (t <= tcap + 1) return;
+        // rows of C.A the new buffers hold (never fewer than alloc_small's min(l, n) + 1, also after a failed growth)
+        const int rows = std::min(l, std::max({t, 2 * (tcap + 1), std::min(l, n) + 1}));
+        sm_sync();
+        // until every new buffer exists the handle holds no working set: a cudaMalloc failure below throws with tcap = -1,
+        // so need_ws refuses every later call and the next gather_active allocates afresh
+        tcap = -1;
+        for (double** p : {&dCA, &dCA2, &dFA, &dtauA, &dFL, &dtauL}) { if (*p) cudaFree(*p); *p = nullptr; }
+        for (int** p : {&dpA, &dipA, &dpL, &dipL}) { if (*p) cudaFree(*p); *p = nullptr; }
+        qw.drop_graphs();                 // captured QR graphs hold the old factor and scratch pointers
+        sm_check(cudaMalloc(&dCA, sizeof(double) * (size_t)rows * n), "cudaMalloc");
+        sm_check(cudaMalloc(&dFA, sizeof(double) * (size_t)n * rows), "cudaMalloc");
+        sm_check(cudaMalloc(&dtauA, sizeof(double) * rows), "cudaMalloc");
+        sm_check(cudaMalloc(&dFL, sizeof(double) * (size_t)rows * std::min(rows, n)), "cudaMalloc");   // t x min(n, t)
+        sm_check(cudaMalloc(&dtauL, sizeof(double) * rows), "cudaMalloc");
+        for (int** p : {&dpA, &dipA, &dpL, &dipL}) sm_check(cudaMalloc(p, sizeof(int) * rows), "cudaMalloc");
+        const int qcols = std::max(rows, n + 1);       // [J | r] and J2 need n + 1 columns whatever t is
+        if (qcols > qw.cap_cols && alloc_qr_cols(qcols) != 0) sm_check(cudaErrorMemoryAllocation, "cudaMalloc");
+        ta_valid = tl_valid = jq1_valid = false;
+        tcap = rows - 1;
+        ++n_ws_grow;
+    }
+    // every small-stage entry point that takes t: refuse a working set the buffers do not hold
+    void need_ws(int t) const {
+        if (t > tcap + 1)
+            throw std::runtime_error("device small stage: working set of " + std::to_string(t) + " rows exceeds the " +
+                                     std::to_string(tcap + 1) + " rows of its buffers");
+    }
+    void qrcp(double* f, int rows, int cols, double* tau, int* jpvt) {
+        const int rc = enl_small::qrcp_device(f, rows, cols, tau, jpvt, qw, st);
+        if (rc < 0) throw std::runtime_error("device small stage: pivoted QR with more columns than its scratch holds");
+        launches += rc;
+        ++n_dev_qrcp;
     }
     int grid_rows() const {   // CTAs for the warp-per-row kernels
         long long want = (m_local + 7) / 8;
@@ -651,7 +699,9 @@ struct LargeHandle : LargeOps, SmallBackend {
         LCU(cudaSetDevice(device));
         if (gv) {      // plain Householder QR of the column-major [J | r] (dgeqrf order), R -> [J~ | r~]
             LCU(cudaEventRecord(e1, st));
-            launches += enl_small::qrcp_device(dQ, (int)m_local, n + 1, dtauQ, dpQ, qw, st, 1);
+            const int rc = enl_small::qrcp_device(dQ, (int)m_local, n + 1, dtauQ, dpQ, qw, st, 1);
+            if (rc < 0) return lfail(ENLSIPB200_ECUDA, "QR of [J | r]: more columns than the QR scratch holds");
+            launches += rc;
             const long long ne = (long long)(n + 1) * (n + 1);
             enl_small::upper_to_square_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(dQ, (int)m_local, n + 1, dJc);
             ++launches;
@@ -828,6 +878,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void gather_active(const int* active, int t) override {
         SmallScope sc_(this);
+        ensure_ws_capacity(t);
         ca_rows = t;
         if (t <= 0) return;
         up_i(dact, active, t);
@@ -836,6 +887,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void evaluate_scaling(int t, bool scaling, double* rown) override {
         SmallScope sc_(this);
+        need_ws(t);
         if (t <= 0) return;
         enl_small::row_norm_scale_kernel<<<t, 256, 0, st>>>(dCA, n, scaling ? 1 : 0, dvec[0]);
         ++launches;
@@ -845,6 +897,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void rebuild_scaled_rows(const int* active, int t, const double* diag_scale) override {
         SmallScope sc_(this);
+        need_ws(t);
         if (t <= 0) return;
         up_i(dact, active, t);
         up(dvec[0], diag_scale, t);
@@ -853,6 +906,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void remove_active_row(int s0) override {
         SmallScope sc_(this);
+        need_ws(ca_rows);
         const int below = ca_rows - 1 - s0;
         if (below > 0) {
             if (!dCA2) sm_check(cudaMalloc(&dCA2, sizeof(double) * (size_t)(tcap + 1) * n), "cudaMalloc");
@@ -864,27 +918,27 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void factor_A(int t, FactorInfo& F) override {
         SmallScope sc_(this);
+        need_ws(t);
         fa_rows = n; fa_cols = t; fa_k = n < t ? n : t;
         jq1_valid = false;
         if (t > 0) {
             sm_check(cudaMemcpyAsync(dFA, dCA, sizeof(double) * (size_t)n * t, cudaMemcpyDeviceToDevice, st), "D2D");
-            launches += enl_small::qrcp_device(dFA, n, t, dtauA, dpA, qw, st);
+            qrcp(dFA, n, t, dtauA, dpA);
             ta_valid = false;
-            ++n_dev_qrcp;
         }
         finish_factor(dFA, n, t, dpA, dipA, F, hpA);
     }
     void factor_L11(FactorInfo& F) override {    // qr(F_A.R', ColumnNorm()); F_A.R is min(n, t) x t
         SmallScope sc_(this);
         const int kr = fa_k, t = fa_cols;
+        need_ws(t);
         fl_rows = t; fl_cols = kr; fl_k = t < kr ? t : kr;
         if (t > 0 && kr > 0) {
             const long long ne = (long long)t * kr;
             enl_small::build_rt_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(dFA, n, t, kr, dFL);
             ++launches;
-            launches += enl_small::qrcp_device(dFL, t, kr, dtauL, dpL, qw, st);
+            qrcp(dFL, t, kr, dtauL, dpL);
             tl_valid = false;
-            ++n_dev_qrcp;
         }
         finish_factor(dFL, t, kr, dpL, dipL, F, hpL);
     }
@@ -906,14 +960,14 @@ struct LargeHandle : LargeOps, SmallBackend {
         f2_rows = mt; f2_cols = cols2; f2_k = mt < cols2 ? mt : cols2;
         if (cols2 > 0) {
             sm_check(cudaMemcpyAsync(dF2, dJQ1 + (size_t)rankA * mt, sizeof(double) * (size_t)mt * cols2, cudaMemcpyDeviceToDevice, st), "D2D");
-            launches += enl_small::qrcp_device(dF2, mt, cols2, dtau2, dp2, qw, st);
+            qrcp(dF2, mt, cols2, dtau2, dp2);
             t2_valid = false;
-            ++n_dev_qrcp;
         }
         finish_factor(dF2, mt, cols2, dp2, dip2, F, hp2);
     }
     void first_lagrange(int prankA, int t, const Vec& gradf, const Vec& Ccx, Vec& v, Vec& u, double& grad_res) override {
         SmallScope sc_(this);
+        need_ws(t);
         Vec y0(t > 0 ? t : 1, 0.0);
         for (int i = 0; i < prankA; ++i) y0[i] = -Ccx[hpA[i]];
         up(dvec[0], gradf.data(), n);
@@ -935,6 +989,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void second_lagrange(int prankA, int t, const Vec& p_gn, Vec& v) override {
         SmallScope sc_(this);
+        need_ws(t);
         ensure_jq1();
         const int mt = n + 1;
         const double* rtd = dJc + (size_t)mt * n;
@@ -949,6 +1004,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void sub_search_direction(int t, int rankA, int dimA, int dimJ2, int code, const Vec& Ccx, Vec& p, Vec& b, Vec& d) override {
         SmallScope sc_(this);
+        need_ws(t);
         ensure_jq1();
         const int mt = n + 1;
         const double* rtd = dJc + (size_t)mt * n;
@@ -991,6 +1047,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void subspace_rhs(int t, const Vec& Ccx, Vec& b) override {
         SmallScope sc_(this);
+        need_ws(t);
         ensure_jq1();
         Vec b0(t > 0 ? t : 1, 0.0);
         for (int i = 0; i < t; ++i) b0[i] = -Ccx[hpA[i]];
@@ -1024,6 +1081,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     void products(const Vec& p, int t, Vec& Jp, Vec& Ap, Vec& active_Ap) override {
         SmallScope sc_(this);
+        need_ws(t);
         const int mt = n + 1;
         up(dvec[0], p.data(), n);
         launches += enl_small::gemv_n(dJc, mt, mt, n, dvec[0], 1.0, nullptr, 0.0, dvec[1], st);
@@ -1039,6 +1097,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     }
     double At_c_norm(int t, const Vec& Ccx) override {
         SmallScope sc_(this);
+        need_ws(t);
         if (ca_rows <= 0 || t <= 0) return 0.0;
         up(dvec[0], Ccx.data(), t);
         launches += enl_small::gemv_n(dCA, n, n, t, dvec[0], 1.0, nullptr, 0.0, dvec[1], st);
@@ -1353,10 +1412,10 @@ int enlsipb200_large_factor(enlsipb200_large hh, const double* x, double* R, flo
 int enlsipb200_large_stats(enlsipb200_large hh, double* out, int count) {
     LargeHandle* h = LH(hh);
     if (!h || !out) return lfail(ENLSIPB200_EINVAL, "NULL argument");
-    double v[12] = {(double)h->n_newpoint, h->ms_build, h->ms_tsqr, h->ms_ls, h->ms_total, (double)h->n_ls,
+    double v[13] = {(double)h->n_newpoint, h->ms_build, h->ms_tsqr, h->ms_ls, h->ms_total, (double)h->n_ls,
                     (double)h->launches, (double)h->rows_pad, (double)h->n_dev_qrcp, (double)h->n_dev_mulq, h->ms_small,
-                    (double)h->n_factor};
-    for (int i = 0; i < count && i < 12; ++i) out[i] = v[i];
+                    (double)h->n_factor, (double)h->n_ws_grow};
+    for (int i = 0; i < count && i < 13; ++i) out[i] = v[i];
     return 0;
 }
 

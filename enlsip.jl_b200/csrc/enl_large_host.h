@@ -22,6 +22,7 @@
 // Newton steps (EF:348-423) do not exist in this regime: `second_derivatives` is forced off when
 // n + m >= 1000 (EF:2658), and the entry point rejects smaller problems (they belong to the batched engine).
 #pragma once
+#include <float.h>
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -66,6 +67,19 @@ inline double dot_n(const double* a, const double* b, int n) {
     return (s0 + s1) + (s2 + s3);
 }
 inline double norm_n(const double* a, int n) { return sqrt(dot_n(a, a, n)); }
+// dnrm2 as dgeqp3 / dlaqp2 / dlarfg call it (OpenBLAS' x86-64 kernel sums the squares in x87 extended precision, then
+// rounds the square root to double).  With row scaling every column of C.A' has norm 1 up to an ulp, and the pivot
+// order is decided by how that last bit rounds: a plain double sum picks other pivots than the reference.
+// Where long double is not the x87 format (aarch64: IEEE quad) the sum stays in double.
+inline double nrm2_ext(const double* a, int n) {
+#if LDBL_MANT_DIG == 64
+    long double s = 0.0L;
+    for (int i = 0; i < n; ++i) s += (long double)a[i] * a[i];
+    return (double)sqrtl(s);
+#else
+    return norm_n(a, n);
+#endif
+}
 inline double dotv(const Vec& a, const Vec& b) { return dot_n(a.data(), b.data(), (int)a.size()); }
 inline double normv(const Vec& a) { return norm_n(a.data(), (int)a.size()); }
 inline double lapy2(double x, double y) {
@@ -125,7 +139,7 @@ struct QRP {
         Vec vn1(cols), vn2(cols);
         for (int j = 0; j < cols; ++j) {
             p[j] = j;
-            vn1[j] = vn2[j] = norm_n(f.col(j), rows);
+            vn1[j] = vn2[j] = nrm2_ext(f.col(j), rows);
         }
         Vec wv(cols);
         for (int i = 0; i < k; ++i) {
@@ -143,7 +157,7 @@ struct QRP {
             double tau_i = 0.0;
             if (i < rows - 1) {
                 double alpha = ci[i];
-                double xn = norm_n(ci + i + 1, rows - i - 1);
+                double xn = nrm2_ext(ci + i + 1, rows - i - 1);
                 if (xn != 0.0) {
                     double beta = -copysign(lapy2(alpha, xn), alpha);
                     tau_i = (beta - alpha) / beta;
@@ -172,7 +186,7 @@ struct QRP {
                     double temp2 = temp * (rq * rq);
                     if (temp2 <= TOL3Z) {
                         if (i < rows - 1) {
-                            vn1[j] = vn2[j] = norm_n(f.col(j) + i + 1, rows - i - 1);
+                            vn1[j] = vn2[j] = nrm2_ext(f.col(j) + i + 1, rows - i - 1);
                         } else {
                             vn1[j] = vn2[j] = 0.0;
                         }
@@ -750,7 +764,9 @@ public:
             if (dimA > t || dimA > F_L11.k) throw WouldThrow{"BoundsError R11[1:dimA,1:dimA]"};
             need_nonzero_diag(F_L11, std::max(dimA, 0), "SingularException (upper)");
             if (t - dimA < 0) throw WouldThrow{"negative zeros() length"};
-            if (F_L11.cols != t) throw WouldThrow{"BoundsError in invperm indexing"};
+            // [dp1; zeros(t - dimA)][invperm(F_L11)] indexes a t-vector with a permutation of length min(n, t):
+            // legal in Julia unless the permutation is the longer one
+            if (F_L11.cols > t) throw WouldThrow{"BoundsError in invperm indexing"};
             if (rankA > t) throw WouldThrow{"BoundsError [1:rankA]"};
             np1 = rankA;
         } else {

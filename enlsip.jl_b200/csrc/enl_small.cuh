@@ -1328,10 +1328,12 @@ inline int qr_enqueue_panel(double* f, int rows, int cols, double* tau, int* jpv
 }
 
 // f: rows x cols column major on the device, factored in place (dgeqp3 layout); tau [min(rows, cols)]; jpvt [cols]
-// (0-based).  Returns the number of kernels launched.  At most one host synchronisation (blocked phase only).
+// (0-based).  Returns the number of kernels launched, or -1 (nothing launched) when `cols` exceeds the per-column scratch
+// of `wk` (wk.cap_cols).  At most one host synchronisation (blocked phase only).
 inline int qrcp_device(double* f, int rows, int cols, double* tau, int* jpvt, QrWork& wk, cudaStream_t st, int nopivot = 0) {
     const int minmn = rows < cols ? rows : cols;
     if (minmn <= 0) return 0;
+    if (cols > wk.cap_cols) return -1;
     // cluster size: the smallest of 2 / 4 / 8 CTAs whose shared memory holds the matrix with at most one column per warp
     // (a single round of the warp-per-column update), else 8; ENLSIP_QC_NC overrides it.  Measured (B200, 512 threads):
     // 256 x 64: 0.43 / 0.34 / 0.30 / 0.34 ms with 1 / 2 / 4 / 8 CTAs, 64 x 64: 0.34 / 0.29 / 0.26 / 0.27 ms -- a column step

@@ -1684,7 +1684,7 @@ struct Solver {
 #pragma unroll 1
         for (int i = Q + 1; i <= l; ++i) {
             if (cx[i - 1] <= 0.0) {
-                if (t < T) active[t] = i;
+                active[t] = i;          // t < l <= LMAX: the whole initial working set is kept, also beyond T
                 t += 1;
             } else {
                 inactive[lmt++] = i;
@@ -1693,7 +1693,9 @@ struct Solver {
         cur = IterRec{};
         cur.alpha = 1.0;
         cur.code = 1;
-        if (t > T) { exit_code = EXIT_CAPACITY; t = T; return; }
+        // more active rows than the shared-memory factorisations hold: x = x0, f = ||r(x0)||^2, no iteration, and
+        // nact / active report the whole initial working set (store)
+        if (t > T) { exit_code = EXIT_CAPACITY; return; }
         cur.t = t;
         gather_active();
         prev = cur;
@@ -1770,7 +1772,7 @@ struct Solver {
 #pragma unroll 1
         for (int i = Q + 1; i <= l; ++i) {
             if (cx[i - 1] <= 0.0) {
-                if (t < T) active[t] = i;
+                active[t] = i;          // t < l <= LMAX: the whole initial working set is kept, also beyond T
                 t += 1;
             } else {
                 inactive[lmt++] = i;
@@ -1779,21 +1781,24 @@ struct Solver {
         cur = IterRec{};
         cur.alpha = 1.0;
         cur.code = 1;
-        if (t > T) { exit_code = EXIT_CAPACITY; t = T; return; }
+        if (t > T) { exit_code = EXIT_CAPACITY; return; }
         cur.t = t;
         gather_active();
         evaluate_scaling();
         update_working_set();
         if (threw) exit_code = EXIT_WOULD_THROW;
     }
-    // p [N], lam [T] (in working-set order, 0 padded), active [LMAX], info = {t, rankA, rankJ2, index_del, code}
+    // p [N], lam [T] (in working-set order, 0 padded), active [LMAX], info = {t, rankA, rankJ2, index_del, code}.  A
+    // problem that ends with an error code gets p = 0 and lam = 0: -97 returns before any direction is computed, so
+    // the slot's p / lam still hold whatever problem it served before.
     ENL_NOINL void store_step(double* p_out, double* lam_out, int* active_out, int* info_out, long long bidx) {
         if (grp().lane != 0) return;
+        const bool ok = exit_code == 0;
 #pragma unroll 1
-        for (int j = 0; j < N; ++j) p_out[bidx * N + j] = p[j];
+        for (int j = 0; j < N; ++j) p_out[bidx * N + j] = ok ? p[j] : 0.0;
         if (lam_out)
 #pragma unroll 1
-            for (int i = 0; i < T; ++i) lam_out[bidx * T + i] = (i < t) ? lam[i] : 0.0;
+            for (int i = 0; i < T; ++i) lam_out[bidx * T + i] = (ok && i < t) ? lam[i] : 0.0;
         if (active_out)
 #pragma unroll 1
             for (int i = 0; i < LMAX; ++i) active_out[bidx * LMAX + i] = (i < t) ? active[i] : 0;

@@ -169,10 +169,10 @@ class LargeCnlsModel:
         return R, float(b.value), float(t.value)
 
     def stats(self):
-        v = np.zeros(12)
-        capi.check_large(self._lib.enlsipb200_large_stats(self._h, v.ctypes.data, 12), self._lib)
+        v = np.zeros(13)
+        capi.check_large(self._lib.enlsipb200_large_stats(self._h, v.ctypes.data, 13), self._lib)
         keys = ("points", "build_ms", "tsqr_ms", "linesearch_ms", "solve_wall_ms", "linesearch_evals",
-                "launches", "rows_pad", "device_qrcp", "device_mulq", "small_stage_ms", "factorisations")
+                "launches", "rows_pad", "device_qrcp", "device_mulq", "small_stage_ms", "factorisations", "ws_growths")
         return dict(zip(keys, [float(a) for a in v]))
 
     def launch_count(self):

@@ -50,7 +50,12 @@ extern "C" {
 /* extra per-problem exit codes (besides the reference's, EF:2371-2396) */
 #define ENLSIPB200_EXIT_WOULD_THROW -99  /* the reference raises a Julia exception at this point      */
 #define ENLSIPB200_EXIT_WOULD_HANG -98   /* the reference loops forever at this point (EF:621-647)    */
-#define ENLSIPB200_EXIT_CAPACITY -97     /* initial working set larger than min(l, n)                 */
+#define ENLSIPB200_EXIT_CAPACITY -97     /* batched regime only: initial working set larger than       */
+                                         /* min(lmax, n); x = x0, f = ||r(x0)||^2, iterations 0, nact / */
+                                         /* active = the whole initial working set, counters = {2, 2}   */
+                                         /* (the one evaluation of r, c, J and A at x0: unlike -11 with */
+                                         /* time_limit < 0, which reports 0).  The large regime has no  */
+                                         /* such limit (its buffers grow with the working set).         */
 
 #define ENLSIPB200_TRACE_HDR 16          /* doubles per trace row before the n iterate entries         */
 
@@ -115,7 +120,8 @@ ENLSIPB200_API int enlsipb200_eval_batch(enlsipb200_handle h, long long B, const
  * possible deletion) applied to r [B, m], J [B, n, m], c [B, lmax], A [B, lmax, n] in the layout enlsipb200_eval_batch
  * writes, from the working set of init_working_set (:826-859).  Outputs: p [B, n] (Gauss-Newton direction), lam
  * [B, min(lmax, n)] (multipliers in working-set order, 0 padded; may be NULL), active [B, lmax] (may be NULL),
- * info [B, 5] = {t, rankA, rankJ2, index_del, error code (0, -99, -97)} (may be NULL).  DEVICE buffers only. */
+ * info [B, 5] = {t, rankA, rankJ2, index_del, error code (0, -99, -97)} (may be NULL).  A problem with a nonzero error
+ * code gets p = 0 and lam = 0; with -97, t and active are the whole initial working set.  DEVICE buffers only. */
 ENLSIPB200_API int enlsipb200_step_batch(enlsipb200_handle h, long long B, const double* x, const double* r, const double* J,
                                          const double* c, const double* A, const enlsipb200_options* opt, double* p, double* lam,
                                          int* active, int* info, int on_device, void* stream);
@@ -205,7 +211,8 @@ ENLSIPB200_API int enlsipb200_large_factor(enlsipb200_large h, const double* x, 
 /* cumulative counters: {points evaluated (new_point!), build ms, tsqr ms, linesearch ms, solve wall ms, linesearch
  * evaluations (host clock around launch..result), kernels launched, padded local rows, device QRCPs, device M*Q products,
  * ms inside the small-stage calls (host clock: kernels + the waits for their results), factorisations of [J | r] (one per
- * point from which the iteration continued)} */
+ * point from which the iteration continued), growths of the working-set buffers (a working set of more than
+ * min(l, n) + 1 rows)}; `count` may stop short of the last entries */
 ENLSIPB200_API int enlsipb200_large_stats(enlsipb200_large h, double* out, int count);
 
 /* Known-answer hooks of the small stage's dense kernels (csrc/enl_small.cuh), host buffers, column major:
