@@ -9,7 +9,8 @@ device is missing -- there is no CPU fallback.
 from . import capi, synth
 from .model import (CnlsModel, UserFamily, solve, solve_b, status, solution, sum_sq_residuals, constraints_values,
                     total_nb_constraints, dict_status_codes, evaluate, gn_step)
-from .model_large import LargeCnlsModel, LargeUserFamily, solve_large
+from .model_large import LargeCnlsModel, LargeUserFamily, shard_rows, solve_large
 
 __all__ = ["capi", "synth", "CnlsModel", "UserFamily", "solve", "solve_b", "status", "solution", "sum_sq_residuals",
-           "constraints_values", "total_nb_constraints", "dict_status_codes", "evaluate", "gn_step", "LargeCnlsModel", "LargeUserFamily", "solve_large"]
+           "constraints_values", "total_nb_constraints", "dict_status_codes", "evaluate", "gn_step", "LargeCnlsModel", "LargeUserFamily", "shard_rows",
+           "solve_large"]

@@ -20,6 +20,7 @@ HEADERS_LARGE = [os.path.join(_HERE, "csrc", f) for f in ("enl_base.h", "enl_tsq
 OBJ_DIR = os.path.join(_HERE, "lib", "obj")
 FAMILY_SINGLE_INDEX = 16
 FAMILY_LARGE_CHAINED_ROSENBROCK = 17
+LARGE_FACTOR_TSQR = 0x100   # OR-ed into the family: row families factor [J | r] with the TSQR and may be row-sharded
 
 FAMILY_HS65 = 0
 FAMILY_GAUSS_PEAKS = 1

@@ -13,6 +13,9 @@
 //   li_dir_kernel        v = W p, Jp = s .* v, {r.r, r.Jp, Jp.Jp}                              (EF:2222-2224)
 //   li_ls_kernel         per trial step: ||r(x + a p)||^2 and the linesearch model dots        (EF:1307-1340, 1665-1689)
 //   NCCL all-reduce      of those few doubles
+// General row families (enl_large_generic.cuh) take the same TSQR path when created with ENLSIPB200_LARGE_FACTOR_TSQR
+// (lg_build_rows_kernel -> tsqr_factor on n rounded up to 32 columns -> rows_unpad_kernel); without it their column-major
+// [J | r] goes through the plain-Householder mode of qrcp_device.
 // sm_100a only; no CPU fallback (every entry point fails with ENLSIPB200_ENOGPU without a device).
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -313,6 +316,33 @@ __global__ void r_to_colmajor_kernel(const double* __restrict__ R, int ld, int n
     }
 }
 
+// TSQR path of the row families: R of [J | 0 | r] (row major, leading dimension ld; nt = n rounded up to 32, r in column
+// nt) -> the column-major (n+1) x (n+1) [R_J | z ; 0 | rho] of the compressed problem.  The zero columns n..nt-1 got
+// identity reflectors (tau = 0), so rows n..nt-1 of the r column hold entries of r that no reflector reduced, and R[nt][nt]
+// is the norm of what the panels left in the r column below the extracted rows.  rho counts each of them once:
+// rho = sqrt(R[nt][nt]^2 + sum_{k=n}^{nt-1} R[k][nt]^2) (= R[n][n] itself when nt = n).
+__global__ void rows_unpad_kernel(const double* __restrict__ R, int ld, int n, int nt, double* __restrict__ out) {
+    const int nc = n + 1;
+    const long long ne = (long long)nc * nc;
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < ne; e += (long long)gridDim.x * blockDim.x) {
+        const int c = (int)(e / nc), r = (int)(e % nc);
+        double v;
+        if (c < n) {
+            v = (r <= c) ? R[(size_t)r * ld + c] : 0.0;
+        } else if (r < n) {
+            v = R[(size_t)r * ld + nt];
+        } else if (nt == n) {
+            v = R[(size_t)nt * ld + nt];
+        } else {
+            double sq = 0.0;
+            for (int k = n; k < nt; ++k) sq = fma(R[(size_t)k * ld + nt], R[(size_t)k * ld + nt], sq);
+            const double d = R[(size_t)nt * ld + nt];
+            v = sqrt(fma(d, d, sq));
+        }
+        out[e] = v;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // device implementation of LargeOps
 // ---------------------------------------------------------------------------------------------
@@ -367,6 +397,13 @@ struct LargeHandle : LargeOps, SmallBackend {
     const double* gd[2] = {nullptr, nullptr};     // family data slots
     double* gown[2] = {nullptr, nullptr};
     int jac_fd = 0;                   // forward-difference Jacobians requested (cnls_model.jl:65-82)
+    // ENLSIPB200_LARGE_FACTOR_TSQR: [J | 0 | r] row major in dA (nt columns for J, nt = n rounded up to 32), factored by
+    // tsqr_factor like the single-index family; a row-major copy of J (dJrow) serves J p.  This rank holds the global rows
+    // row0 .. row0 + m_local - 1; rows_joined: the shards are known to cover m (always so when m_local = m).
+    bool tsqr_rows = false, rows_joined = true;
+    long long row0 = 0;
+    double* dJrow = nullptr;
+    int nt = 0;                       // columns the TSQR factors: n rounded up to 32 on that path, n otherwise
     std::vector<double> hxcur;        // the point of the last eval (linesearch trial points are x + alpha p)
     long long m_local = 0, rows_pad = 0, dT_subtiles = 0;
     int ld = 0, rr_rows = 0;
@@ -409,10 +446,10 @@ struct LargeHandle : LargeOps, SmallBackend {
         for (double** p : {&dTA, &dTL, &dT2, &dwpart, &dP, &dPscal}) { if (*p) cudaFree(*p); *p = nullptr; }
         tree_dist = false;
         ta_valid = tl_valid = t2_valid = false;
-        for (double* p : {dQ, dJkeep, dtauQ, dcu, gown[0], gown[1]})
+        for (double* p : {dQ, dJkeep, dtauQ, dcu, dJrow, gown[0], gown[1]})
             if (p) cudaFree(p);
         if (dpQ) cudaFree(dpQ);
-        dQ = dJkeep = dtauQ = dcu = nullptr; dpQ = nullptr; gown[0] = gown[1] = nullptr;
+        dQ = dJkeep = dtauQ = dcu = dJrow = nullptr; dpQ = nullptr; gown[0] = gown[1] = nullptr;
         for (int* p : {dpA, dipA, dpL, dipL, dp2, dip2, dact, dbidx, qw.flags, qw.pidx})
             if (p) cudaFree(p);
         qw.drop_graphs();
@@ -447,18 +484,23 @@ struct LargeHandle : LargeOps, SmallBackend {
         LCU(cudaSetDevice(device));
         LCU(cudaStreamCreate(&st));
         LCU(cudaEventCreate(&e0)); LCU(cudaEventCreate(&e1)); LCU(cudaEventCreate(&e2));
-        ld = n + 8;
+        nt = tsqr_rows ? (n + TS_B - 1) / TS_B * TS_B : n;
+        ld = nt + 8;
         rows_pad = ((m_local + TS_B - 1) / TS_B) * TS_B;
         if (rows_pad < TS_B) rows_pad = TS_B;
-        rr_rows = n + TS_B;   // rows of an R factor padded to a multiple of 32
+        rr_rows = nt + TS_B;   // rows of an R factor padded to a multiple of 32
         if (gv) {
             const size_t mm = (size_t)(m_local > 0 ? m_local : 1);
-            LCU(cudaMalloc(&dQ, sizeof(double) * mm * (n + 1)));
-            LCU(cudaMalloc(&dJkeep, sizeof(double) * mm * n));
-            LCU(cudaMalloc(&dtauQ, sizeof(double) * (n + 1)));
-            LCU(cudaMalloc(&dpQ, sizeof(int) * (n + 1)));
+            if (tsqr_rows) {
+                LCU(cudaMalloc(&dJrow, sizeof(double) * mm * n));
+            } else {
+                LCU(cudaMalloc(&dQ, sizeof(double) * mm * (n + 1)));
+                LCU(cudaMalloc(&dJkeep, sizeof(double) * mm * n));
+                LCU(cudaMalloc(&dtauQ, sizeof(double) * (n + 1)));
+                LCU(cudaMalloc(&dpQ, sizeof(int) * (n + 1)));
+                rows_pad = TS_B;      // no TSQR work matrix
+            }
             LCU(cudaMalloc(&dcu, sizeof(double) * (ncu > 0 ? ncu : 1)));
-            rows_pad = TS_B;      // no TSQR work matrix
         }
         LCU(cudaMalloc(&dA, sizeof(double) * rows_pad * ld));
         LCU(cudaMemsetAsync(dA, 0, sizeof(double) * rows_pad * ld, st));
@@ -472,8 +514,8 @@ struct LargeHandle : LargeOps, SmallBackend {
         LCU(cudaMalloc(&dpart, sizeof(double) * LI_PARTS * 4));
         LCU(cudaMalloc(&dout, sizeof(double) * 8));
         LCU(cudaHostAlloc(&hpin, sizeof(double) * 8, cudaHostAllocDefault));
-        LCU(cudaMalloc(&dgpart, sizeof(double) * LI_PARTS * (size_t)(n + 1)));
-        LCU(cudaMalloc(&dgrad, sizeof(double) * (n + 1)));
+        LCU(cudaMalloc(&dgpart, sizeof(double) * LI_PARTS * (size_t)(nt + 1)));
+        LCU(cudaMalloc(&dgrad, sizeof(double) * (nt + 1)));
         LCU(cudaHostAlloc(&hgrad, sizeof(double) * (n + 1), cudaHostAllocDefault));
         LCU(cudaMalloc(&dR, sizeof(double) * rr_rows * ld));
         LCU(cudaMalloc(&dJc, sizeof(double) * (size_t)(n + 1) * (n + 1)));
@@ -609,8 +651,40 @@ struct LargeHandle : LargeOps, SmallBackend {
     bool point_factored = true;
     long long n_factor = 0;
 
+    // row families on the TSQR path: [J | 0 | r] and the copy of J at x, J'r and r'r over CTAs and ranks -> hgrad
+    int eval_at_rows(const double* x) {
+        hxcur.assign(x, x + n);
+        LCU(cudaMemcpyAsync(dx, x, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+        jq1_valid = false;
+        LCU(cudaEventRecord(e0, st));
+        const int parts = grid_rows();
+        gv->build_rows(parts, st, n, m_local, rows_pad, row0, dx, gd[0], gd[1], jac_fd, nt, ld, dA, dJrow, dr);
+        // [J'r | 0 | r'r]: the zero columns give zero sums
+        li_grad_kernel<<<parts, 256, 0, st>>>(dA, ld, m_local, nt, dgpart);
+        li_grad_finish_kernel<<<(nt + 8) / 8, 256, 0, st>>>(dgpart, parts, nt, dgrad);
+        launches += 3;
+        if (nranks > 1) {
+            int rc = g_nccl.AllReduce(dgrad, dgrad, (size_t)nt + 1, NCCL_FLOAT64, NCCL_SUM, comm, st);
+            if (rc != 0) return lfail(ENLSIPB200_ECUDA, std::string("ncclAllReduce: ") + g_nccl.GetErrorString(rc));
+        }
+        gv->cons(st, n, ncu, dx, gd[0], gd[1], dcu);
+        gv->jac_cons(st, n, ncu, dx, gd[0], gd[1], jac_fd, dcu, dArow);
+        launches += 2;
+        LCU(cudaEventRecord(e1, st));
+        LCU(cudaMemcpyAsync(hgrad, dgrad, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+        LCU(cudaMemcpyAsync(hgrad + n, dgrad + nt, sizeof(double), cudaMemcpyDeviceToHost, st));
+        if (ncu > 0) LCU(cudaMemcpyAsync(hst, dcu, sizeof(double) * ncu, cudaMemcpyDeviceToHost, st));
+        LCU(cudaStreamSynchronize(st));
+        LCU(cudaGetLastError());
+        LCU(cudaEventElapsedTime(&last_build_ms, e0, e1));
+        ms_build += last_build_ms;
+        ++n_newpoint;
+        point_factored = false;
+        return 0;
+    }
     // r, s, u and [J | r] at x (li_build_kernel), gradient J'r and r'r reduced over CTAs and ranks -> hgrad (pinned)
     int eval_at_generic(const double* x) {
+        if (tsqr_rows) return eval_at_rows(x);
         hxcur.assign(x, x + n);
         LCU(cudaMemcpyAsync(dx, x, sizeof(double) * n, cudaMemcpyHostToDevice, st));
         jq1_valid = false;
@@ -697,7 +771,7 @@ struct LargeHandle : LargeOps, SmallBackend {
     int factor_point(bool want_host_R = true) {
         if (point_factored) return lfail(ENLSIPB200_EINVAL, "point already factored");
         LCU(cudaSetDevice(device));
-        if (gv) {      // plain Householder QR of the column-major [J | r] (dgeqrf order), R -> [J~ | r~]
+        if (gv && !tsqr_rows) {      // plain Householder QR of the column-major [J | r] (dgeqrf order), R -> [J~ | r~]
             LCU(cudaEventRecord(e1, st));
             const int rc = enl_small::qrcp_device(dQ, (int)m_local, n + 1, dtauQ, dpQ, qw, st, 1);
             if (rc < 0) return lfail(ENLSIPB200_ECUDA, "QR of [J | r]: more columns than the QR scratch holds");
@@ -730,20 +804,24 @@ struct LargeHandle : LargeOps, SmallBackend {
                 LargeHandle* h = static_cast<LargeHandle*>(c);
                 return g_nccl.AllReduce(buf, buf, count, NCCL_FLOAT64, NCCL_SUM, h->comm, s);
             };
-            const int rc = tsqr_factor(dA, ld, rows_pad, n, dR, ld, dT, dpart, st, &td);
+            const int rc = tsqr_factor(dA, ld, rows_pad, nt, dR, ld, dT, dpart, st, &td);
             if (rc < 0) return lfail(ENLSIPB200_ECUDA, "NCCL collective inside the row-sharded TSQR failed");
             launches += rc;
         } else {
-            launches += tsqr_factor(dA, ld, rows_pad, n, dR, ld, dT, dpart, st);
+            launches += tsqr_factor(dA, ld, rows_pad, nt, dR, ld, dT, dpart, st);
         }
         if (nranks > 1 && !tree_dist) {
             int rc = g_nccl.AllGather(dR, dStack, (size_t)rr_rows * ld, NCCL_FLOAT64, comm, st);
             if (rc != 0) return lfail(ENLSIPB200_ECUDA, std::string("ncclAllGather: ") + g_nccl.GetErrorString(rc));
             LCU(cudaMemsetAsync(dR2, 0, sizeof(double) * rr_rows * ld, st));
-            launches += tsqr_factor(dStack, ld, (long long)nranks * rr_rows, n, dR2, ld, dT, dpart, st);
+            launches += tsqr_factor(dStack, ld, (long long)nranks * rr_rows, nt, dR2, ld, dT, dpart, st);
             dfinal = dR2;
         }
-        {
+        if (tsqr_rows) {
+            const long long ne = (long long)(n + 1) * (n + 1);
+            rows_unpad_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(dfinal, ld, n, nt, dJc);
+            ++launches;
+        } else {
             const int nc = n + 1;
             dim3 grid((nc + 31) / 32, (nc + 31) / 32), block(32, 8);
             r_to_colmajor_kernel<<<grid, block, 0, st>>>(dfinal, ld, nc, dJc);
@@ -1133,7 +1211,9 @@ struct LargeHandle : LargeOps, SmallBackend {
         auto t0 = std::chrono::steady_clock::now();
         LCU(cudaMemcpyAsync(dp, p, sizeof(double) * n, cudaMemcpyHostToDevice, st));
         cur_parts = grid_rows();
-        if (gv) {
+        if (gv && tsqr_rows) {
+            lg_dir_rows_kernel<<<cur_parts, 256, 0, st>>>(dJrow, n, m_local, dp, dr, dJp, dpart);
+        } else if (gv) {
             launches += enl_small::gemv_n(dJkeep, (int)m_local, (int)m_local, n, dp, 1.0, nullptr, 0.0, dJp, st);
             lg_dir_sums_kernel<<<cur_parts, 256, 0, st>>>(dr, dJp, m_local, dpart);
         } else {
@@ -1152,7 +1232,7 @@ struct LargeHandle : LargeOps, SmallBackend {
         auto t0 = std::chrono::steady_clock::now();
         long long want = (m_local + 255) / 256;
         cur_parts = (int)(want < LI_PARTS ? (want > 0 ? want : 1) : LI_PARTS);
-        if (gv) gv->ls(cur_parts, st, n, m_local, dx, dp, alpha, gd[0], gd[1], dr, dJp, with_coeffs, dpart);
+        if (gv) gv->ls(cur_parts, st, n, m_local, row0, dx, dp, alpha, gd[0], gd[1], dr, dJp, with_coeffs, dpart);
         else li_ls_kernel<<<cur_parts, 256, 0, st>>>(du, dv, dy, dr, dJp, m_local, alpha, with_coeffs, dpart);
         ++launches;
         int rc = finish4(o);
@@ -1215,6 +1295,8 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
                             enlsipb200_large* out) {
     if (!out) return lfail(ENLSIPB200_EINVAL, "out is NULL");
     *out = nullptr;
+    const bool want_tsqr = (family & ENLSIPB200_LARGE_FACTOR_TSQR) != 0;
+    family &= ~ENLSIPB200_LARGE_FACTOR_TSQR;
     const GenericVt* gv = nullptr;
 #if defined(ENL_LARGE_USER_FAMILY)
     if (family == ENLSIPB200_FAMILY_USER) gv = generic_vt<LFamUser>();
@@ -1225,8 +1307,12 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
 #endif
     if (gv) {
         if (n < 3) return lfail(ENLSIPB200_EINVAL, "n >= 3 required");
-        if (m_local != gv->m_of(n) || m_global != m_local)
+        if (want_tsqr) {
+            if (m_global != gv->m_of(n) || m_local < 0 || m_local > m_global)
+                return lfail(ENLSIPB200_EINVAL, "row families with ENLSIPB200_LARGE_FACTOR_TSQR: 0 <= m_local <= m_global = the family's m(n)");
+        } else if (m_local != gv->m_of(n) || m_global != m_local) {
             return lfail(ENLSIPB200_EINVAL, "general families are not row-sharded: m_local = m_global = the family's m(n)");
+        }
         nb = 0; ineq = 0; rho = nullptr;
     } else if (n < TS_B || n % TS_B != 0) {
         return lfail(ENLSIPB200_EINVAL, "n must be a positive multiple of 32");
@@ -1250,6 +1336,8 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
     h->sc.set_bounds(x_low, x_upp);
     h->l = h->sc.l(); h->q = h->sc.q();
     h->gv = gv;
+    h->tsqr_rows = gv && want_tsqr;
+    h->rows_joined = !h->tsqr_rows || m_local == m_global;
     if (gv) {
         h->q = gv->q_of(n);
         h->ncu = h->q + gv->ni_of(n);
@@ -1306,7 +1394,11 @@ int enlsipb200_large_comm_id(void* id128) {
 int enlsipb200_large_comm_init(enlsipb200_large hh, const void* id128, int rank, int nranks) {
     LargeHandle* h = LH(hh);
     if (!h || !id128 || nranks < 1 || rank < 0 || rank >= nranks) return lfail(ENLSIPB200_EINVAL, "bad comm arguments");
-    if (nranks == 1) { h->rank = 0; h->nranks = 1; return 0; }
+    if (nranks == 1) {
+        if (h->tsqr_rows && h->m_local != h->m) return lfail(ENLSIPB200_EINVAL, "row shards: one rank must hold all m_global rows");
+        h->rank = 0; h->nranks = 1; h->rows_joined = true;
+        return 0;
+    }
     if (!g_nccl.load()) return lfail(ENLSIPB200_ECUDA, g_nccl.err);
     LCU(cudaSetDevice(h->device));
     NcclApi::UniqueId id;
@@ -1314,6 +1406,29 @@ int enlsipb200_large_comm_init(enlsipb200_large hh, const void* id128, int rank,
     int rc = g_nccl.CommInitRank(&h->comm, nranks, id, rank);
     if (rc != 0) return lfail(ENLSIPB200_ECUDA, std::string("ncclCommInitRank: ") + g_nccl.GetErrorString(rc));
     h->rank = rank; h->nranks = nranks;
+    if (h->tsqr_rows) {   // row shards of a row family: every rank learns every m_local, takes its row0 and checks the total
+        double* dm = nullptr;
+        LCU(cudaMalloc(&dm, sizeof(double) * (nranks + 1)));
+        const double mine = (double)h->m_local;
+        std::vector<double> all(nranks, 0.0);
+        cudaError_t ce = cudaMemcpy(dm + nranks, &mine, sizeof(double), cudaMemcpyHostToDevice);
+        rc = ce == cudaSuccess ? g_nccl.AllGather(dm + nranks, dm, 1, NCCL_FLOAT64, h->comm, nullptr) : 0;
+        if (ce == cudaSuccess && rc == 0) ce = cudaMemcpy(all.data(), dm, sizeof(double) * nranks, cudaMemcpyDeviceToHost);
+        cudaFree(dm);
+        LCU(ce);
+        if (rc != 0) return lfail(ENLSIPB200_ECUDA, std::string("ncclAllGather: ") + g_nccl.GetErrorString(rc));
+        long long below = 0, total = 0;
+        for (int k = 0; k < nranks; ++k) {
+            total += (long long)all[k];
+            if (k < rank) below += (long long)all[k];
+        }
+        // every rank sees the same counts, so every rank refuses together and none waits in a later collective
+        if (total != h->m)
+            return lfail(ENLSIPB200_EINVAL, "row shards: the ranks hold " + std::to_string(total) + " rows, m_global is " +
+                                                std::to_string(h->m));
+        h->row0 = below;
+        h->rows_joined = true;
+    }
     LCU(cudaMalloc(&h->dStack, sizeof(double) * (size_t)nranks * h->rr_rows * h->ld));
     LCU(cudaMalloc(&h->dR2, sizeof(double) * (size_t)h->rr_rows * h->ld));
     {   // the cross-rank stage as one more level of every panel's tree (TsqrDist) needs a 32-row block on every rank
@@ -1321,7 +1436,7 @@ int enlsipb200_large_comm_init(enlsipb200_large hh, const void* id128, int rank,
         LCU(cudaMalloc(&h->dP, sizeof(double) * prow * h->ld));
         LCU(cudaMemset(h->dP, 0, sizeof(double) * prow * h->ld));
         LCU(cudaMalloc(&h->dPscal, sizeof(double) * 2));
-        const double mine = (h->rows_pad < TS_B || h->gv) ? 1.0 : 0.0;
+        const double mine = (h->rows_pad < TS_B || (h->gv && !h->tsqr_rows)) ? 1.0 : 0.0;
         LCU(cudaMemcpy(h->dPscal, &mine, sizeof(double), cudaMemcpyHostToDevice));
         rc = g_nccl.AllReduce(h->dPscal, h->dPscal, 1, NCCL_FLOAT64, NCCL_SUM, h->comm, nullptr);
         if (rc != 0) return lfail(ENLSIPB200_ECUDA, std::string("ncclAllReduce: ") + g_nccl.GetErrorString(rc));
@@ -1348,6 +1463,7 @@ int enlsipb200_large_solve(enlsipb200_large hh, const double* x0, const enlsipb2
     LargeHandle* h = LH(hh);
     if (!h || !x0 || !o || !x || !f) return lfail(ENLSIPB200_EINVAL, "NULL argument");
     if (!h->gv && (!h->dW || !h->dy)) return lfail(ENLSIPB200_EINVAL, "family data (W, y) not set");
+    if (!h->rows_joined) return lfail(ENLSIPB200_EINVAL, "row shard (m_local < m_global) not joined: enlsipb200_large_comm_init first");
     h->jac_fd = (o->jac_mode == ENLSIPB200_JAC_FORWARD_DIFF) ? 1 : 0;
     if (h->jac_fd && !h->gv && h->n > 3072)
         return lfail(ENLSIPB200_EINVAL, "forward-difference Jacobians of the single-index family: n <= 3072 (x and the steps are staged in 48 KB of shared memory)");
@@ -1398,6 +1514,7 @@ int enlsipb200_large_factor(enlsipb200_large hh, const double* x, double* R, flo
     LargeHandle* h = LH(hh);
     if (!h || !x) return lfail(ENLSIPB200_EINVAL, "NULL argument");
     if (!h->gv && (!h->dW || !h->dy)) return lfail(ENLSIPB200_EINVAL, "family data (W, y) not set");
+    if (!h->rows_joined) return lfail(ENLSIPB200_EINVAL, "row shard (m_local < m_global) not joined: enlsipb200_large_comm_init first");
     int rc = h->factor_at(x);
     if (rc != 0) return rc;
     const int nc = h->n + 1;

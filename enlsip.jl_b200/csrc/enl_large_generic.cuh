@@ -3,6 +3,8 @@
 // cons_eval! / jaccons_eval! (src/cnls_model.jl:40-62) and of jac_forward_diff (src/cnls_model.jl:65-82) when the
 // problem is not the single-index family with its specialised kernels (enl_large.cu).  [J | r] is built column major
 // (m x (n+1)) and factored by the plain-Householder mode of qrcp_device (enl_small.cuh); a copy of J serves J p.
+// With ENLSIPB200_LARGE_FACTOR_TSQR the family builds the TSQR's row-major work matrix instead (lg_build_rows_kernel:
+// [J | 0 | r], n padded to a multiple of 32) and J p comes from a row-major copy of J (lg_dir_rows_kernel).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -58,6 +60,70 @@ __global__ void __launch_bounds__(256) lg_build_kernel(int n, long long m, const
     }
 }
 
+// TSQR work matrix (rows_pad x ld, row major): one warp per row, lanes over the columns (coalesced stores).  Row i holds
+// [J_i | 0 | r_i | 0]: J in columns 0..n-1, zeros up to column nt - 1 (nt = n rounded up to 32), r in column nt, zeros up
+// to ld - 1; rows m..rows_pad-1 are all zero.  Every entry of the row is rewritten at each point, so nothing the previous
+// factorisation left in the matrix survives.  Entries of J by the arithmetic of lg_build_kernel; the family sees the
+// global row row0 + i.  Jrow: row-major m x n copy of J for the direction products.
+template <class F>
+__global__ void __launch_bounds__(256) lg_build_rows_kernel(int n, long long m, long long rows_pad, long long row0,
+                                                            const double* __restrict__ x, const double* __restrict__ d0,
+                                                            const double* __restrict__ d1, int fd, int nt, int ld,
+                                                            double* __restrict__ A, double* __restrict__ Jrow,
+                                                            double* __restrict__ r_out) {
+    const int lane = threadIdx.x & 31;
+    const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long i = warp0; i < rows_pad; i += nwarps) {
+        double* ar = A + i * ld;
+        if (i >= m) {
+            for (int j = lane; j < ld; j += 32) ar[j] = 0.0;
+            continue;
+        }
+        const long long gi = row0 + i;
+        const double ri = F::residual(gi, n, XPlain{x}, d0, d1);
+        double* jr = Jrow + i * n;
+        for (int j = lane; j < ld; j += 32) {
+            double v = 0.0;
+            if (j < n) {
+                if (fd || !F::HAS_JAC) {
+                    const double dj = __dmul_rn(fmax(fabs(x[j]), 1.0), G_SQRT_EPS);
+                    v = __ddiv_rn(__dsub_rn(F::residual(gi, n, XPert{x, j, dj}, d0, d1), ri), dj);
+                } else {
+                    v = F::jac_residual(gi, j, n, x, d0, d1);
+                }
+                jr[j] = v;
+            } else if (j == nt) {
+                v = ri;
+            }
+            ar[j] = v;
+        }
+        if (lane == 0) r_out[i] = ri;
+    }
+}
+
+// Jp = J p from the row-major copy of J (one warp per row) and the sums {r.r, r.Jp, Jp.Jp, 0}
+__global__ void __launch_bounds__(256) lg_dir_rows_kernel(const double* __restrict__ J, int n, long long m,
+                                                          const double* __restrict__ p, const double* __restrict__ r,
+                                                          double* __restrict__ Jp, double* __restrict__ part) {
+    const int lane = threadIdx.x & 31;
+    const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+    double sums[4] = {0.0, 0.0, 0.0, 0.0};
+    for (long long i = warp0; i < m; i += nwarps) {
+        const double* jr = J + i * n;
+        double acc = 0.0;
+        for (int j = lane; j < n; j += 32) acc = fma(jr[j], p[j], acc);
+        const double jp = g_warp_sum(acc);
+        if (lane == 0) {
+            const double ri = r[i];
+            Jp[i] = jp;
+            sums[0] = fma(ri, ri, sums[0]); sums[1] = fma(ri, jp, sums[1]); sums[2] = fma(jp, jp, sums[2]);
+        }
+    }
+    g_block_reduce4(sums, part);
+}
+
 // sums {r.r, r.Jp, Jp.Jp, 0} for the direction just set
 __global__ void __launch_bounds__(256) lg_dir_sums_kernel(const double* __restrict__ r, const double* __restrict__ Jp, long long m,
                                                           double* __restrict__ part) {
@@ -71,14 +137,14 @@ __global__ void __launch_bounds__(256) lg_dir_sums_kernel(const double* __restri
 
 // trial point x + alpha p: partial sums {r_a.r_a, r.v2, Jp.v2, v2.v2}, v2 = ((r_a - r)/alpha - Jp)/alpha  (EF:1687)
 template <class F>
-__global__ void __launch_bounds__(256) lg_ls_kernel(int n, long long m, const double* __restrict__ x, const double* __restrict__ p,
+__global__ void __launch_bounds__(256) lg_ls_kernel(int n, long long m, long long row0, const double* __restrict__ x, const double* __restrict__ p,
                                                     double alpha, const double* __restrict__ d0, const double* __restrict__ d1,
                                                     const double* __restrict__ r, const double* __restrict__ Jp, int with_coeffs,
                                                     double* __restrict__ part) {
     double sums[4] = {0.0, 0.0, 0.0, 0.0};
     const XStep xs{x, p, alpha};
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (long long)gridDim.x * blockDim.x) {
-        const double ra = F::residual(i, n, xs, d0, d1);
+        const double ra = F::residual(row0 + i, n, xs, d0, d1);
         sums[0] = fma(ra, ra, sums[0]);
         if (with_coeffs) {
             const double ri = r[i], jp = Jp[i];
@@ -120,8 +186,10 @@ struct GenericVt {
     int (*q_of)(int);
     int (*ni_of)(int);
     void (*build)(int grid, cudaStream_t st, int n, long long m, const double* x, const double* d0, const double* d1, int fd, double* Q, double* r);
-    void (*ls)(int grid, cudaStream_t st, int n, long long m, const double* x, const double* p, double alpha, const double* d0,
-               const double* d1, const double* r, const double* Jp, int with_coeffs, double* part);
+    void (*build_rows)(int grid, cudaStream_t st, int n, long long m, long long rows_pad, long long row0, const double* x,
+                       const double* d0, const double* d1, int fd, int nt, int ld, double* A, double* Jrow, double* r);
+    void (*ls)(int grid, cudaStream_t st, int n, long long m, long long row0, const double* x, const double* p, double alpha,
+               const double* d0, const double* d1, const double* r, const double* Jp, int with_coeffs, double* part);
     void (*cons)(cudaStream_t st, int n, int nc, const double* x, const double* d0, const double* d1, double* c);
     void (*jac_cons)(cudaStream_t st, int n, int nc, const double* x, const double* d0, const double* d1, int fd, const double* c0, double* Arow);
 };
@@ -132,9 +200,13 @@ const GenericVt* generic_vt() {
         [](int grid, cudaStream_t st, int n, long long m, const double* x, const double* d0, const double* d1, int fd, double* Q, double* r) {
             lg_build_kernel<F><<<grid, 256, 0, st>>>(n, m, x, d0, d1, fd, Q, r);
         },
-        [](int grid, cudaStream_t st, int n, long long m, const double* x, const double* p, double alpha, const double* d0,
-           const double* d1, const double* r, const double* Jp, int with_coeffs, double* part) {
-            lg_ls_kernel<F><<<grid, 256, 0, st>>>(n, m, x, p, alpha, d0, d1, r, Jp, with_coeffs, part);
+        [](int grid, cudaStream_t st, int n, long long m, long long rows_pad, long long row0, const double* x, const double* d0,
+           const double* d1, int fd, int nt, int ld, double* A, double* Jrow, double* r) {
+            lg_build_rows_kernel<F><<<grid, 256, 0, st>>>(n, m, rows_pad, row0, x, d0, d1, fd, nt, ld, A, Jrow, r);
+        },
+        [](int grid, cudaStream_t st, int n, long long m, long long row0, const double* x, const double* p, double alpha,
+           const double* d0, const double* d1, const double* r, const double* Jp, int with_coeffs, double* part) {
+            lg_ls_kernel<F><<<grid, 256, 0, st>>>(n, m, row0, x, p, alpha, d0, d1, r, Jp, with_coeffs, part);
         },
         [](cudaStream_t st, int n, int nc, const double* x, const double* d0, const double* d1, double* c) {
             if (nc > 0) lg_cons_kernel<F><<<(nc + 127) / 128, 128, 0, st>>>(n, nc, x, d0, d1, c);

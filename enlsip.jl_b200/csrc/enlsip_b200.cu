@@ -736,8 +736,8 @@ int enlsipb200_large_compile_family(const char* source, long long m, int nb_eq, 
     if (!fp) return fail(ENLSIPB200_EINVAL, "cannot write " + pre);
     fprintf(fp, "// generated by enlsipb200_large_compile_family\n#pragma once\n#define ENL_LARGE_USER_FAMILY 1\n"
                 "#define ENL_LUSER_M %lldLL\n#define ENL_LUSER_Q %d\n#define ENL_LUSER_NI %d\n#define ENL_LUSER_HAS_JAC %d\n"
-                "#include <cuda_runtime.h>\n#include <math.h>\n#line 1 \"user_family_source\"\n%s\n",
-            m, nb_eq, nb_ineq, has_jacobians ? 1 : 0, source);
+                "#include <cuda_runtime.h>\n#include <math.h>\n#include \"%s/enl_base.h\"\n#line 1 \"user_family_source\"\n%s\n",
+            m, nb_eq, nb_ineq, has_jacobians ? 1 : 0, csrc.c_str(), source);
     fclose(fp);
     const std::string log = wd + "/enl_large_user_build.log";
     const char* nvcc = getenv("ENLSIP_NVCC");

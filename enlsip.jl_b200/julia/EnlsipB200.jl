@@ -167,6 +167,7 @@ total_nb_constraints(model::CnlsModel) = model.nb_constraints                   
 # ---------------------------------------------------------------------------------------------------
 const FAMILY_SINGLE_INDEX = Cint(16)
 const FAMILY_LARGE_CHAINED_ROSENBROCK = Cint(17)
+const LARGE_FACTOR_TSQR = Cint(0x100)      # OR-ed into the family of a row family: TSQR of [J | r], row sharding
 
 """
     large_compile_family(source; m, nb_eqcons=0, nb_ineqcons=0, has_jacobians=false) -> library handle
@@ -231,31 +232,48 @@ function LargeCnlsModel(family::Symbol, starting_point::Vector{Float64}; W::Matr
 end
 
 """
-    LargeCnlsModel(:chained_rosenbrock, starting_point; x_low, x_upp, jacobian=:analytic)
-    LargeCnlsModel(lib, starting_point; m, nb_eqcons=0, nb_ineqcons=0, data=(), x_low, x_upp, jacobian=:forward_diff)
+    LargeCnlsModel(:chained_rosenbrock, starting_point; x_low, x_upp, jacobian=:analytic, factor=:householder, shard=nothing)
+    LargeCnlsModel(lib, starting_point; m, nb_eqcons=0, nb_ineqcons=0, data=(), x_low, x_upp, jacobian=:forward_diff,
+                   factor=:householder, shard=nothing)
 
 General row families: the reference's own chained Rosenbrock test (test/problems/chained_rosenbrock.jl, any n; the
 reference runs n = 1000), or a user family compiled by `large_compile_family`.  `data`: up to two Float64 arrays
-handed to the family's functions (copied to the device here).
+handed to the family's functions (copied to the device here; whole on every rank).  `factor=:tsqr` compresses [J | r]
+with the tall-skinny QR (LARGE_FACTOR_TSQR); with it, `shard=(rank, nranks)` gives this process the rows of
+`shard_rows(m, rank, nranks)`, after which every rank calls `join!`.
 """
 function LargeCnlsModel(family::Symbol, starting_point::Vector{Float64}; x_low=fill(-Inf, length(starting_point)),
-                        x_upp=fill(Inf, length(starting_point)), jacobian::Symbol=:analytic, device::Integer=-1)
+                        x_upp=fill(Inf, length(starting_point)), jacobian::Symbol=:analytic, device::Integer=-1,
+                        factor::Symbol=:householder, shard=nothing)
     family === :chained_rosenbrock || error("row families: :chained_rosenbrock, or a library from large_compile_family")
     n = length(starting_point)
     return _row_family_model(C_NULL, FAMILY_LARGE_CHAINED_ROSENBROCK, starting_point, 2 * (n - 1), n - 2, 0, (), x_low, x_upp,
-                             jacobian, device)
+                             jacobian, device, factor, shard)
 end
 LargeCnlsModel(lib::Ptr{Cvoid}, starting_point::Vector{Float64}; m::Integer, nb_eqcons::Integer=0, nb_ineqcons::Integer=0,
                data=(), x_low=fill(-Inf, length(starting_point)), x_upp=fill(Inf, length(starting_point)),
-               jacobian::Symbol=:forward_diff, device::Integer=-1) =
-    _row_family_model(lib, FAMILY_USER, starting_point, m, nb_eqcons, nb_ineqcons, data, x_low, x_upp, jacobian, device)
+               jacobian::Symbol=:forward_diff, device::Integer=-1, factor::Symbol=:householder, shard=nothing) =
+    _row_family_model(lib, FAMILY_USER, starting_point, m, nb_eqcons, nb_ineqcons, data, x_low, x_upp, jacobian, device,
+                      factor, shard)
 
-function _row_family_model(lib, fam, starting_point, m, q, ni, data, x_low, x_upp, jacobian, device)
+"Rows (row0, rows) of `rank` among `nranks` shards of m rows: multiples of 256 (one level-0 TSQR subtile), the last rank takes the remainder."
+function shard_rows(m::Integer, rank::Integer, nranks::Integer)
+    0 <= rank < nranks || error("shard must be (rank, nranks) with 0 <= rank < nranks")
+    chunk = max(256, div(div(m, nranks), 256) * 256)
+    row0 = min(rank * chunk, m)
+    return row0, rank == nranks - 1 ? m - row0 : min(chunk, m - row0)
+end
+
+function _row_family_model(lib, fam, starting_point, m, q, ni, data, x_low, x_upp, jacobian, device, factor=:householder,
+                           shard=nothing)
+    factor in (:householder, :tsqr) || error("factor must be :householder or :tsqr")
+    shard === nothing || factor === :tsqr || error("shard=(rank, nranks) needs factor=:tsqr")
     n = length(starting_point)
+    rows = shard === nothing ? m : shard_rows(m, shard...)[2]
     h = Ref{Ptr{Cvoid}}(C_NULL)
     checkl(ccall(fsym(lib, :enlsipb200_large_create), Cint,
                  (Cint, Cint, Clonglong, Clonglong, Cint, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Cint, Ptr{Ptr{Cvoid}}),
-                 fam, n, m, m, 0, 0, C_NULL, x_low, x_upp, Cint(device), h))
+                 factor === :tsqr ? fam | LARGE_FACTOR_TSQR : fam, n, rows, m, 0, 0, C_NULL, x_low, x_upp, Cint(device), h))
     for (slot, arr) in enumerate(data)      # copied host -> device inside the call: nothing to keep alive
         checkl(ccall(fsym(lib, :enlsipb200_large_set_data), Cint, (Ptr{Cvoid}, Cint, Ptr{Cdouble}, Clonglong, Cint),
                      h[], Cint(slot - 1), arr, length(arr), Cint(0)))

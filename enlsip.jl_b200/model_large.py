@@ -11,6 +11,9 @@ status / solution / sum_sq_residuals        same accessors (cnls_model.jl:206-22
 Row sharding over the GPUs of one box (BASELINE.json config 4): one process per GPU, each builds a model
 from its own rows and calls ``model.join(rank, world)`` once (NCCL unique id broadcast through
 ``torch.distributed``); afterwards every rank calls ``solve`` with identical arguments and gets identical results.
+Row families (chained Rosenbrock, LargeUserFamily) compress [J | r] by a plain Householder QR of the column-major matrix
+unless ``factor="tsqr"``: then they take the single-index family's tall-skinny QR, and ``shard=(rank, world)`` gives this
+process its slice of the rows (``shard_rows``) before ``join(rank, world)``.  Data slots stay whole on every rank.
 There is no CPU execution path.
 """
 from __future__ import annotations
@@ -32,6 +35,20 @@ _ROW_FAMILIES = {
 }
 
 
+SHARD_ALIGN = 256       # rows of one level-0 subtile of the TSQR tree (8 blocks of 32)
+
+
+def shard_rows(m, rank, world):
+    """(row0, rows) of `rank` among `world` shards of m rows: equal slices in multiples of SHARD_ALIGN, the last rank
+    takes the remainder (ranks past the end of a small problem hold no rows)."""
+    if world < 1 or not 0 <= rank < world:
+        raise ValueError("shard must be (rank, world) with 0 <= rank < world")
+    chunk = max(SHARD_ALIGN, (m // world) // SHARD_ALIGN * SHARD_ALIGN)
+    row0 = min(rank * chunk, m)
+    rows = m - row0 if rank == world - 1 else min(chunk, m - row0)
+    return row0, rows
+
+
 class LargeUserFamily:
     """A problem of the large regime defined by user CUDA source: the replacement of the reference's closure arguments
     (residuals, eq_constraints, ineq_constraints, jacobian_*; cnls_model.jl:345-359) when n + m >= 1000.  `source` defines
@@ -50,9 +67,15 @@ class LargeUserFamily:
 
 class LargeCnlsModel:
     def __init__(self, family, starting_point, data=None, ineq=False, x_low=None, x_upp=None, m_global=None, device=-1,
-                 jacobian="analytic"):
+                 jacobian="analytic", factor="householder", shard=None):
         if jacobian not in ("analytic", "forward_diff"):
             raise AssertionError("jacobian must be 'analytic' or 'forward_diff'")
+        if factor not in ("householder", "tsqr"):
+            raise AssertionError("factor must be 'householder' or 'tsqr'")
+        if shard is not None and factor != "tsqr":
+            raise AssertionError("shard=(rank, world) needs factor='tsqr'")
+        self.factor_mode, self.shard = factor, shard
+        self._flag = capi.LARGE_FACTOR_TSQR if factor == "tsqr" else 0
         self.jacobian = jacobian
         self.family = family
         self.B = 1
@@ -87,7 +110,7 @@ class LargeCnlsModel:
         self.nb_constraints = nb + int(np.isfinite(self.x_low).sum()) + int(np.isfinite(self.x_upp).sum())
         self.lmax = self.nb_constraints
         h = ctypes.c_void_p()
-        capi.check_large(self._lib.enlsipb200_large_create(capi.FAMILY_SINGLE_INDEX, n, rows, self.nb_residuals, nb,
+        capi.check_large(self._lib.enlsipb200_large_create(capi.FAMILY_SINGLE_INDEX | self._flag, n, rows, self.nb_residuals, nb,
                                                             1 if ineq else 0, rho.ctypes.data, self.x_low.ctypes.data,
                                                             self.x_upp.ctypes.data, device, ctypes.byref(h)), self._lib)
         self._h = h
@@ -98,14 +121,15 @@ class LargeCnlsModel:
     def _init_row_family(self, fam_id, n, m, q, ni, keys, data, x_low, x_upp, device):
         """A general family: residual rows / constraints as device functions of the point (csrc/enl_large_family.h), the
         counterpart of CnlsModel(residuals, n, m; eq_constraints, nb_eqcons, ...) for an arbitrary model."""
-        self.nb_parameters, self.rows, self.nb_residuals = n, m, m
+        self.row0, self.rows = (0, m) if self.shard is None else shard_rows(m, *self.shard)
+        self.nb_parameters, self.nb_residuals = n, m
         self.x_low = np.full(n, -np.inf) if x_low is None else np.ascontiguousarray(x_low, dtype=np.float64)
         self.x_upp = np.full(n, np.inf) if x_upp is None else np.ascontiguousarray(x_upp, dtype=np.float64)
         self.nb_eqcons = q
         self.nb_constraints = q + ni + int(np.isfinite(self.x_low).sum()) + int(np.isfinite(self.x_upp).sum())
         self.lmax = self.nb_constraints
         h = ctypes.c_void_p()
-        capi.check_large(self._lib.enlsipb200_large_create(fam_id, n, m, m, 0, 0, None, self.x_low.ctypes.data,
+        capi.check_large(self._lib.enlsipb200_large_create(fam_id | self._flag, n, self.rows, m, 0, 0, None, self.x_low.ctypes.data,
                                                             self.x_upp.ctypes.data, device, ctypes.byref(h)), self._lib)
         self._h = h
         for slot, key in enumerate(keys):

@@ -153,7 +153,8 @@ ENLSIPB200_API int enlsipb200_compile_family(const char* source, int n, int m, i
  * and, if has_jacobians != 0,
  *     __device__ double jac_residual(long long i, int j, int n, const double* x, const double* d0, const double* d1);
  *     __device__ double jac_constraint(int k, int j, int n, const double* x, const double* d0, const double* d1);
- * (entry (i, j) of the dense Jacobian).  d0 / d1: the two data slots of enlsipb200_large_set_data (any length).
+ * (entry (i, j) of the dense Jacobian).  d0 / d1: the two data slots of enlsipb200_large_set_data (any length).  The
+ * helpers of csrc/enl_base.h are visible in namespace enl (enl::det_tanh, ...); ENL_LUSER_M holds m.
  * The resulting library exports the enlsipb200_large_* API; create the handle with family = ENLSIPB200_FAMILY_USER,
  * m_local = m_global = m, any n >= 3 (nb / ineq / rho ignored), bounds through x_low / x_upp.  Without Jacobians the
  * solve differentiates by forward differences (cnls_model.jl:65-82). */
@@ -181,9 +182,19 @@ ENLSIPB200_API int enlsipb200_det_exp(const double* x, double* y, long long n, i
 
 #define ENLSIPB200_FAMILY_LARGE_CHAINED_ROSENBROCK 17 /* test/problems/chained_rosenbrock.jl:8-53 at ANY n (the reference
                                              runs n = 1000: m = 2(n-1) = 1998 residuals, q = n-2 = 998 nonlinear
-                                             equalities); a general "row family": no restriction on n, not row-sharded
-                                             (m_local = m_global = 2(n-1); nb / ineq / rho are ignored); analytic or
-                                             forward-difference Jacobians (opt->jac_mode)                              */
+                                             equalities); a general "row family": no restriction on n; analytic or
+                                             forward-difference Jacobians (opt->jac_mode); nb / ineq / rho are ignored.
+                                             m_local = m_global = 2(n-1), unless ENLSIPB200_LARGE_FACTOR_TSQR is set:
+                                             then the rows may be sharded (m_local <= m_global)                       */
+
+/* OR-ed into `family` of enlsipb200_large_create.  Row families (built-in or ENLSIPB200_FAMILY_USER) then build [J | r]
+ * row major, with n padded to a multiple of 32 by zero columns, and compress it with the tall-skinny QR of the
+ * single-index family instead of the plain Householder QR of a column-major [J | r].  The rows may then be sharded over
+ * GPUs: each rank passes its own m_local <= m_global = m(n) rows, enlsipb200_large_comm_init places the shards in rank
+ * order (row0 = the rows of the lower ranks) and refuses, on every rank, a total other than m_global.  Data slots stay
+ * whole on every rank and the family is called with global row indices.  The single-index family accepts the flag and
+ * ignores it. */
+#define ENLSIPB200_LARGE_FACTOR_TSQR 0x100
 
 typedef struct enlsipb200_large_s* enlsipb200_large;
 
@@ -198,7 +209,8 @@ ENLSIPB200_API int enlsipb200_large_destroy(enlsipb200_large h);
 /* slot 0 = W [m_local, n] row major, slot 1 = y [m_local].  on_device != 0: device pointer that must stay
  * valid (and resident on the handle's device) for the solves; otherwise copied host -> device. */
 ENLSIPB200_API int enlsipb200_large_set_data(enlsipb200_large h, int slot, const double* ptr, long long count, int on_device);
-/* multi-GPU: rank 0 creates a 128-byte NCCL unique id, the host layer distributes it, every rank joins */
+/* multi-GPU: rank 0 creates a 128-byte NCCL unique id, the host layer distributes it, every rank joins.  A row family
+ * created with ENLSIPB200_LARGE_FACTOR_TSQR and m_local < m_global must join before its first solve or factor. */
 ENLSIPB200_API int enlsipb200_large_comm_id(void* id128);
 ENLSIPB200_API int enlsipb200_large_comm_init(enlsipb200_large h, const void* id128, int rank, int nranks);
 /* blocking solve; outputs as in enlsipb200_solve_batch for B = 1 (active [l], trace [trace_cap, TRACE_HDR + n]) */
