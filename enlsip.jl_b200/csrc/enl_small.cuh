@@ -462,28 +462,10 @@ __global__ void __launch_bounds__(256) qr_panel_gemv_kernel(const double* __rest
         for (int j = j0 + tid; j <= jc; j += blockDim.x) F[(size_t)j * QR_NB + k] = 0.0;
 }
 
-// Trailing update of a finished panel (kb = stt->k columns): A(j0+kb:, j0+kb:) -= A(j0+kb:, j0:j0+kb) F(j0+kb:, 0:kb)'
-__global__ void __launch_bounds__(256) qr_panel_trail_kernel(double* __restrict__ f, int rows, int cols,
-                                                             const double* __restrict__ F, const QrState* stt) {
-    __shared__ double As[32][65];
-    __shared__ double Bs[32][65];
-    if (!stt->active) return;
-    const int j0 = stt->j0, kb = stt->k;
-    if (kb <= 0) return;
-    const int r0 = j0 + kb, c0 = j0 + kb;
-    const int M = rows - r0, N = cols - c0;
-    if (M <= 0 || N <= 0) return;
-    const double* A = f + (size_t)j0 * rows + r0;          // M x kb, lda = rows
-    const double* B = F + (size_t)c0 * QR_NB;               // F(c0:, 0:kb)' = kb x N column major, ldb = QR_NB
-    double* C = f + (size_t)c0 * rows + r0;
-    const int tmn = (M + 63) / 64, tnn = (N + 63) / 64;
-    for (int t = blockIdx.x; t < tmn * tnn; t += gridDim.x)
-        gemm_tile<false>(A, rows, B, QR_NB, C, rows, M, N, kb, -1.0, 1.0, t % tmn, t / tmn, As, Bs);
-}
-
-// The same rank-kb update on the FP64 FMA pipe with coalesced accesses to the trailing matrix (default).  At K = 32 the
-// update is bound by reading and writing C (2 x 8 bytes against 64 flops per element), not by the tensor pipe, and the
-// DMMA fragment layout touches C in 8 x 8 patches (half-used sectors; measured 1.0 TB/s, profiles/r2_qr_panel_trail_ncu.txt).
+// Trailing update of a finished panel (kb = stt->k columns): A(j0+kb:, j0+kb:) -= A(j0+kb:, j0:j0+kb) F(j0+kb:, 0:kb)',
+// on the FP64 FMA pipe with coalesced accesses to the trailing matrix.  At K = 32 the update is bound by reading and
+// writing C (2 x 8 bytes against 64 flops per element), not by the tensor pipe, and a DMMA tile form touches C in 8 x 8
+// patches (half-used sectors; measured 1.0 TB/s, profiles/r2_qr_panel_trail_ncu.txt).
 // Here a thread owns one row of a 128 x 32 tile (its 32 panel entries in registers) and 16 of its columns; the lanes of
 // a warp are 32 consecutive rows of one column (256-byte segments), F is read from shared memory as 16-byte broadcasts.
 constexpr int QT_ROWS = 128, QT_COLS = 32;
@@ -1268,12 +1250,6 @@ struct QrWork {          // scratch of one factorisation (sized for the largest 
     }
 };
 
-// trailing update of a finished panel: FMA kernel with coalesced C accesses (default) or the DMMA tile kernel (ENLSIP_QR_TRAIL=dmma)
-inline void qr_launch_trail(double* f, int rows, int cols, QrWork& wk, cudaStream_t st) {
-    static const bool dmma = [] { const char* e = getenv("ENLSIP_QR_TRAIL"); return e && e[0] == 'd'; }();
-    if (dmma) qr_panel_trail_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F, wk.state);
-    else qr_panel_trail_fma_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F, wk.state);
-}
 // grid of the persistent panel kernel (one CTA per SM, co-resident: cooperative launch); 0 = not available
 inline int qp_grid() {
     static const int g = [] {
@@ -1306,7 +1282,7 @@ inline int qr_enqueue_panel_persist(double* f, int rows, int cols, double* tau, 
     unsigned int* bar = wk.ticket + 1;
     void* args[] = {&f, &rows, &cols, &vn1, &vn2, &jpvt, &tau, &F, &flags, &stt, &pbest, &pidx, &pany, &ppart, &bar};
     cudaLaunchCooperativeKernel((const void*)qr_panel_persist_kernel, dim3(G), dim3(QP_THREADS), args, qp_smem_bytes(rows, G), st);
-    qr_launch_trail(f, rows, cols, wk, st);
+    qr_panel_trail_fma_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F, wk.state);
     qr_panel_close_kernel<<<148, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, wk.flags, wk.state, topbmn, wk.ticket);
     return 3;
 }
@@ -1322,7 +1298,7 @@ inline int qr_enqueue_panel(double* f, int rows, int cols, double* tau, int* jpv
         launches += 3;
     }
     qr_panel_finish_pivot_kernel<<<g_fin, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, jpvt, wk.F, wk.auxv, wk.flags, wk.state, wk.pbest, wk.pidx, QR_NB);
-    qr_launch_trail(f, rows, cols, wk, st);
+    qr_panel_trail_fma_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F, wk.state);
     qr_panel_close_kernel<<<148, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, wk.flags, wk.state, topbmn, wk.ticket);
     return launches + 3;
 }

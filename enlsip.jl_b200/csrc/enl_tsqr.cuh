@@ -9,15 +9,14 @@
 //   for each 32-column panel j:
 //     level 0, 1, 2, ...: the rows are cut into blocks of 32; a "subtile" is 8 blocks (stride 8^level
 //       blocks apart, i.e. at level >= 1 the top blocks of the subtiles of the level below).
-//       tsqr_panel_kernel  : one CTA per subtile; Householder QR of its 256 x 32 panel held in
-//                            registers (lane = column, 8 warps x 32 rows), ONE block barrier per column
-//                            (a single pass of dot products with the raw pivot column gives the norm and every
-//                            v_i . a_c); compact-WY T = (striu(V'V) + diag(1/tau))^-1; V is stored in place, T
-//                            in a side buffer; the residual column of [J | r] is updated here as well
-//                            (b <- (I - V T' V') b with the reflectors still in registers)
-//       tsqr_trail_kernel  : one CTA per (subtile, 32-column block of the trailing matrix):
-//                            B <- (I - V T' V')B with three FP64 tensor-core products
-//                            (mma.sync.m8n8k4.f64 = DMMA.8x8x4): G = V'B, W = -T'G, B += V W
+//       tsqr_panel_cg_kernel     : one CTA per subtile; Householder QR of its 256 x 32 panel held in
+//                                  registers (warp w = columns 4w..4w+3 of all 256 rows), ONE block barrier per
+//                                  column; compact-WY T = (striu(V'V) + diag(1/tau))^-1; V is stored in place, T
+//                                  in a side buffer; the residual column of [J | r] is updated here as well
+//                                  (b <- (I - V T' V') b with the reflectors still in registers)
+//       tsqr_trail_staged_kernel : one CTA per (subtile, chunk of 32-column blocks of the trailing matrix):
+//                                  B <- (I - V T' V')B with three FP64 tensor-core products
+//                                  (mma.sync.m8n8k4.f64 = DMMA.8x8x4): G = V'B, W = -T'G, B += V W
 //     the top 32 rows of the last level are the finished rows 32j..32j+31 of R: copied out, then
 //     zeroed in place so later panels see them as empty rows.
 //   after the last panel the residual column only needs its norm (R[n][n]).
@@ -25,21 +24,12 @@
 // price is 1/7 more flops than a flat tree (each level re-factors 1/8 of the rows).
 // Algorithmic flops: 2 m n^2 (n = number of columns).  See DESIGN.md for the roofline accounting.
 #pragma once
-#include <cuda.h>
 #include <cuda_runtime.h>
-#include <cudaTypedefs.h>
-#include <stdlib.h>
 
 namespace enl_large {
 
 constexpr int TS_B = 32;     // block rows = panel width
 constexpr int TS_FAN = 8;    // blocks per subtile
-constexpr int TS_CG = 4;     // panel columns per unrolled group (code size: the group body must stay in the 32 KB L1.5 I-cache)
-constexpr int TS_KEEP = 12;   // published-column entries kept in registers between the dot and the update pass
-#ifndef TS_TRAIL_CB
-#define TS_TRAIL_CB 32
-#endif
-constexpr int TS_LDS = 36;   // shared-memory leading dimension (doubles): conflict-free m8n8k4 fragment loads
 
 __device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
     asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
@@ -48,224 +38,22 @@ __device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double
 }
 
 // ---------------------------------------------------------------------------------------------
-// panel factorisation of one subtile
+// panel factorisation of one subtile: warp w owns columns 4w..4w+3 of all 256 rows of the subtile
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256, 2)
-tsqr_panel_kernel(double* __restrict__ A, int ld, long long nblk, long long stride, int col0, int upper_only,
-                  int rcol, double* __restrict__ Tbuf) {
-    // One block-wide barrier per column: the raw column i is published (per warp), ONE pass of dot products
-    // g_c = sum_{rows below the pivot} a_i[r] a_c[r] gives both the norm (g_i) and, because the reflector
-    // v_i = e_i + scale * a_i[below] is linear in the raw column, every v_i . a_c = a_c[i] + scale * g_c.
-    __shared__ __align__(16) double vbuf[TS_FAN][TS_B];
-    __shared__ double dots[2][TS_FAN][TS_B];
-    __shared__ double rowi[2][TS_B];        // row i of the top block (warp 0), double-buffered like dots
-    __shared__ double Gs[TS_B][TS_B + 1];   // Gs[c][i] = v_c . v_i, c < i
-    __shared__ double taus[TS_B];
-    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long long sub = blockIdx.x;
-    const long long blk = (sub * TS_FAN + w) * stride;
-    const bool valid = blk < nblk;
-    double* base = A + (blk * TS_B) * (long long)ld + col0 + lane;
-    double a[TS_B];
-    double myscale = 0.0;   // scale of this lane's own reflector (set when its column is the pivot)
-    // the residual column of [J | r] (column rcol): lane = row here; updated at the end of this kernel with the
-    // block reflector of the panel, so the trailing-update kernel only sees full 32-column blocks
-    double* bptr = A + (blk * TS_B + lane) * (long long)ld + rcol;
-    double bval = (valid && rcol >= 0) ? *bptr : 0.0;
-#pragma unroll
-    for (int r = 0; r < TS_B; ++r) {
-        double v = valid ? base[(long long)r * ld] : 0.0;
-        if (upper_only && r > lane) v = 0.0;   // level >= 1: below the diagonal lie stale reflectors of the level below
-        a[r] = v;
-    }
-    // Columns are processed in groups of TS_CG: the group body is unrolled (compile-time register indices), the
-    // loop over groups is not (the fully unrolled kernel is 160 KB of code and starves on instruction fetch).
-    // After a group the top block (warp 0) stores its TS_CG finished rows and zeroes them, and every warp rotates
-    // its register rows by TS_CG, so that the pivot rows of the next group are again rows 0..TS_CG-1.
-#pragma unroll 1
-    for (int ib = 0; ib < TS_B / TS_CG; ++ib) {
-#pragma unroll
-        for (int k = 0; k < TS_CG; ++k) {
-            const int i = ib * TS_CG + k;
-            const int buf = k & 1;
-            __syncwarp();
-            // (1) lane i publishes its raw column (pivot row and the rows above it masked in the top block)
-            if (lane == i) {
-#pragma unroll
-                for (int r = 0; r < TS_B; r += 2) {
-                    double2 v = make_double2(a[r], a[r + 1]);
-                    if (w == 0) {
-                        if (r <= k) v.x = 0.0;
-                        if (r + 1 <= k) v.y = 0.0;
-                    }
-                    *reinterpret_cast<double2*>(&vbuf[w][r]) = v;
-                }
-            }
-            if (w == 0) rowi[buf][lane] = a[k];
-            __syncwarp();
-            // (2) g_c over this warp's 32 rows; the first TS_KEEP entries of the published column stay in registers for
-            // step (3) (the kernel is bound by shared-memory loads: every kept value saves one 16-byte broadcast load)
-            double vk[TS_KEEP];
-            double d0 = 0.0, d1 = 0.0, d2 = 0.0, d3 = 0.0;
-#pragma unroll
-            for (int r = 0; r < TS_B; r += 4) {
-                const double2 v01 = *reinterpret_cast<const double2*>(&vbuf[w][r]);
-                const double2 v23 = *reinterpret_cast<const double2*>(&vbuf[w][r + 2]);
-                if (r < TS_KEEP) { vk[r] = v01.x; vk[r + 1] = v01.y; vk[r + 2] = v23.x; vk[r + 3] = v23.y; }
-                d0 = fma(v01.x, a[r + 0], d0); d1 = fma(v01.y, a[r + 1], d1);
-                d2 = fma(v23.x, a[r + 2], d2); d3 = fma(v23.y, a[r + 3], d3);
-            }
-            dots[buf][w][lane] = (d0 + d1) + (d2 + d3);
-            __syncthreads();
-            const double g = ((dots[buf][0][lane] + dots[buf][1][lane]) + (dots[buf][2][lane] + dots[buf][3][lane])) +
-                             ((dots[buf][4][lane] + dots[buf][5][lane]) + (dots[buf][6][lane] + dots[buf][7][lane]));
-            const double sigma = __shfl_sync(0xffffffffu, g, i);   // lane i's own column: the same sum, bit for bit
-            const double alpha = rowi[buf][i];
-            double tau = 0.0, scale = 0.0, beta = alpha;
-            if (sigma != 0.0) {   // dlarfg: beta = -sign(alpha) * ||(alpha, x)||, tau = (beta - alpha) / beta
-                // one rsqrt and one reciprocal instead of sqrt + two divisions (the scalar chain is on the critical
-                // path of every column): ||.|| = s * rsqrt(s), 1/beta = -sign(alpha) * rsqrt(s); each within ~1 ulp,
-                // which perturbs H by O(eps) exactly like the rounding of tau itself
-                const double s2 = fma(alpha, alpha, sigma);
-                const double rs = rsqrt(s2);
-                beta = -copysign(s2 * rs, alpha);
-                const double dab = alpha - beta;
-                scale = __drcp_rn(dab);
-                tau = dab * copysign(rs, alpha);
-            }
-            // (3) v_i . (column of this lane): columns > i get updated, columns < i feed the Gram matrix of V
-            // Finished columns (lanes < i) keep their reflector UNSCALED in registers (u_c = raw column below its pivot,
-            // v_c = e_c + myscale_c u_c): scaling happens once, when the panel is stored, instead of 32 single-lane
-            // multiplications per column.  rowi[c] then holds u_c[i], g_c = u_i . u_c over the rows below i.
-            if (lane == i) myscale = scale;
-            const double gv = fma(scale, g, rowi[buf][lane]);
-            const double wc = (lane > i) ? tau * gv : 0.0;
-            if (w == 0) {
-                if (lane < i) Gs[lane][i] = myscale * gv;     // v_c . v_i = myscale_c (u_c[i] + scale_i g_c)
-                if (lane == i) taus[i] = tau;
-                a[k] = (lane == i) ? beta : a[k] - wc;
-            }
-            const double cs = wc * scale;
-#pragma unroll
-            for (int r = 0; r < TS_KEEP; ++r) a[r] = fma(-cs, vk[r], a[r]);
-#pragma unroll
-            for (int r = TS_KEEP; r < TS_B; r += 2) {
-                const double2 v = *reinterpret_cast<const double2*>(&vbuf[w][r]);
-                a[r] = fma(-cs, v.x, a[r]);
-                a[r + 1] = fma(-cs, v.y, a[r + 1]);
-            }
-        }
-        if (w == 0) {   // finished rows of the top block: R on and above the diagonal, scaled reflector entries below it
-#pragma unroll
-            for (int r = 0; r < TS_CG; ++r) {
-                const int row = ib * TS_CG + r;
-                base[(long long)row * ld] = (row > lane) ? a[r] * myscale : a[r];
-                a[r] = 0.0;
-            }
-        }
-        double tmp[TS_CG];
-#pragma unroll
-        for (int r = 0; r < TS_CG; ++r) tmp[r] = a[r];
-#pragma unroll
-        for (int r = 0; r < TS_B - TS_CG; ++r) a[r] = a[r + TS_CG];
-#pragma unroll
-        for (int r = 0; r < TS_CG; ++r) a[TS_B - TS_CG + r] = tmp[r];
-    }
-    if (valid && w > 0) {
-#pragma unroll
-        for (int r = 0; r < TS_B; ++r) base[(long long)r * ld] = a[r] * myscale;
-    }
-    __syncthreads();
-    // compact-WY factor: T = U^-1 with U = striu(V'V) + diag(1/tau); column `lane` by back substitution.
-    // tau_r = 0 (H_r = I) gives a zero row/column r, as in dlarft.
-    if (w == 0) {
-        double t[TS_B];
-#pragma unroll
-        for (int r = TS_B - 1; r >= 0; --r) {
-            double sa = (r == lane) ? 1.0 : 0.0, sb = 0.0;
-#pragma unroll
-            for (int k = r + 1; k < TS_B; k += 2) {
-                sa = fma(-Gs[r][k], t[k], sa);
-                if (k + 1 < TS_B) sb = fma(-Gs[r][k + 1], t[k + 1], sb);
-            }
-            t[r] = (r <= lane) ? (sa + sb) * taus[r] : 0.0;
-        }
-        double* Tg = Tbuf + sub * (TS_B * TS_B);
-#pragma unroll
-        for (int r = 0; r < TS_B; ++r) Tg[r * TS_B + lane] = t[r];
-    }
-    if (rcol < 0) return;
-    // ---- residual column: b <- (I - V T' V') b for this subtile (the same update the trailing kernel applies to
-    //      the 32-column blocks, here with FMAs on the reflectors still held in registers) ----
-    double vs = myscale;
-    if (w == 0) {   // the top block's registers were cleared row by row: reload its unit lower trapezoid (own stores)
-#pragma unroll
-        for (int r = 0; r < TS_B; ++r) a[r] = (r > lane) ? base[(long long)r * ld] : ((r == lane) ? 1.0 : 0.0);
-        vs = 1.0;
-    }
-    __syncwarp();
-    vbuf[w][lane] = bval;
-    __syncwarp();
-    {
-        double g0 = 0.0, g1 = 0.0, g2 = 0.0, g3 = 0.0;
-#pragma unroll
-        for (int r = 0; r < TS_B; r += 4) {
-            const double2 b01 = *reinterpret_cast<const double2*>(&vbuf[w][r]);
-            const double2 b23 = *reinterpret_cast<const double2*>(&vbuf[w][r + 2]);
-            g0 = fma(b01.x, a[r + 0], g0); g1 = fma(b01.y, a[r + 1], g1);
-            g2 = fma(b23.x, a[r + 2], g2); g3 = fma(b23.y, a[r + 3], g3);
-        }
-        dots[0][w][lane] = ((g0 + g1) + (g2 + g3)) * vs;       // (V_w' b_w)[lane]
-    }
-    __syncthreads();
-    if (w == 0) {
-        const double gc = ((dots[0][0][lane] + dots[0][1][lane]) + (dots[0][2][lane] + dots[0][3][lane])) +
-                          ((dots[0][4][lane] + dots[0][5][lane]) + (dots[0][6][lane] + dots[0][7][lane]));
-        rowi[0][lane] = gc;
-        __syncwarp();
-        const double* Tg = Tbuf + sub * (TS_B * TS_B);          // column `lane` of T: this lane's own stores
-        double w0 = 0.0, w1 = 0.0;
-#pragma unroll
-        for (int k = 0; k < TS_B; k += 2) {
-            w0 = fma(Tg[k * TS_B + lane], rowi[0][k], w0);
-            w1 = fma(Tg[(k + 1) * TS_B + lane], rowi[0][k + 1], w1);
-        }
-        rowi[1][lane] = -(w0 + w1);                              // W = -T' G
-    }
-    __syncthreads();
-    {
-        const double wc = rowi[1][lane] * vs;
-#pragma unroll
-        for (int r = 0; r < TS_B; ++r) a[r] *= wc;              // lane c: V[r][c] W[c] for the 32 rows of the warp
-        // butterfly reduce-scatter over the lanes: afterwards a[0] of lane r is sum_c V[r][c] W[c]
-#pragma unroll
-        for (int sft = 16; sft > 0; sft >>= 1) {
-            const bool up = (lane & sft) != 0;
-#pragma unroll
-            for (int j = 0; j < sft; ++j) {
-                const double keep = up ? a[j + sft] : a[j];
-                const double send = up ? a[j] : a[j + sft];
-                a[j] = keep + __shfl_xor_sync(0xffffffffu, send, sft);
-            }
-        }
-        if (valid) *bptr = bval + a[0];
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// panel factorisation, column-group form: warp w owns columns 4w..4w+3 of all 256 rows of the subtile
-// ---------------------------------------------------------------------------------------------
-// Same algorithm, same outputs (V in place, unscaled until stored; T; residual column) as tsqr_panel_kernel.  What
-// changes is the ownership: lane l of warp w holds columns 4w..4w+3 of the rows 32 r + l (r = 0..7: one row of every
-// 32-row block of the subtile).  Consequences:
-//   * a finished column group costs its warp only the 32 dot products that feed the T factor: no update, and none of
-//     the scalar chain;
-//   * the scalar chain of a column (norm, rsqrt, reciprocal -- dlarfg) runs in ONE warp, the owner of the column,
-//     which publishes the raw column together with tau and scale; the other 7 warps no longer replicate it;
+// Lane l of warp w holds columns 4w..4w+3 of the rows 32 r + l (r = 0..7: one row of every 32-row block of the subtile).
+// One block barrier per column i:
+//   * the scalar chain of the column (norm, rsqrt, reciprocal -- dlarfg) runs in ONE warp, the owner of the column,
+//     which publishes the raw column u_i (the entries below the pivot) together with tau and scale;
+//   * every warp then takes ONE pass of dot products g_c = u_i . a_c with its columns.  The reflector
+//     v_i = e_i + scale * u_i is linear in the raw column, so v_i . a_c = a_c[i] + scale * g_c: live columns (c > i)
+//     are updated with it, finished ones (c < i) give v_c . v_i, the Gram matrix of V that the T factor needs;
+//   * a finished column group costs its warp only those 32 dot products: no update, and none of the scalar chain;
 //   * every dot product is reduced inside a warp (shuffles), there is no cross-warp reduction; the pivot-row entry of
 //     a column is fetched from the owning lane by one shuffle.
-// One block barrier per column, as before.  Top block: rows <= i are masked out of the published column, so the
-// finished rows of R simply stay where they are (no progressive store, no register rotation).
+// Finished columns keep their reflector UNSCALED in registers (u_c, v_c = e_c + scale_c u_c): scaling happens once, when
+// the panel is stored.  Top block: rows <= i are masked out of the published column, so the finished rows of R simply
+// stay where they are.  The residual column of [J | r] (column rcol) is updated at the end with the block reflector of
+// the panel, so the trailing-update kernel only sees full 32-column blocks.
 __device__ __forceinline__ double warp_allsum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -340,7 +128,10 @@ tsqr_panel_cg_kernel(double* __restrict__ A, int ld, long long nblk, long long s
                 const double sigma = warp_allsum(s0 + s1);
                 const double alpha = __shfl_sync(0xffffffffu, a[k][0], i);
                 double tau = 0.0, scale = 0.0, beta = alpha;
-                if (sigma != 0.0) {   // dlarfg: beta = -sign(alpha) ||(alpha, x)||, tau = (beta - alpha) / beta (see tsqr_panel_kernel)
+                if (sigma != 0.0) {   // dlarfg: beta = -sign(alpha) * ||(alpha, x)||, tau = (beta - alpha) / beta
+                    // one rsqrt and one reciprocal instead of sqrt + two divisions (the scalar chain is on the critical
+                    // path of every column): ||.|| = s * rsqrt(s), 1/beta = -sign(alpha) * rsqrt(s); each within ~1 ulp,
+                    // which perturbs H by O(eps) exactly like the rounding of tau itself
                     const double s2 = fma(alpha, alpha, sigma);
                     const double rs = rsqrt(s2);
                     beta = -copysign(s2 * rs, alpha);
@@ -411,7 +202,8 @@ tsqr_panel_cg_kernel(double* __restrict__ A, int ld, long long nblk, long long s
     }
     bsh[w][lane] = bval;
     __syncthreads();
-    // compact-WY factor (as in tsqr_panel_kernel): T = U^-1, U = striu(V'V) + diag(1/tau); lane = column
+    // compact-WY factor: T = U^-1 with U = striu(V'V) + diag(1/tau); column `lane` by back substitution.
+    // tau_r = 0 (H_r = I) gives a zero row/column r, as in dlarft.
     if (w == 0) {
         double t[TS_B];
 #pragma unroll
@@ -472,155 +264,6 @@ tsqr_panel_cg_kernel(double* __restrict__ A, int ld, long long nblk, long long s
 }
 
 // ---------------------------------------------------------------------------------------------
-// trailing update of one (subtile, column block)
-// ---------------------------------------------------------------------------------------------
-template <int CB>
-__device__ __forceinline__ void tsqr_trail_body(double* __restrict__ A, int ld, long long nblk, long long stride,
-                                                int col0, int ccol0, long long sub, const double* __restrict__ Tbuf,
-                                                double* smem) {
-    constexpr int NT = CB / 8;          // 8-column tiles per block row
-    constexpr int CBP = CB + 4;         // padded leading dimension of the CB-wide shared tiles
-    constexpr int NV = 4 * NT * 2;      // accumulator values per thread
-    double (*Ts)[TS_LDS] = reinterpret_cast<double (*)[TS_LDS]>(smem);
-    double (*Gs)[CBP] = reinterpret_cast<double (*)[CBP]>(smem + TS_B * TS_LDS);
-    double (*Ws)[CBP] = reinterpret_cast<double (*)[CBP]>(smem + TS_B * TS_LDS + TS_B * CBP);
-    double* Ps = smem + TS_B * TS_LDS + 2 * TS_B * (TS_B + 4);   // 4 partial-sum buffers, [value][lane]
-    const int tid = threadIdx.x, w = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-    const long long blk = (sub * TS_FAN + w) * stride;
-    const bool valid = blk < nblk;
-    const double* Vb = A + (blk * TS_B) * (long long)ld + col0;
-    double* Bb = A + (blk * TS_B) * (long long)ld + ccol0;
-    const double* Tg = Tbuf + sub * (TS_B * TS_B);
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        int idx = tid + 256 * q;
-        Ts[idx >> 5][idx & 31] = Tg[idx];
-    }
-    // reflector block element (row, c) of this warp's block: unit lower trapezoid for the top block
-    auto vload = [&](int row, int c) -> double {
-        double v = Vb[(long long)row * ld + c];
-        if (w == 0) v = (row < c) ? 0.0 : ((row == c) ? 1.0 : v);
-        return v;
-    };
-    // pass 1: partial G = V_w' B_w over this warp's 32 rows
-    double acc[4][NT][2];
-#pragma unroll
-    for (int ti = 0; ti < 4; ++ti)
-#pragma unroll
-        for (int tj = 0; tj < NT; ++tj) acc[ti][tj][0] = acc[ti][tj][1] = 0.0;
-    if (valid) {
-#pragma unroll
-        for (int kk = 0; kk < 8; ++kk) {
-            const int row = kk * 4 + t;
-            double av[4], bv[NT];
-#pragma unroll
-            for (int ti = 0; ti < 4; ++ti) av[ti] = vload(row, ti * 8 + g);
-#pragma unroll
-            for (int tj = 0; tj < NT; ++tj) bv[tj] = Bb[(long long)row * ld + tj * 8 + g];
-#pragma unroll
-            for (int ti = 0; ti < 4; ++ti)
-#pragma unroll
-                for (int tj = 0; tj < NT; ++tj) dmma884(acc[ti][tj][0], acc[ti][tj][1], av[ti], bv[tj]);
-        }
-    }
-    // deterministic pairwise tree over the 8 warps: (w, w + 4), then (w, w + 2), then (0, 1)
-    auto put = [&](int b) {
-#pragma unroll
-        for (int ti = 0; ti < 4; ++ti)
-#pragma unroll
-            for (int tj = 0; tj < NT; ++tj) {
-                Ps[(b * NV + (ti * NT + tj) * 2) * 32 + lane] = acc[ti][tj][0];
-                Ps[(b * NV + (ti * NT + tj) * 2 + 1) * 32 + lane] = acc[ti][tj][1];
-            }
-    };
-    auto take = [&](int b) {
-#pragma unroll
-        for (int ti = 0; ti < 4; ++ti)
-#pragma unroll
-            for (int tj = 0; tj < NT; ++tj) {
-                acc[ti][tj][0] += Ps[(b * NV + (ti * NT + tj) * 2) * 32 + lane];
-                acc[ti][tj][1] += Ps[(b * NV + (ti * NT + tj) * 2 + 1) * 32 + lane];
-            }
-    };
-    if (w >= 4) put(w - 4);
-    __syncthreads();
-    if (w < 4) take(w);
-    if (w == 2 || w == 3) put(w);      // its own buffer: nobody else reads it before the next barrier
-    __syncthreads();
-    if (w < 2) take(w + 2);
-    if (w == 1) put(1);
-    __syncthreads();
-    if (w == 0) {
-        take(1);
-#pragma unroll
-        for (int ti = 0; ti < 4; ++ti)
-#pragma unroll
-            for (int tj = 0; tj < NT; ++tj) {
-                Gs[ti * 8 + g][tj * 8 + 2 * t] = acc[ti][tj][0];
-                Gs[ti * 8 + g][tj * 8 + 2 * t + 1] = acc[ti][tj][1];
-            }
-    }
-    // the block of B in accumulator layout for pass 2: issued here so that the loads fly during the W stage
-    double b2[4][NT][2];
-    if (valid) {
-#pragma unroll
-        for (int ri = 0; ri < 4; ++ri)
-#pragma unroll
-            for (int cj = 0; cj < NT; ++cj) {
-                double2 v = *reinterpret_cast<const double2*>(Bb + (long long)(ri * 8 + g) * ld + cj * 8 + 2 * t);
-                b2[ri][cj][0] = v.x; b2[ri][cj][1] = v.y;
-            }
-    }
-    __syncthreads();
-    // W = -T' G  (4 x NT tiles over the 8 warps)
-    for (int id = w; id < 4 * NT; id += TS_FAN) {
-        const int ti = id / NT, tj = id % NT;
-        double c0 = 0.0, c1 = 0.0;
-#pragma unroll
-        for (int kk = 0; kk < 8; ++kk) dmma884(c0, c1, Ts[kk * 4 + t][ti * 8 + g], Gs[kk * 4 + t][tj * 8 + g]);
-        Ws[ti * 8 + g][tj * 8 + 2 * t] = -c0;
-        Ws[ti * 8 + g][tj * 8 + 2 * t + 1] = -c1;
-    }
-    __syncthreads();
-    // pass 2: B_w += V_w W
-    if (valid) {
-#pragma unroll
-        for (int kk = 0; kk < 8; ++kk) {
-            double av[4], bw[NT];
-#pragma unroll
-            for (int ri = 0; ri < 4; ++ri) av[ri] = vload(ri * 8 + g, kk * 4 + t);
-#pragma unroll
-            for (int cj = 0; cj < NT; ++cj) bw[cj] = Ws[kk * 4 + t][cj * 8 + g];
-#pragma unroll
-            for (int ri = 0; ri < 4; ++ri)
-#pragma unroll
-                for (int cj = 0; cj < NT; ++cj) dmma884(b2[ri][cj][0], b2[ri][cj][1], av[ri], bw[cj]);
-        }
-#pragma unroll
-        for (int ri = 0; ri < 4; ++ri)
-#pragma unroll
-            for (int cj = 0; cj < NT; ++cj)
-                *reinterpret_cast<double2*>(Bb + (long long)(ri * 8 + g) * ld + cj * 8 + 2 * t) =
-                    make_double2(b2[ri][cj][0], b2[ri][cj][1]);
-    }
-}
-
-constexpr int TS_TRAIL_SMEM = (TS_B * TS_LDS + 2 * TS_B * (TS_B + 4) + 4 * 32 * 32) * (int)sizeof(double);
-
-// 1-D grid of nsub * ncb32 CTAs, column block fastest (CTAs sharing a reflector block V run together, so V is read
-// from HBM once): item cb is the 32-column block col0 + 32 (cb + 1).  The residual column of [J | r] is updated by the
-// panel kernel itself.
-template <int CB>
-__global__ void __launch_bounds__(256, (CB == 32 ? 2 : 3))
-tsqr_trail_kernel(double* __restrict__ A, int ld, long long nblk, long long stride, int col0, int ncb,
-                  const double* __restrict__ Tbuf) {
-    extern __shared__ __align__(16) double smem[];
-    const long long sub = blockIdx.x / (unsigned)ncb;
-    const int cb = (int)(blockIdx.x % (unsigned)ncb);
-    tsqr_trail_body<CB>(A, ld, nblk, stride, col0, col0 + TS_B + CB * cb, sub, Tbuf, smem);
-}
-
-// ---------------------------------------------------------------------------------------------
 // trailing update, staged form: one CTA per (subtile, chunk of 32-column blocks)
 // ---------------------------------------------------------------------------------------------
 // The reflector block V (256 x 32) and T are brought into shared memory ONCE per CTA with cp.async and serve every
@@ -636,9 +279,7 @@ tsqr_trail_kernel(double* __restrict__ A, int ld, long long nblk, long long stri
 // B is read from HBM once and written once; V once per chunk.
 constexpr int TR_LD = 36;
 constexpr int TR_ROWS = TS_B * TS_FAN;   // 256
-#ifndef TR_NW
-#define TR_NW 8                          // warps per CTA (8 or 16)
-#endif
+constexpr int TR_NW = 8;                 // warps per CTA
 constexpr int TR_KS = TR_NW / 4;         // row splits of pass 1 (each split: 4 warps = the 4 quadrants of G)
 constexpr int TR_SMEM = (2 * TR_ROWS * TR_LD + (2 + TR_KS) * TS_B * TR_LD) * (int)sizeof(double);   // V, B | T, W, G[KS]
 
@@ -798,413 +439,6 @@ tsqr_trail_staged_kernel(double* __restrict__ A, int ld, long long nblk, long lo
     }
 }
 
-// ---------------------------------------------------------------------------------------------
-// trailing update fed by TMA: the staged kernel above with its operand traffic taken out of the math warps
-// ---------------------------------------------------------------------------------------------
-// A ninth warp is the producer: it moves V (once per CTA) and every 256 x 32 block of B from the row-major work matrix
-// into the padded shared-memory tiles with bulk asynchronous copies (cp.async.bulk.shared::cluster.global with
-// mbarrier::complete_tx::bytes: the TMA unit, UBLKCP in SASS), one 256-byte row per copy so that the conflict-free
-// leading dimension of 36 doubles survives; an mbarrier per buffer carries the byte count.  The eight math warps issue
-// LDS + DMMA (+ the stores of their result rows) and wait on the mbarrier instead of cp.async.wait_group + a block
-// barrier.  Schedule, tiles and results are those of tsqr_trail_staged_kernel (bit-identical output).
-// MEASURED SLOWER than the cp.async kernel (see tsqr_factor) and therefore not the default: selectable with
-// ENLSIP_TRAIL=3, covered by test_tsqr_tma_trailing_kernel_matches.
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-    unsigned done;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    } while (!done);
-}
-__device__ __forceinline__ void bulk_g2s(double* smem_dst, const double* gsrc, unsigned bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-constexpr int TR_TMA_SMEM = TR_SMEM + 64;
-
-template <int NW>
-__global__ void __launch_bounds__(32 * (NW + 1), 1)
-tsqr_trail_tma_kernel(double* __restrict__ A, int ld, long long nblk, long long stride, int col0, int ncb, int cbpc,
-                      const double* __restrict__ Tbuf) {
-    constexpr int NTH = 32 * NW;          // math threads
-    constexpr int KS = NW / 4;
-    constexpr int KROWS = TR_ROWS / KS;
-    constexpr int RW = TR_ROWS / NW;
-    constexpr int RT = RW / 8;
-    extern __shared__ __align__(16) double smem[];
-    double* Vs = smem;
-    double* Bs = Vs + TR_ROWS * TR_LD;
-    double* Ts = Bs + TR_ROWS * TR_LD;
-    double* Ws = Ts + TS_B * TR_LD;
-    double* Gs = Ws + TS_B * TR_LD;
-    unsigned long long* bars = reinterpret_cast<unsigned long long*>(Gs + KS * TS_B * TR_LD);   // [0]: V, [1]: B
-    const int tid = threadIdx.x, w = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-    const bool producer = (w == NW);
-    const int nchunks = (ncb + cbpc - 1) / cbpc;
-    const long long sub = blockIdx.x / (unsigned)nchunks;
-    const int chunk = (int)(blockIdx.x % (unsigned)nchunks);
-    const int cb_begin = chunk * cbpc;
-    const int cb_end = (cb_begin + cbpc < ncb) ? cb_begin + cbpc : ncb;
-    int nvalid = 0;                        // 32-row blocks of this subtile that exist
-#pragma unroll
-    for (int b = 0; b < TS_FAN; ++b) nvalid += ((sub * TS_FAN + b) * stride < nblk) ? 1 : 0;
-    const unsigned tile_bytes = (unsigned)nvalid * TS_B * TS_B * (unsigned)sizeof(double);
-    // producer: 256 x 32 tile at column c0 -> dst, one bulk copy per existing row (lane owns rows lane, lane + 32, ...)
-    auto tma_stage = [&](double* dst, int c0, unsigned long long* bar) {
-        if (lane == 0) mbar_expect_tx(bar, tile_bytes);
-        __syncwarp();
-#pragma unroll
-        for (int q = 0; q < TS_FAN; ++q) {
-            const int row = lane + 32 * q;
-            const long long blk = (sub * TS_FAN + q) * stride;
-            if (blk < nblk) bulk_g2s(dst + row * TR_LD, A + (blk * TS_B + lane) * (long long)ld + c0, TS_B * sizeof(double), bar);
-        }
-    };
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);
-        mbar_init(&bars[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    // rows of missing blocks are never written by a copy: zero them once (both tiles)
-    for (int idx = tid; idx < TR_ROWS * TS_B; idx += 32 * (NW + 1)) {
-        const int row = idx >> 5, c = idx & 31;
-        if ((sub * TS_FAN + (row >> 5)) * stride >= nblk) { Vs[row * TR_LD + c] = 0.0; Bs[row * TR_LD + c] = 0.0; }
-    }
-    __syncthreads();
-    if (producer) {
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        tma_stage(Vs, col0, &bars[0]);
-        tma_stage(Bs, col0 + TS_B * (cb_begin + 1), &bars[1]);
-    } else {
-        const double* Tg = Tbuf + sub * (TS_B * TS_B);
-#pragma unroll
-        for (int q = 0; q < 1024 / NTH; ++q) {
-            const int idx = tid + NTH * q;
-            Ts[(idx >> 5) * TR_LD + (idx & 31)] = Tg[idx];
-        }
-        mbar_wait(&bars[0], 0);
-    }
-    __syncthreads();
-    // the top block of V is a unit lower trapezoid (R of the panel sits on and above its diagonal)
-    if (!producer) {
-#pragma unroll
-        for (int q = 0; q < 1024 / NTH; ++q) {
-            const int idx = tid + NTH * q;
-            const int r = idx >> 5, c = idx & 31;
-            if (r <= c) Vs[r * TR_LD + c] = (r == c) ? 1.0 : 0.0;
-        }
-    }
-    __syncthreads();
-    const int wm = producer ? 0 : w;
-    const long long myblk = (sub * TS_FAN + ((wm * RW) >> 5)) * stride;
-    const bool valid = myblk < nblk;
-    const int kh = wm >> 2, qd = wm & 3;
-    const int ti0 = (qd >> 1) * 2, tj0 = (qd & 1) * 2;
-    double* Gk = Gs + kh * (TS_B * TR_LD);
-    unsigned phase = 0;
-    for (int cb = cb_begin; cb < cb_end; ++cb) {
-        if (producer) {
-            __syncthreads();                  // (a) the math warps have taken the block out of Bs
-            if (cb + 1 < cb_end) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                tma_stage(Bs, col0 + TS_B * (cb + 2), &bars[1]);
-            }
-            __syncthreads();                  // (b) W stage done
-            continue;
-        }
-        mbar_wait(&bars[1], phase);
-        phase ^= 1u;
-        // ---- pass 1: this warp's quadrant of G over its share of the rows ----
-        double acc[2][2][2];
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int j = 0; j < 2; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-        {
-            const double* vp = Vs + (kh * KROWS + t) * TR_LD + ti0 * 8 + g;
-            const double* bp = Bs + (kh * KROWS + t) * TR_LD + tj0 * 8 + g;
-#pragma unroll 8
-            for (int kk = 0; kk < KROWS / 4; ++kk) {
-                const double a0 = vp[kk * 4 * TR_LD], a1 = vp[kk * 4 * TR_LD + 8];
-                const double b0 = bp[kk * 4 * TR_LD], b1 = bp[kk * 4 * TR_LD + 8];
-                dmma884(acc[0][0][0], acc[0][0][1], a0, b0);
-                dmma884(acc[0][1][0], acc[0][1][1], a0, b1);
-                dmma884(acc[1][0][0], acc[1][0][1], a1, b0);
-                dmma884(acc[1][1][0], acc[1][1][1], a1, b1);
-            }
-        }
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-                *reinterpret_cast<double2*>(Gk + ((ti0 + i) * 8 + g) * TR_LD + (tj0 + j) * 8 + 2 * t) =
-                    make_double2(acc[i][j][0], acc[i][j][1]);
-        double b2[RT][4][2];
-#pragma unroll
-        for (int ri = 0; ri < RT; ++ri)
-#pragma unroll
-            for (int cj = 0; cj < 4; ++cj) {
-                const double2 v = *reinterpret_cast<const double2*>(Bs + (w * RW + ri * 8 + g) * TR_LD + cj * 8 + 2 * t);
-                b2[ri][cj][0] = v.x; b2[ri][cj][1] = v.y;
-            }
-        __syncthreads();                      // (a) Bs is free: the producer streams the next block in
-        // ---- W = -T' G ----
-#pragma unroll
-        for (int id = w; id < 16; id += NW) {
-            const int ti = id >> 2, tj = id & 3;
-            double c0 = 0.0, c1 = 0.0;
-#pragma unroll
-            for (int kk = 0; kk < 8; ++kk) {
-                const int o = (kk * 4 + t) * TR_LD + tj * 8 + g;
-                double gv;
-                if (KS == 2) gv = Gs[o] + Gs[TS_B * TR_LD + o];
-                else gv = (Gs[o] + Gs[TS_B * TR_LD + o]) + (Gs[2 * TS_B * TR_LD + o] + Gs[3 * TS_B * TR_LD + o]);
-                dmma884(c0, c1, Ts[(kk * 4 + t) * TR_LD + ti * 8 + g], gv);
-            }
-            *reinterpret_cast<double2*>(Ws + (ti * 8 + g) * TR_LD + tj * 8 + 2 * t) = make_double2(-c0, -c1);
-        }
-        __syncthreads();                      // (b)
-        // ---- pass 2: B_w += V_w W ----
-        {
-            const double* vp = Vs + (w * RW + g) * TR_LD + t;
-            const double* wp = Ws + t * TR_LD + g;
-#pragma unroll
-            for (int kk = 0; kk < 8; ++kk) {
-                double av[RT], bw[4];
-#pragma unroll
-                for (int ri = 0; ri < RT; ++ri) av[ri] = vp[ri * 8 * TR_LD + kk * 4];
-#pragma unroll
-                for (int cj = 0; cj < 4; ++cj) bw[cj] = wp[kk * 4 * TR_LD + cj * 8];
-#pragma unroll
-                for (int ri = 0; ri < RT; ++ri)
-#pragma unroll
-                    for (int cj = 0; cj < 4; ++cj) dmma884(b2[ri][cj][0], b2[ri][cj][1], av[ri], bw[cj]);
-            }
-        }
-        if (valid) {
-            double* Bb = A + (myblk * TS_B + ((w * RW) & 31)) * (long long)ld + col0 + TS_B * (cb + 1);
-#pragma unroll
-            for (int ri = 0; ri < RT; ++ri)
-#pragma unroll
-                for (int cj = 0; cj < 4; ++cj)
-                    *reinterpret_cast<double2*>(Bb + (long long)(ri * 8 + g) * ld + cj * 8 + 2 * t) =
-                        make_double2(b2[ri][cj][0], b2[ri][cj][1]);
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// trailing update fed by TMA, tensor-map form: one cp.async.bulk.tensor.2d per 32 x 16 box (4 KB), 128-byte swizzle
-// ---------------------------------------------------------------------------------------------
-// The work matrix is described once by a 2-D tensor map (row major, inner dimension = ld doubles); a 256 x 32 tile is
-// 8 row blocks x 2 column halves = 16 boxes of 32 rows x 16 doubles, each landing as 32 rows of 128 bytes whose 16-byte
-// chunks are XOR-swizzled with the row number (CU_TENSOR_MAP_SWIZZLE_128B).  Row blocks beyond the matrix are
-// out-of-bounds boxes: the TMA unit zero-fills them and still delivers their byte count.  The fragment loads are
-// re-assigned so that the swizzled tiles are read without bank conflicts:
-//   pass 1 (G = V'B: lanes = 4 k-rows x 8 columns): the four k-rows of a DMMA step are rows b, b+2, b+4, b+6 of an
-//          8-row group (distinct (row >> 1) & 3 => their 16-byte chunk pairs fall into disjoint bank groups);
-//   pass 2 (B += V W: lanes = 8 rows x 4 k-columns) and the accumulator tiles: fragment row g is row
-//          QROW(g) = {0,4,2,6,1,5,3,7}[g] of its 8-row tile, for the same reason.
-// Same schedule as tsqr_trail_staged_kernel; the summation order inside G differs (other row grouping), results agree
-// to rounding.
-constexpr int TM_BOX_ROWS = 32, TM_BOX_COLS = 16;
-constexpr int TM_BOX_DOUBLES = TM_BOX_ROWS * TM_BOX_COLS;                 // 512 doubles = 4 KB
-constexpr int TM_TILE_DOUBLES = 16 * TM_BOX_DOUBLES;                      // 256 x 32
-// element (r, c) of a swizzled 256 x 32 tile, r < 256, c < 32
-__device__ __forceinline__ int tm_off(int r, int c) {
-    const int box = ((r >> 5) << 1) | (c >> 4), rr = r & 31, cc = c & 15;
-    return box * TM_BOX_DOUBLES + rr * 16 + ((((cc >> 1) ^ (rr & 7)) << 1) | (cc & 1));
-}
-__device__ __forceinline__ int tm_qrow(int g) { return ((g & 1) << 2) | (g & 2) | (g >> 2); }   // 0,4,2,6,1,5,3,7
-__device__ __forceinline__ void tma_load_2d(double* smem_dst, const CUtensorMap* tmap, int c0, int c1, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"(smem_u32(smem_dst)), "l"(tmap), "r"(c0), "r"(c1), "r"(smem_u32(bar)) : "memory");
-}
-constexpr int tm_smem_bytes(int nw) { return (2 * TM_TILE_DOUBLES + (2 + nw / 4) * TS_B * TR_LD) * (int)sizeof(double) + 64 + 1024; }
-
-template <int NW>
-__global__ void __launch_bounds__(32 * (NW + 1), 1)
-tsqr_trail_tmap_kernel(const __grid_constant__ CUtensorMap tmap, double* __restrict__ A, int ld, long long nblk, long long stride,
-                       int col0, int ncb, int cbpc, const double* __restrict__ Tbuf) {
-    constexpr int NTH = 32 * NW;
-    constexpr int KS = NW / 4;
-    constexpr int KROWS = TR_ROWS / KS;
-    constexpr int RW = TR_ROWS / NW;
-    constexpr int RT = RW / 8;
-    extern __shared__ __align__(1024) double smem_raw[];
-    double* smem = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    double* Vs = smem;
-    double* Bs = Vs + TM_TILE_DOUBLES;
-    double* Ts = Bs + TM_TILE_DOUBLES;
-    double* Ws = Ts + TS_B * TR_LD;
-    double* Gs = Ws + TS_B * TR_LD;
-    unsigned long long* bars = reinterpret_cast<unsigned long long*>(Gs + KS * TS_B * TR_LD);
-    const int tid = threadIdx.x, w = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-    const bool producer = (w == NW);
-    const int nchunks = (ncb + cbpc - 1) / cbpc;
-    const long long sub = blockIdx.x / (unsigned)nchunks;
-    const int chunk = (int)(blockIdx.x % (unsigned)nchunks);
-    const int cb_begin = chunk * cbpc;
-    const int cb_end = (cb_begin + cbpc < ncb) ? cb_begin + cbpc : ncb;
-    // producer: lanes 0..15 each issue one box of the tile at column c0 (row block lane >> 1, column half lane & 1)
-    auto tma_stage = [&](double* dst, int c0, unsigned long long* bar) {
-        if (lane == 0) mbar_expect_tx(bar, (unsigned)(TM_TILE_DOUBLES * sizeof(double)));
-        __syncwarp();
-        if (lane < 16) {
-            const long long blk = (sub * TS_FAN + (lane >> 1)) * stride;
-            // a block index past the matrix is an out-of-bounds box (zero filled); keep the coordinate in int range
-            const long long row = blk < nblk ? blk * TS_B : (long long)nblk * TS_B;
-            tma_load_2d(dst + lane * TM_BOX_DOUBLES, &tmap, c0 + (lane & 1) * TM_BOX_COLS, (int)row, bar);
-        }
-    };
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);
-        mbar_init(&bars[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (producer) {
-        tma_stage(Vs, col0, &bars[0]);
-        tma_stage(Bs, col0 + TS_B * (cb_begin + 1), &bars[1]);
-    } else {
-        const double* Tg = Tbuf + sub * (TS_B * TS_B);
-#pragma unroll
-        for (int q = 0; q < 1024 / NTH; ++q) {
-            const int idx = tid + NTH * q;
-            Ts[(idx >> 5) * TR_LD + (idx & 31)] = Tg[idx];
-        }
-        mbar_wait(&bars[0], 0);
-    }
-    __syncthreads();
-    // the top block of V is a unit lower trapezoid (R of the panel sits on and above its diagonal)
-    if (!producer) {
-#pragma unroll
-        for (int q = 0; q < 1024 / NTH; ++q) {
-            const int idx = tid + NTH * q;
-            const int r = idx >> 5, c = idx & 31;
-            if (r <= c) Vs[tm_off(r, c)] = (r == c) ? 1.0 : 0.0;
-        }
-    }
-    __syncthreads();
-    const int wm = producer ? 0 : w;
-    const long long myblk = (sub * TS_FAN + ((wm * RW) >> 5)) * stride;
-    const bool valid = myblk < nblk;
-    const int kh = wm >> 2, qd = wm & 3;
-    const int ti0 = (qd >> 1) * 2, tj0 = (qd & 1) * 2;
-    double* Gk = Gs + kh * (TS_B * TR_LD);
-    const int qg = tm_qrow(g);
-    unsigned phase = 0;
-    for (int cb = cb_begin; cb < cb_end; ++cb) {
-        if (producer) {
-            __syncthreads();                  // (a) the math warps have taken the block out of Bs
-            if (cb + 1 < cb_end) tma_stage(Bs, col0 + TS_B * (cb + 2), &bars[1]);
-            __syncthreads();                  // (b) W stage done
-            continue;
-        }
-        mbar_wait(&bars[1], phase);
-        phase ^= 1u;
-        // ---- pass 1: this warp's quadrant of G over its share of the rows; k-rows of step kk: base + 2 t ----
-        double acc[2][2][2];
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int j = 0; j < 2; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-#pragma unroll 8
-        for (int kk = 0; kk < KROWS / 4; ++kk) {
-            const int r = kh * KROWS + ((kk >> 1) << 3) + (kk & 1) + 2 * t;
-            const double a0 = Vs[tm_off(r, ti0 * 8 + g)], a1 = Vs[tm_off(r, ti0 * 8 + 8 + g)];
-            const double b0 = Bs[tm_off(r, tj0 * 8 + g)], b1 = Bs[tm_off(r, tj0 * 8 + 8 + g)];
-            dmma884(acc[0][0][0], acc[0][0][1], a0, b0);
-            dmma884(acc[0][1][0], acc[0][1][1], a0, b1);
-            dmma884(acc[1][0][0], acc[1][0][1], a1, b0);
-            dmma884(acc[1][1][0], acc[1][1][1], a1, b1);
-        }
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-                *reinterpret_cast<double2*>(Gk + ((ti0 + i) * 8 + g) * TR_LD + (tj0 + j) * 8 + 2 * t) =
-                    make_double2(acc[i][j][0], acc[i][j][1]);
-        // accumulators of pass 2: this warp's rows of the staged block (fragment row g = tile row QROW(g))
-        double b2[RT][4][2];
-#pragma unroll
-        for (int ri = 0; ri < RT; ++ri)
-#pragma unroll
-            for (int cj = 0; cj < 4; ++cj) {
-                const double2 v = *reinterpret_cast<const double2*>(Bs + tm_off(w * RW + ri * 8 + qg, cj * 8 + 2 * t));
-                b2[ri][cj][0] = v.x; b2[ri][cj][1] = v.y;
-            }
-        __syncthreads();                      // (a) Bs is free: the producer streams the next block in
-        // ---- W = -T' G ----
-#pragma unroll
-        for (int id = w; id < 16; id += NW) {
-            const int ti = id >> 2, tj = id & 3;
-            double c0 = 0.0, c1 = 0.0;
-#pragma unroll
-            for (int kk = 0; kk < 8; ++kk) {
-                const int o = (kk * 4 + t) * TR_LD + tj * 8 + g;
-                double gv;
-                if (KS == 2) gv = Gs[o] + Gs[TS_B * TR_LD + o];
-                else gv = (Gs[o] + Gs[TS_B * TR_LD + o]) + (Gs[2 * TS_B * TR_LD + o] + Gs[3 * TS_B * TR_LD + o]);
-                dmma884(c0, c1, Ts[(kk * 4 + t) * TR_LD + ti * 8 + g], gv);
-            }
-            *reinterpret_cast<double2*>(Ws + (ti * 8 + g) * TR_LD + tj * 8 + 2 * t) = make_double2(-c0, -c1);
-        }
-        __syncthreads();                      // (b)
-        // ---- pass 2: B_w += V_w W ----
-        {
-            const double* wp = Ws + t * TR_LD + g;
-#pragma unroll
-            for (int kk = 0; kk < 8; ++kk) {
-                double av[RT], bw[4];
-#pragma unroll
-                for (int ri = 0; ri < RT; ++ri) av[ri] = Vs[tm_off(w * RW + ri * 8 + qg, kk * 4 + t)];
-#pragma unroll
-                for (int cj = 0; cj < 4; ++cj) bw[cj] = wp[kk * 4 * TR_LD + cj * 8];
-#pragma unroll
-                for (int ri = 0; ri < RT; ++ri)
-#pragma unroll
-                    for (int cj = 0; cj < 4; ++cj) dmma884(b2[ri][cj][0], b2[ri][cj][1], av[ri], bw[cj]);
-            }
-        }
-        if (valid) {
-            double* Bb = A + (myblk * TS_B + ((w * RW) & 31)) * (long long)ld + col0 + TS_B * (cb + 1);
-#pragma unroll
-            for (int ri = 0; ri < RT; ++ri)
-#pragma unroll
-                for (int cj = 0; cj < 4; ++cj)
-                    *reinterpret_cast<double2*>(Bb + (long long)(ri * 8 + qg) * ld + cj * 8 + 2 * t) =
-                        make_double2(b2[ri][cj][0], b2[ri][cj][1]);
-        }
-    }
-}
-
-// host side: the tensor map of a row-major work matrix (rows_pad x ld doubles), boxes of 32 rows x 16 doubles
-inline bool tsqr_make_tensor_map(CUtensorMap* tm, double* A, int ld, long long rows_pad) {
-    static PFN_cuTensorMapEncodeTiled encode = [] {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-            qres != cudaDriverEntryPointSuccess)
-            fn = nullptr;
-        return (PFN_cuTensorMapEncodeTiled)fn;
-    }();
-    if (!encode) return false;
-    const cuuint64_t gdim[2] = {(cuuint64_t)ld, (cuuint64_t)rows_pad};
-    const cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(double)};
-    const cuuint32_t box[2] = {TM_BOX_COLS, TM_BOX_ROWS};
-    const cuuint32_t estr[2] = {1, 1};
-    return encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, A, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 // rows 0..31 of the matrix now hold rows col0..col0+31 of R: copy them out and clear them in place
 // (one CTA per row: at n = 4096 a single CTA needed 140 us per panel)
 __global__ void tsqr_extract_kernel(double* __restrict__ A, int ld, int col0, int ncols, double* __restrict__ Rout,
@@ -1279,16 +513,9 @@ struct TsqrDist {
     int (*allreduce_sum)(void* ctx, double* buf, size_t count, cudaStream_t st) = nullptr;
 };
 
-inline int tsqr_chunk_mode() {           // ENLSIP_TSQR_CHUNK=0: the first heuristic (halve the chunk until 296 CTAs exist)
-    static const int v = [] { const char* e = getenv("ENLSIP_TSQR_CHUNK"); return (e && e[0] == '0') ? 0 : 1; }();
-    return v;
-}
-
-inline int tsqr_chunk_prologue2() {     // twice the prologue of a chunk in units of one column block (ENLSIP_TSQR_CHUNK_P; measured
-                                        // at n = 4096, m = 16384: 48.7 / 49.1 / 49.5 / 50.4 ms per factorisation for 1 / 2 / 4 / 8)
-    static const int v = [] { const char* e = getenv("ENLSIP_TSQR_CHUNK_P"); const int x = e ? atoi(e) : 1; return x < 0 ? 0 : x; }();
-    return v;
-}
+// Chunking of the trailing launches: twice the prologue of a chunk (V and T staged), in units of one column block.
+// Measured on B200 at n = 4096, m = 16384: 48.7 / 49.1 / 49.5 / 50.4 ms per factorisation with 1 / 2 / 4 / 8.
+constexpr int TS_CHUNK_PROLOGUE2 = 1;
 
 // Host-side launcher.  A: rows_pad x ld row major, rows_pad a multiple of 32, pad rows zero.
 // ncols = n + 1 with n a multiple of 32 (columns n+1 .. ld-1 must be zero; ld = n + 8).
@@ -1301,29 +528,11 @@ inline int tsqr_factor(double* A, int ld, long long rows_pad, int n, double* Rou
     const int npanels = n / TS_B;
     int launches = 0;
     // > 48 KB of dynamic shared memory needs the opt-in (per device, so it is simply set on every call)
-    cudaFuncSetAttribute(tsqr_trail_kernel<TS_TRAIL_CB>, cudaFuncAttributeMaxDynamicSharedMemorySize, TS_TRAIL_SMEM);
     cudaFuncSetAttribute(tsqr_trail_staged_kernel<TR_NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, TR_SMEM);
-    cudaFuncSetAttribute(tsqr_trail_tma_kernel<TR_NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, TR_TMA_SMEM);
-    cudaFuncSetAttribute(tsqr_trail_tmap_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, tm_smem_bytes(8));
-    cudaFuncSetAttribute(tsqr_trail_tmap_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, tm_smem_bytes(16));
-    static const int tmap_nw = [] { const char* e = getenv("ENLSIP_TMAP_NW"); return (e && atoi(e) == 16) ? 16 : 8; }();
-    // development switch: ENLSIP_TRAIL=1 selects the direct-from-global trailing kernel (kept for A/B measurements)
-    // development switch: ENLSIP_PANEL=1 selects the row-tile panel kernel (kept for A/B measurements)
-    static const int panel_mode = [] { const char* e = getenv("ENLSIP_PANEL"); return (e && e[0] == '1') ? 1 : 3; }();
-    // ENLSIP_TRAIL=3: the TMA-fed kernel (bulk copies + mbarrier, producer warp).  Measured on B200 at m = 4M, n = 256:
-    // TSQR 80.1 ms against 52.2 ms with the cp.async kernel -- a copy per 256-byte row is 4.3e8 copy operations per
-    // factorisation and the TMA unit does not sustain that rate; 8 KB tensor-map boxes need a swizzled tile layout
-    // (DESIGN.md 5.3 item 12).  Default (2): the cp.async staged kernel.
-    //                 4: tensor-map TMA kernel (4 KB boxes, 128-byte swizzle).
-    static const int trail_mode_env = [] { const char* e = getenv("ENLSIP_TRAIL"); return (e && e[0] >= '1' && e[0] <= '4') ? e[0] - '0' : 2; }();
-    int trail_mode = trail_mode_env;
-    CUtensorMap tmap;
-    if (trail_mode == 4 && ((ld * (int)sizeof(double)) % 16 != 0 || !tsqr_make_tensor_map(&tmap, A, ld, rows_pad))) trail_mode = 2;
     // all tree levels of panel j on the matrix M (nblk_m blocks of 32 rows)
-    auto panel_levels = [&](double* M, long long nblk_m, int j, int mode) {
+    auto panel_levels = [&](double* M, long long nblk_m, int j) {
         const long long nblk = nblk_m;
         double* A = M;
-        const int trail_mode = mode;
         const int col0 = j * TS_B;
         const int ncb32 = npanels - 1 - j;
         long long stride = 1;
@@ -1331,46 +540,26 @@ inline int tsqr_factor(double* A, int ld, long long rows_pad, int n, double* Rou
             long long nb_level = (nblk + stride - 1) / stride;
             if (level > 0 && nb_level <= 1) break;
             long long nsub = (nb_level + TS_FAN - 1) / TS_FAN;
-            if (panel_mode == 1) tsqr_panel_kernel<<<(unsigned)nsub, 256, 0, st>>>(A, ld, nblk, stride, col0, level > 0, n, Tbuf);
-            else tsqr_panel_cg_kernel<<<(unsigned)nsub, 256, 0, st>>>(A, ld, nblk, stride, col0, level > 0, n, Tbuf);
+            tsqr_panel_cg_kernel<<<(unsigned)nsub, 256, 0, st>>>(A, ld, nblk, stride, col0, level > 0, n, Tbuf);
             ++launches;
-            if (ncb32 > 0 && trail_mode >= 2) {
+            if (ncb32 > 0) {
                 // Column blocks per CTA (chunk).  One CTA per SM is resident (registers, shared memory), so the launch runs
                 // in waves of 148 CTAs; a CTA costs a prologue (V and T staged once per chunk, about half a block's worth) plus
                 // its column blocks.  Pick the chunking with the fewest wave-units: with thousands of subtiles that is one
                 // chunk per subtile, with a few dozen subtiles (m = 4 n, upper tree levels) it avoids a mostly empty last
                 // wave.  The arithmetic of a column block does not depend on the chunk it is in.
                 int cbpc = ncb32;
-                if (tsqr_chunk_mode() == 0) {
-                    while (cbpc > 1 && nsub * ((ncb32 + cbpc - 1) / cbpc) < 2 * 148) cbpc = (cbpc + 1) / 2;
-                } else {
-                    long long best_cost = -1;
-                    for (int c = ncb32; c >= 1; --c) {
-                        const long long chunks = (ncb32 + c - 1) / c;
-                        if (c < ncb32 && (ncb32 + c) / (c + 1) == chunks) continue;      // same chunk count as c + 1: larger CTAs for nothing
-                        const long long waves = (nsub * chunks + 147) / 148;
-                        const long long cost = waves * (tsqr_chunk_prologue2() + 2 * c);
-                        if (best_cost < 0 || cost < best_cost) { best_cost = cost; cbpc = c; }
-                    }
+                long long best_cost = -1;
+                for (int c = ncb32; c >= 1; --c) {
+                    const long long chunks = (ncb32 + c - 1) / c;
+                    if (c < ncb32 && (ncb32 + c) / (c + 1) == chunks) continue;      // same chunk count as c + 1: larger CTAs for nothing
+                    const long long waves = (nsub * chunks + 147) / 148;
+                    const long long cost = waves * (TS_CHUNK_PROLOGUE2 + 2 * c);
+                    if (best_cost < 0 || cost < best_cost) { best_cost = cost; cbpc = c; }
                 }
                 const int nchunks = (ncb32 + cbpc - 1) / cbpc;
-                if (trail_mode == 4 && tmap_nw == 16)
-                    tsqr_trail_tmap_kernel<16><<<(unsigned)(nsub * nchunks), 32 * 17, tm_smem_bytes(16), st>>>(tmap, A, ld, nblk, stride, col0,
-                                                                                                   ncb32, cbpc, Tbuf);
-                else if (trail_mode == 4)
-                    tsqr_trail_tmap_kernel<8><<<(unsigned)(nsub * nchunks), 32 * 9, tm_smem_bytes(8), st>>>(tmap, A, ld, nblk, stride, col0,
-                                                                                                ncb32, cbpc, Tbuf);
-                else if (trail_mode == 3)
-                    tsqr_trail_tma_kernel<TR_NW><<<(unsigned)(nsub * nchunks), 32 * (TR_NW + 1), TR_TMA_SMEM, st>>>(A, ld, nblk, stride, col0,
-                                                                                                        ncb32, cbpc, Tbuf);
-                else
-                    tsqr_trail_staged_kernel<TR_NW><<<(unsigned)(nsub * nchunks), 32 * TR_NW, TR_SMEM, st>>>(A, ld, nblk, stride, col0, ncb32,
-                                                                                              cbpc, Tbuf);
-                ++launches;
-            } else if (ncb32 > 0) {
-                constexpr int CBW = TS_TRAIL_CB;
-                const int ncb = ncb32 * (32 / CBW);
-                tsqr_trail_kernel<CBW><<<(unsigned)(nsub * ncb), 256, TS_TRAIL_SMEM, st>>>(A, ld, nblk, stride, col0, ncb, Tbuf);
+                tsqr_trail_staged_kernel<TR_NW><<<(unsigned)(nsub * nchunks), 32 * TR_NW, TR_SMEM, st>>>(A, ld, nblk, stride, col0, ncb32,
+                                                                                          cbpc, Tbuf);
                 ++launches;
             }
             stride *= TS_FAN;
@@ -1379,10 +568,10 @@ inline int tsqr_factor(double* A, int ld, long long rows_pad, int n, double* Rou
     const bool sharded = dist && dist->nranks > 1;
     for (int j = 0; j < npanels; ++j) {
         const int col0 = j * TS_B;
-        panel_levels(A, nblk, j, trail_mode);
+        panel_levels(A, nblk, j);
         if (sharded) {
             if (dist->allgather(dist->ctx, A, dist->P, (size_t)TS_B * ld, st) != 0) return -1;
-            panel_levels(dist->P, dist->nranks, j, trail_mode == 4 ? 2 : trail_mode);
+            panel_levels(dist->P, dist->nranks, j);
             tsqr_extract_kernel<<<TS_B, 256, 0, st>>>(dist->P, ld, col0, n + 1, Rout, ldr);
             tsqr_copyback_kernel<<<TS_B, 256, 0, st>>>(A, dist->P + (size_t)TS_B * dist->rank * ld, ld, col0 + TS_B);
             launches += 2;

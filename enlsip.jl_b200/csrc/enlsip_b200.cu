@@ -302,27 +302,18 @@ constexpr int nt_thread_per_problem() {
     return fit > 128 ? 128 : (fit < 2 ? 1 : fit);      // (a family too large for 2 problems per SM still gets a kernel that fits)
 }
 
-// family id (+ CTA size for the tuned family) -> template instantiation
+// family id -> template instantiation
 template <class F>
-int with_family(int family, int nt, F&& f) {
+int with_family(int family, F&& f) {
 #if defined(ENL_USER_FAMILY)
     // a user library holds the user's family only (compile time: one kernel instead of ten); few rows: one thread per
     // problem, otherwise one warp per problem
-    (void)nt;
     if (family == ENLSIPB200_FAMILY_USER) return f(FamUser{}, ic<(FamUser::M <= 8 ? 1 : 32)>{}, ic<(FamUser::M <= 8 ? nt_thread_per_problem<FamUser>() : 32)>{});
     return fail(ENLSIPB200_EINVAL, "this library was compiled for ENLSIPB200_FAMILY_USER only");
 #else
     switch (family) {
         case ENLSIPB200_FAMILY_HS65: return f(FamHS65{}, ic<1>{}, ic<nt_thread_per_problem<FamHS65>()>{});
-        case ENLSIPB200_FAMILY_GAUSS_PEAKS:
-            switch (nt) {
-                case 64: return f(FamGaussPeaks{}, ic<32>{}, ic<64>{});
-                case 128: return f(FamGaussPeaks{}, ic<32>{}, ic<128>{});
-                case 224: return f(FamGaussPeaks{}, ic<32>{}, ic<224>{});
-                case 448: return f(FamGaussPeaks{}, ic<32>{}, ic<448>{});
-                case 480: return f(FamGaussPeaks{}, ic<32>{}, ic<480>{});
-                default: return f(FamGaussPeaks{}, ic<32>{}, ic<512>{});   // 16 problems per SM: all the shared memory and registers
-            }
+        case ENLSIPB200_FAMILY_GAUSS_PEAKS: return f(FamGaussPeaks{}, ic<32>{}, ic<512>{});   // 16 problems per SM: all the shared memory and registers
         case ENLSIPB200_FAMILY_OSBORNE2: return f(FamOsborne2{}, ic<32>{}, ic<32>{});
         case ENLSIPB200_FAMILY_CHAINED_ROSENBROCK10: return f(FamChainedRosenbrock<10>{}, ic<32>{}, ic<32>{});
         case ENLSIPB200_FAMILY_CHAINED_WOOD20: return f(FamChainedWood<20>{}, ic<32>{}, ic<32>{});
@@ -332,8 +323,6 @@ int with_family(int family, int nt, F&& f) {
     return fail(ENLSIPB200_EINVAL, "unknown family id");
 #endif
 }
-
-static int gp_nt() { const char* e = getenv("ENLSIP_GP_NT"); int v = e ? atoi(e) : 512; return (v == 480 || v == 448 || v == 224 || v == 128 || v == 64) ? v : 512; }
 
 Options make_options(const enlsipb200_options* o, int n, int m) {
     enlsipb200_options d;
@@ -382,7 +371,7 @@ int enlsipb200_create(int family, const double* x_low, const double* x_upp, int 
     if (!out) return fail(ENLSIPB200_EINVAL, "out is NULL");
     *out = nullptr;
     FamilyInfo fi{0, 0, 0, 0, 0};
-    int known = with_family(family, 0, [&](auto fam, auto, auto) {
+    int known = with_family(family, [&](auto fam, auto, auto) {
         using Fm = decltype(fam);
         fi = {Fm::N, Fm::M, Fm::Q, Fm::NI, Fm::MAXB};
         return 0;
@@ -421,7 +410,7 @@ int enlsipb200_create(int family, const double* x_low, const double* x_upp, int 
         for (int i = 0; i < 128; ++i) tt[i] = FamGaussPeaks::abscissa(i);
         if (cudaMemcpyToSymbol(g_gp_t, tt, sizeof(tt)) != cudaSuccess) { enlsipb200_destroy(h); return fail(ENLSIPB200_ECUDA, "cudaMemcpyToSymbol"); }
     }
-    rc = with_family(family, gp_nt(), [&](auto fam, auto g_, auto nt_) {
+    rc = with_family(family, [&](auto fam, auto g_, auto nt_) {
         return configure<decltype(fam), decltype(g_)::value, decltype(nt_)::value>(h);
     });
     if (rc != 0) { enlsipb200_destroy(h); return rc; }
@@ -514,7 +503,7 @@ int enlsipb200_solve_batch(enlsipb200_handle h, long long B, const double* x0, c
         a.x0 = x0;
         a.out.x = x; a.out.f = f; a.out.exit_code = exit_code; a.out.status = status; a.out.iters = iters;
         a.out.nact = nact; a.out.active = active; a.out.counters = counters; a.out.trace = trace;
-        int rc = with_family(h->family, h->nt, [&](auto fam, auto g_, auto nt_) {
+        int rc = with_family(h->family, [&](auto fam, auto g_, auto nt_) {
             return launch<decltype(fam), decltype(g_)::value, decltype(nt_)::value>(h, a, st);
         });
         if (rc != 0) return rc;
@@ -587,7 +576,7 @@ int enlsipb200_solve_batch(enlsipb200_handle h, long long B, const double* x0, c
         ac.out.x = d_x + off * n; ac.out.f = d_f + off; ac.out.exit_code = d_ec + off; ac.out.status = d_st + off;
         ac.out.iters = d_it + off; ac.out.nact = d_na + off; ac.out.active = d_act + off * lmax; ac.out.counters = d_cnt + off * 2;
         ac.out.trace = trace ? d_tr + (size_t)off * trace_cap * row_w : nullptr;
-        int rc = with_family(h->family, h->nt, [&](auto fam, auto g_, auto nt_) {
+        int rc = with_family(h->family, [&](auto fam, auto g_, auto nt_) {
             return launch<decltype(fam), decltype(g_)::value, decltype(nt_)::value>(h, ac, st, c == 0, c == nchunk - 1);
         });
         if (rc != 0) return rc;
@@ -645,7 +634,7 @@ static int eval_or_step(enlsipb200_handle h, long long B, const double* x, const
     a.bnd = h->bnd;
     a.r = r; a.J = J; a.c = c; a.A = A;
     a.step = step; a.p = p; a.lam = lam; a.active = active; a.info = info;
-    int rc = with_family(h->family, h->nt, [&](auto fam, auto g_, auto nt_) {
+    int rc = with_family(h->family, [&](auto fam, auto g_, auto nt_) {
         using Fm = decltype(fam);
         constexpr int G = decltype(g_)::value, NT = decltype(nt_)::value;
         auto kern = enlsip_eval_batch_kernel<Fm, G, NT>;

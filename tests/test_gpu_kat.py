@@ -136,11 +136,11 @@ def test_trsv_coop_vs_dtrtrs(L, frows, k, kind):
     assert np.abs(res).max() <= 1e-12 * (np.abs(R).max() * np.abs(out).max() * k ** 0.5 + np.abs(v).max())
 
 
-@pytest.mark.parametrize("env", [{"ENLSIP_QR_PANEL": "graph"}, {"ENLSIP_QR_TRAIL": "dmma"}])
+@pytest.mark.parametrize("env", [{"ENLSIP_QR_PANEL": "graph"}])
 def test_qrcp_alternative_paths_vs_dgeqp3(env):
-    """The selectable forms of the blocked QRCP stay correct: three kernels per column inside a CUDA graph (also the path
-    of matrices with more than 32768 rows) and the DMMA trailing update.  The switches are read once per process, so the
-    factorisation runs in a child process (tools/qrcp_time.py compares pivots, R and tau with LAPACK)."""
+    """The graph form of the blocked QRCP stays correct: three kernels per column inside a CUDA graph (the path of
+    matrices with more than 32768 rows).  The switch is read once per process, so the factorisation runs in a child
+    process (tools/qrcp_time.py compares pivots, R and tau with LAPACK)."""
     import os
     import re
     import subprocess

@@ -312,30 +312,6 @@ def test_chained_rosenbrock_reference_size_vs_oracle(E, n, jac):
     mod.close()
 
 
-def test_tsqr_tma_trailing_kernel_matches():
-    """The TMA-fed trailing updates (ENLSIP_TRAIL=3: producer warp, cp.async.bulk + mbarrier; ENLSIP_TRAIL=4: one
-    cp.async.bulk.tensor.2d box per 16 x 32 tile through a tensor map, 8 or 16 math warps) against the default cp.async
-    kernel: mode 3 returns its bits, mode 4 agrees to rounding.  The switch is read once per process, so the variant runs in a child process."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = ("import sys, numpy as np; sys.path.insert(0, %r); import enlsip_jl_b200 as E\n"
-            "d = E.synth.gen_single_index(70000, 128, 32, seed=2)\n"
-            "mod = E.LargeCnlsModel('single_index', d['x0'], d, m_global=70000)\n"
-            "R, _, _ = mod.factor(d['x0']); sys.stdout.buffer.write(R.tobytes())\n" % root)
-    outs = []
-    for mode, nw in (("2", "8"), ("3", "8"), ("4", "8"), ("4", "16")):
-        env = dict(os.environ, ENLSIP_TRAIL=mode, ENLSIP_TMAP_NW=nw)
-        outs.append(subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, check=True).stdout)
-    a, b, c8, c16 = (np.frombuffer(o, dtype=np.float64) for o in outs)
-    assert a.size == 129 * 129 and np.array_equal(a.view(np.uint64), b.view(np.uint64))
-    # ENLSIP_TRAIL=4 (tensor-map TMA, 128-byte swizzle): the k order inside a DMMA chain follows the swizzled layout,
-    # so the sums are the same up to rounding, not to the bit
-    for c in (c8, c16):
-        assert c.size == a.size and np.abs(c - a).max() <= 1e-12 * np.abs(a).max()
-
-
 @pytest.mark.parametrize("m,n,nb,seed", [(3000, 32, 8, 41), (5000, 64, 16, 42)])
 def test_single_index_forward_difference_jacobian_vs_oracle(E, m, n, nb, seed):
     """The FD-Jacobian variant of the tall family (SURVEY.md 8d, C4 inputs; jac_forward_diff, cnls_model.jl:65-82): the
