@@ -21,6 +21,7 @@ OBJ_DIR = os.path.join(_HERE, "lib", "obj")
 FAMILY_SINGLE_INDEX = 16
 FAMILY_LARGE_CHAINED_ROSENBROCK = 17
 LARGE_FACTOR_TSQR = 0x100   # OR-ed into the family: row families factor [J | r] with the TSQR and may be row-sharded
+LARGE_MIDSIZE = 0x200       # OR-ed into the family: a row family with n + m < 1000, solved with Newton steps (EF:2658)
 
 FAMILY_HS65 = 0
 FAMILY_GAUSS_PEAKS = 1
@@ -41,7 +42,7 @@ EXPORTS = ["enlsipb200_version", "enlsipb200_last_error", "enlsipb200_default_op
            "enlsipb200_large_set_data", "enlsipb200_large_comm_id", "enlsipb200_large_comm_init",
            "enlsipb200_large_solve", "enlsipb200_large_factor", "enlsipb200_large_stats",
            "enlsipb200_dense_qrcp", "enlsipb200_dense_qr", "enlsipb200_dense_mulq", "enlsipb200_dense_vecop",
-           "enlsipb200_dense_gemv", "enlsipb200_dense_last_ms"]
+           "enlsipb200_dense_gemv", "enlsipb200_dense_potrf", "enlsipb200_dense_last_ms"]
 
 
 class Options(ctypes.Structure):
@@ -120,6 +121,7 @@ def _bind(L, large=True):
         L.enlsipb200_dense_mulq.argtypes = [ci, ci, ci, vp, vp, vp, ci]
         L.enlsipb200_dense_vecop.argtypes = [ci, ci, ci, vp, vp, vp, ci]
         L.enlsipb200_dense_gemv.argtypes = [ci, ci, ci, vp, ci, vp, ctypes.c_double, vp, ctypes.c_double, vp, ci]
+        L.enlsipb200_dense_potrf.argtypes = [ci, vp, vp, ci]
         L.enlsipb200_dense_last_ms.restype = ctypes.c_float
     return L
 

@@ -405,6 +405,15 @@ struct LargeHandle : LargeOps, SmallBackend {
     double* dJrow = nullptr;
     int nt = 0;                       // columns the TSQR factors: n rounded up to 32 on that path, n otherwise
     std::vector<double> hxcur;        // the point of the last eval (linesearch trial points are x + alpha p)
+    // ENLSIPB200_LARGE_MIDSIZE: second derivatives on (Newton steps, EF:348-423).  n x n matrices G, E = Q1' G Q1 and its
+    // scratch, the k2 x n block [W21 | W22] and the Cholesky factor; r at x; x / lam / active of the Hessian; the bound
+    // values (x_low then x_upp, in the order of dbidx).  Allocated with the handle, midsize handles only.
+    bool midsize = false;
+    double *dG = nullptr, *dE = nullptr, *dWn = nullptr, *dU = nullptr, *dhr = nullptr, *dxn = nullptr, *dlamn = nullptr, *dbval = nullptr;
+    int *dactn = nullptr, *dinfo = nullptr;
+    cudaEvent_t eh0 = nullptr, eh1 = nullptr;
+    double ms_hess = 0;
+    long long n_newton = 0;
     long long m_local = 0, rows_pad = 0, dT_subtiles = 0;
     int ld = 0, rr_rows = 0;
     SingleIndexConstraints sc;
@@ -450,6 +459,11 @@ struct LargeHandle : LargeOps, SmallBackend {
             if (p) cudaFree(p);
         if (dpQ) cudaFree(dpQ);
         dQ = dJkeep = dtauQ = dcu = dJrow = nullptr; dpQ = nullptr; gown[0] = gown[1] = nullptr;
+        for (double** p : {&dG, &dE, &dWn, &dU, &dhr, &dxn, &dlamn, &dbval}) { if (*p) cudaFree(*p); *p = nullptr; }
+        for (int** p : {&dactn, &dinfo}) { if (*p) cudaFree(*p); *p = nullptr; }
+        if (eh0) cudaEventDestroy(eh0);
+        if (eh1) cudaEventDestroy(eh1);
+        eh0 = eh1 = nullptr;
         for (int* p : {dpA, dipA, dpL, dipL, dp2, dip2, dact, dbidx, qw.flags, qw.pidx})
             if (p) cudaFree(p);
         qw.drop_graphs();
@@ -571,7 +585,23 @@ struct LargeHandle : LargeOps, SmallBackend {
             LCU(cudaMalloc(&dbidx, sizeof(int) * idx.size()));
             LCU(cudaMemcpyAsync(dbidx, idx.data(), sizeof(int) * idx.size(), cudaMemcpyHostToDevice, st));
             si_jac_bounds_kernel<<<(nlo + nup + 255) / 256, 256, 0, st>>>(dbidx, nlo, nup, gv ? ncu : sc.nb, n, dArow);
+            if (midsize) {
+                std::vector<double> val(sc.lo_val);
+                val.insert(val.end(), sc.up_val.begin(), sc.up_val.end());
+                LCU(cudaMalloc(&dbval, sizeof(double) * val.size()));
+                LCU(cudaMemcpyAsync(dbval, val.data(), sizeof(double) * val.size(), cudaMemcpyHostToDevice, st));
+            }
             LCU(cudaStreamSynchronize(st));
+        }
+        if (midsize) {
+            const size_t nn = (size_t)n * n;
+            for (double** p : {&dG, &dE, &dWn, &dU}) LCU(cudaMalloc(p, sizeof(double) * nn));
+            LCU(cudaMalloc(&dhr, sizeof(double) * (size_t)m_local));
+            LCU(cudaMalloc(&dxn, sizeof(double) * n));
+            LCU(cudaMalloc(&dlamn, sizeof(double) * (l + 1)));
+            LCU(cudaMalloc(&dactn, sizeof(int) * (l + 1)));
+            LCU(cudaMalloc(&dinfo, sizeof(int)));
+            LCU(cudaEventCreate(&eh0)); LCU(cudaEventCreate(&eh1));
         }
         LCU(cudaGetLastError());
         return 0;
@@ -1185,8 +1215,98 @@ struct LargeHandle : LargeOps, SmallBackend {
         sm_sync();
         return hst[0];
     }
+    // EF:348-423 (the driver has checked the sizes): p1 from R_A' (t == rankA) or F_L11 (t > rankA), G at x,
+    // E = (Q1' G) Q1 -- G is symmetric, so Q1' G = (G Q1)' --, permuted by F_L11.p when t > rankA, [W21 | W22] from E and
+    // J~Q1 (J2'J2, J2'J1 and J2'r are invariant under the left orthogonal factor of [J | r], so the compressed problem gives
+    // them), d = -W21 p1 - J2' r~, the upper Cholesky factor of (W22 + W22') / 2, two triangular solves, p = Q1 [p1; p2].
+    int newton_direction(const double* x, const Vec& lam, const int* active, int t, int rankA, const Vec& Ccx, Vec& p) override {
+        if (!midsize) return -1;
+        SmallScope sc_(this);
+        need_ws(t);
+        ensure_jq1();
+        const int mt = n + 1, k2 = n - rankA;
+        const double* rtd = dJc + (size_t)mt * n;
+        double* p1 = dvec[2];                                            // rankA entries
+        if (t > 0) {
+            Vec b0(t);
+            for (int i = 0; i < t; ++i) b0[i] = -Ccx[hpA[i]];
+            up(dvec[0], b0.data(), t);
+            if (t == rankA) {
+                k_trsv_upperT(dFA, n, t, dvec[0]);                      // R_A' p1 = -c[P]
+                p1 = dvec[0];
+            } else {
+                k_reflect(dFL, fl_rows, fl_k, dtauL, dvec[0], 1);       // b = Q_L11' (-c[P])
+                k_copy_pad(dvec[1], dvec[0], rankA, rankA);
+                k_trsv_upper(dFL, fl_rows, rankA, dvec[1]);              // R11 \ b[1:rankA]
+                if (rankA > 0) {
+                    sm_check(cudaMemsetAsync(dvec[2], 0, sizeof(double) * rankA, st), "memset");
+                    enl_small::scatter_perm_kernel<<<(rankA + 255) / 256, 256, 0, st>>>(dvec[2], dvec[1], dpL, rankA, rankA);
+                    ++launches;
+                }
+            }
+        }
+        if (hessian(x, lam.data(), active, t, dG) != 0) throw std::runtime_error(g_lerr);
+        if (fa_k > 0) {
+            double* TA = wy_t_of(dFA, n, fa_k, dtauA);
+            launches += enl_small::mulq_device(dG, n, n, dFA, n, fa_k, dtauA, ww, st, TA, false);   // G Q1
+            dim3 grid((n + 31) / 32, (n + 31) / 32), block(32, 8);
+            enl_small::transpose_kernel<<<grid, block, 0, st>>>(dG, n, dE);                        // Q1' G
+            ++launches;
+            launches += enl_small::mulq_device(dE, n, n, dFA, n, fa_k, dtauA, ww, st, TA, false);   // (Q1' G) Q1
+            n_dev_mulq += 2;
+        } else {
+            sm_check(cudaMemcpyAsync(dE, dG, sizeof(double) * (size_t)n * n, cudaMemcpyDeviceToDevice, st), "D2D");
+        }
+        const long long nw = (long long)k2 * n;
+        enl_small::newton_assemble_kernel<<<(unsigned)std::min<long long>((nw + 7) / 8, 148 * 16), 256, 0, st>>>(
+            dE, n, rankA, t > rankA ? dpL : nullptr, dJQ1, mt, dWn);
+        const long long nu = (long long)k2 * k2;
+        enl_small::newton_sym_kernel<<<(unsigned)((nu + 255) / 256), 256, 0, st>>>(dWn, k2, rankA, dU);
+        launches += 2 + enl_small::gemv_t(dJQ1 + (size_t)rankA * mt, mt, mt, k2, rtd, dvec[3], st);   // J2' r~
+        launches += enl_small::gemv_n(dWn, k2, k2, rankA, p1, -1.0, dvec[3], -1.0, dvec[4], st);     // d = -W21 p1 - J2' r~
+        if (enl_small::potrf_upper(dU, k2, k2, dinfo, st) < 0) throw std::runtime_error("Newton step: reduced Hessian too large");
+        ++launches;
+        int info = 0;
+        sm_check(cudaMemcpyAsync(hsti, dinfo, sizeof(int), cudaMemcpyDeviceToHost, st), "D2H");
+        sm_sync();
+        info = hsti[0];
+        ++n_newton;
+        if (info != 0) {
+            p.assign(n, 0.0);
+            return 1;
+        }
+        k_trsv_upperT(dU, k2, k2, dvec[4]);
+        k_trsv_upper(dU, k2, k2, dvec[4]);
+        if (rankA > 0) sm_check(cudaMemcpyAsync(dvec[5], p1, sizeof(double) * rankA, cudaMemcpyDeviceToDevice, st), "D2D");
+        sm_check(cudaMemcpyAsync(dvec[5] + rankA, dvec[4], sizeof(double) * k2, cudaMemcpyDeviceToDevice, st), "D2D");
+        k_reflect(dFA, n, fa_k, dtauA, dvec[5], 0);                     // p = Q1 [p1; p2]
+        down(0, dvec[5], n);
+        sm_sync();
+        p.assign(hst, hst + n);
+        return 0;
+    }
 
     // ---- LargeOps ----
+    // G (device, n x n) at x by lg_hessian_kernel over the family's rows and the active constraints; its device time
+    // (CUDA events) adds to the Hessian ms of enlsipb200_large_stats
+    int hessian(const double* x, const double* lam, const int* active, int t, double* G) override {
+        if (!midsize || !gv) return lfail(ENLSIPB200_EINVAL, "second derivatives: row families created with ENLSIPB200_LARGE_MIDSIZE only");
+        LCU(cudaMemcpyAsync(dxn, x, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+        if (t > 0) {
+            LCU(cudaMemcpyAsync(dlamn, lam, sizeof(double) * t, cudaMemcpyHostToDevice, st));
+            LCU(cudaMemcpyAsync(dactn, active, sizeof(int) * t, cudaMemcpyHostToDevice, st));
+        }
+        LCU(cudaEventRecord(eh0, st));
+        gv->hessian(st, n, m_local, dxn, gd[0], gd[1], dhr, ncu, (int)sc.lo_idx.size(), dbidx, dbval, t, dactn, dlamn, G);
+        launches += 2;
+        LCU(cudaEventRecord(eh1, st));
+        LCU(cudaStreamSynchronize(st));
+        LCU(cudaGetLastError());
+        float ms = 0.0f;
+        LCU(cudaEventElapsedTime(&ms, eh0, eh1));
+        ms_hess += ms;
+        return 0;
+    }
     // the host-matrix forms of new_point! belong to the CPU test backend; the product keeps A and J~ in HBM
     // (new_point_eval / new_point_compress above) and has no host path to fall back to
     int eval_point(const double*, double*, double*, double*, double*) override {
@@ -1296,7 +1416,8 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
     if (!out) return lfail(ENLSIPB200_EINVAL, "out is NULL");
     *out = nullptr;
     const bool want_tsqr = (family & ENLSIPB200_LARGE_FACTOR_TSQR) != 0;
-    family &= ~ENLSIPB200_LARGE_FACTOR_TSQR;
+    const bool midsize = (family & ENLSIPB200_LARGE_MIDSIZE) != 0;
+    family &= ~(ENLSIPB200_LARGE_FACTOR_TSQR | ENLSIPB200_LARGE_MIDSIZE);
     const GenericVt* gv = nullptr;
 #if defined(ENL_LARGE_USER_FAMILY)
     if (family == ENLSIPB200_FAMILY_USER) gv = generic_vt<LFamUser>();
@@ -1305,6 +1426,16 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
     if (family == ENLSIPB200_FAMILY_LARGE_CHAINED_ROSENBROCK) gv = generic_vt<LFamChainedRosenbrock>();
     else if (family != ENLSIPB200_FAMILY_SINGLE_INDEX) return lfail(ENLSIPB200_EINVAL, "unknown large-regime family");
 #endif
+    if (midsize) {
+        if (!gv)
+            return lfail(ENLSIPB200_EINVAL, "ENLSIPB200_LARGE_MIDSIZE: row families only (the single-index family has no Newton step)");
+        if (want_tsqr)
+            return lfail(ENLSIPB200_EINVAL, "ENLSIPB200_LARGE_MIDSIZE and ENLSIPB200_LARGE_FACTOR_TSQR do not combine (mid-size problems are not sharded)");
+        if ((long long)n + m_global >= 1000)
+            return lfail(ENLSIPB200_EINVAL, "ENLSIPB200_LARGE_MIDSIZE: n + m < 1000 required (larger problems run without second derivatives, EF:2658)");
+        if (m_global < (long long)n + 1)
+            return lfail(ENLSIPB200_EINVAL, "ENLSIPB200_LARGE_MIDSIZE: m >= n + 1 required ([J | r] is compressed by a QR of at least n + 1 rows)");
+    }
     if (gv) {
         if (n < 3) return lfail(ENLSIPB200_EINVAL, "n >= 3 required");
         if (want_tsqr) {
@@ -1320,7 +1451,7 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
         return lfail(ENLSIPB200_EINVAL, "single-index family: n <= 6144 (x is staged in 48 KB of shared memory)");
     }
     if (m_local < 0 || m_global < m_local || nb < 0 || 4 * nb > n) return lfail(ENLSIPB200_EINVAL, "bad sizes");
-    if ((long long)n + m_global < 1000)
+    if ((long long)n + m_global < 1000 && !midsize)
         return lfail(ENLSIPB200_EINVAL, "n + m < 1000: second derivatives stay on in the reference (EF:2658); use the batched engine");
     if (nb > 0 && !rho) return lfail(ENLSIPB200_EINVAL, "rho is NULL");
     int ndev = 0;
@@ -1337,6 +1468,7 @@ int enlsipb200_large_create(int family, int n, long long m_local, long long m_gl
     h->l = h->sc.l(); h->q = h->sc.q();
     h->gv = gv;
     h->tsqr_rows = gv && want_tsqr;
+    h->midsize = midsize;
     h->rows_joined = !h->tsqr_rows || m_local == m_global;
     if (gv) {
         h->q = gv->q_of(n);
@@ -1471,6 +1603,7 @@ int enlsipb200_large_solve(enlsipb200_large hh, const double* x0, const enlsipb2
     opt.max_iter = o->max_iter;
     opt.scaling = o->scaling;
     opt.time_limit = o->time_limit;
+    opt.second_derivatives = h->midsize;
     double abs_tol = (o->abs_tol == o->abs_tol) ? o->abs_tol : EPS;
     double rel_tol = (o->rel_tol == o->rel_tol) ? o->rel_tol : sqrt(abs_tol);
     opt.eps_rel = rel_tol;
@@ -1529,10 +1662,10 @@ int enlsipb200_large_factor(enlsipb200_large hh, const double* x, double* R, flo
 int enlsipb200_large_stats(enlsipb200_large hh, double* out, int count) {
     LargeHandle* h = LH(hh);
     if (!h || !out) return lfail(ENLSIPB200_EINVAL, "NULL argument");
-    double v[13] = {(double)h->n_newpoint, h->ms_build, h->ms_tsqr, h->ms_ls, h->ms_total, (double)h->n_ls,
+    double v[15] = {(double)h->n_newpoint, h->ms_build, h->ms_tsqr, h->ms_ls, h->ms_total, (double)h->n_ls,
                     (double)h->launches, (double)h->rows_pad, (double)h->n_dev_qrcp, (double)h->n_dev_mulq, h->ms_small,
-                    (double)h->n_factor, (double)h->n_ws_grow};
-    for (int i = 0; i < count && i < 13; ++i) out[i] = v[i];
+                    (double)h->n_factor, (double)h->n_ws_grow, (double)h->n_newton, h->ms_hess};
+    for (int i = 0; i < count && i < 15; ++i) out[i] = v[i];
     return 0;
 }
 
@@ -1585,6 +1718,34 @@ int enlsipb200_dense_qr(int rows, int cols, double* f, double* tau, int device) 
 }
 
 float enlsipb200_dense_last_ms(void) { return g_dense_ms; }
+
+// Known-answer hook of the Newton step's Cholesky factorisation (enl_small::potrf_upper): a [n x n] column major, upper
+// triangle in, U out (dpotrf('U')); info as dpotrf's
+int enlsipb200_dense_potrf(int n, double* a, int* info, int device) {
+    if (n < 1 || n > enl_small::VEC_STAGE_MAX || !a || !info) return lfail(ENLSIPB200_EINVAL, "bad arguments");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return lfail(ENLSIPB200_ENOGPU, "no CUDA device");
+    if (device < 0) LCU(cudaGetDevice(&device));
+    LCU(cudaSetDevice(device));
+    DenseScratch S;
+    double* da = nullptr;
+    int* dinfo = nullptr;
+    if (!S.get(&da, (size_t)n * n) || !S.get(&dinfo, 1)) return lfail(ENLSIPB200_ENOMEM, "cudaMalloc");
+    LCU(cudaMemcpy(da, a, sizeof(double) * (size_t)n * n, cudaMemcpyHostToDevice));
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    LCU(cudaEventCreate(&ev0)); LCU(cudaEventCreate(&ev1));
+    LCU(cudaEventRecord(ev0, nullptr));
+    enl_small::potrf_upper(da, n, n, dinfo, nullptr);
+    LCU(cudaEventRecord(ev1, nullptr));
+    cudaError_t es = cudaDeviceSynchronize();
+    if (es == cudaSuccess) es = cudaGetLastError();
+    cudaEventElapsedTime(&g_dense_ms, ev0, ev1);
+    cudaEventDestroy(ev0); cudaEventDestroy(ev1);
+    LCU(es);
+    LCU(cudaMemcpy(a, da, sizeof(double) * (size_t)n * n, cudaMemcpyDeviceToHost));
+    LCU(cudaMemcpy(info, dinfo, sizeof(int), cudaMemcpyDeviceToHost));
+    return 0;
+}
 
 int enlsipb200_dense_mulq(int mr, int nq, int k, const double* f, const double* tau, double* M, int device) {
     if (mr < 1 || nq < 1 || k < 0 || k > nq || !f || !tau || !M) return lfail(ENLSIPB200_EINVAL, "bad arguments");

@@ -180,6 +180,88 @@ __global__ void lg_jac_cons_kernel(int n, int nc, const double* __restrict__ x, 
     Arow[e] = v;
 }
 
+// r = the residuals at x (the Newton step's weights r_i; the factorisation has overwritten the build's copy in [J | r])
+template <class F>
+__global__ void __launch_bounds__(256) lg_res_kernel(int n, long long m, const double* __restrict__ x, const double* __restrict__ d0,
+                                                     const double* __restrict__ d1, double* __restrict__ r) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (long long)gridDim.x * blockDim.x)
+        r[i] = F::residual(i, n, XPlain{x}, d0, d1);
+}
+
+// x + sj e_j + sk e_k with coordinate j moved first, each move rounded (EF:259-266: xw[j] += ej; xw[k] += ek), so
+// that j == k moves the coordinate twice
+struct XPair {
+    const double* x; int j; double sj; int k; double sk;
+    __device__ __forceinline__ double operator[](int q) const {
+        double v = x[q];
+        if (q == j) v = __dadd_rn(v, sj);
+        if (q == k) v = __dadd_rn(v, sk);
+        return v;
+    }
+};
+
+// constraint kk (0-based, the order of the reference's c: the family's own, then [x - x_low ; x_upp - x]) at a point
+template <class F, class X>
+__device__ __forceinline__ double lg_constraint_at(int kk, int n, const X& xa, const double* d0, const double* d1, int ncu,
+                                                   int nlo, const int* bidx, const double* bval) {
+    if (kk < ncu) return F::constraint(kk, n, xa, d0, d1);
+    const int e = kk - ncu;
+    return e < nlo ? __dsub_rn(xa[bidx[e]], bval[e]) : __dsub_rn(bval[e], xa[bidx[e]]);
+}
+
+// The Hessian of the Lagrangian for the Newton step (EF:243-328, hessian_res! / hessian_cons!):
+//     G[k, j] = sum_i r_i (f1 - f2 - f3 + f4)_i / (4 ej ek)  -  sum_{a < t} lam_a (c1 - c2 - c3 + c4)_{active_a} / (4 ek ej)
+// with f1..f4 (c1..c4) the residuals (constraints) at the four stencil points (+ej, +ek), (-ej, +ek), (+ej, -ek),
+// (-ej, -ek) in coordinates (j, k), e. = max(|x.|, 1) eps^(1/3).  One CTA per pair j <= k, threads over the rows and
+// the active constraints, both sums reduced in a fixed order (no atomics: the same bits every run); G[k, j] and G[j, k]
+// get the same value.  Bound rows are evaluated like every other constraint: (x_j +- e) - x_low_j need not round to
+// an exact zero second difference.
+constexpr int LG_HESS_THREADS = 128;
+template <class F>
+__global__ void __launch_bounds__(LG_HESS_THREADS) lg_hessian_kernel(int n, long long m, const double* __restrict__ x,
+                                                                     const double* __restrict__ d0, const double* __restrict__ d1,
+                                                                     const double* __restrict__ r, int ncu, int nlo,
+                                                                     const int* __restrict__ bidx, const double* __restrict__ bval,
+                                                                     int t, const int* __restrict__ active,
+                                                                     const double* __restrict__ lam, double* __restrict__ G) {
+    constexpr double E1 = 6.055454452393343e-06;   // eps^(1/3)
+    const long long b = blockIdx.x;
+    int k = (int)((sqrt(8.0 * (double)b + 1.0) - 1.0) * 0.5);
+    while ((long long)k * (k + 1) / 2 > b) --k;
+    while ((long long)(k + 1) * (k + 2) / 2 <= b) ++k;
+    const int j = (int)(b - (long long)k * (k + 1) / 2);
+    const double ek = __dmul_rn(fmax(fabs(x[k]), 1.0), E1);
+    const double ej = __dmul_rn(fmax(fabs(x[j]), 1.0), E1);
+    const XPair p1{x, j, ej, k, ek}, p2{x, j, -ej, k, ek}, p3{x, j, ej, k, -ek}, p4{x, j, -ej, k, -ek};
+    double sr = 0.0, sc = 0.0;
+    for (long long i = threadIdx.x; i < m; i += blockDim.x) {
+        const double f1 = F::residual(i, n, p1, d0, d1), f2 = F::residual(i, n, p2, d0, d1);
+        const double f3 = F::residual(i, n, p3, d0, d1), f4 = F::residual(i, n, p4, d0, d1);
+        sr = fma(__dadd_rn(__dsub_rn(__dsub_rn(f1, f2), f3), f4), r[i], sr);
+    }
+    for (int a = threadIdx.x; a < t; a += blockDim.x) {
+        const int kk = active[a] - 1;
+        const double c1 = lg_constraint_at<F>(kk, n, p1, d0, d1, ncu, nlo, bidx, bval);
+        const double c2 = lg_constraint_at<F>(kk, n, p2, d0, d1, ncu, nlo, bidx, bval);
+        const double c3 = lg_constraint_at<F>(kk, n, p3, d0, d1, ncu, nlo, bidx, bval);
+        const double c4 = lg_constraint_at<F>(kk, n, p4, d0, d1, ncu, nlo, bidx, bval);
+        sc = fma(__dadd_rn(__dsub_rn(__dsub_rn(c1, c2), c3), c4), lam[a], sc);
+    }
+    __shared__ double sh[LG_HESS_THREADS / 32][2];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    sr = g_warp_sum(sr);
+    sc = g_warp_sum(sc);
+    if (lane == 0) { sh[w][0] = sr; sh[w][1] = sc; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double tr = 0.0, tc = 0.0;
+        for (int ww = 0; ww < LG_HESS_THREADS / 32; ++ww) { tr += sh[ww][0]; tc += sh[ww][1]; }
+        const double g = tr / (4 * ej * ek) - tc / (4.0 * ek * ej);
+        G[(size_t)j * n + k] = g;
+        G[(size_t)k * n + j] = g;
+    }
+}
+
 // host-side dispatch table of one family
 struct GenericVt {
     long long (*m_of)(int);
@@ -192,6 +274,9 @@ struct GenericVt {
                const double* d0, const double* d1, const double* r, const double* Jp, int with_coeffs, double* part);
     void (*cons)(cudaStream_t st, int n, int nc, const double* x, const double* d0, const double* d1, double* c);
     void (*jac_cons)(cudaStream_t st, int n, int nc, const double* x, const double* d0, const double* d1, int fd, const double* c0, double* Arow);
+    // r (m) at x, then G (n x n, column major) by lg_hessian_kernel
+    void (*hessian)(cudaStream_t st, int n, long long m, const double* x, const double* d0, const double* d1, double* r, int ncu,
+                    int nlo, const int* bidx, const double* bval, int t, const int* active, const double* lam, double* G);
 };
 template <class F>
 const GenericVt* generic_vt() {
@@ -214,6 +299,12 @@ const GenericVt* generic_vt() {
         [](cudaStream_t st, int n, int nc, const double* x, const double* d0, const double* d1, int fd, const double* c0, double* Arow) {
             const long long ne = (long long)nc * n;
             if (ne > 0) lg_jac_cons_kernel<F><<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(n, nc, x, d0, d1, fd, c0, Arow);
+        },
+        [](cudaStream_t st, int n, long long m, const double* x, const double* d0, const double* d1, double* r, int ncu, int nlo,
+           const int* bidx, const double* bval, int t, const int* active, const double* lam, double* G) {
+            lg_res_kernel<F><<<(unsigned)((m + 255) / 256), 256, 0, st>>>(n, m, x, d0, d1, r);
+            const long long pairs = (long long)n * (n + 1) / 2;
+            lg_hessian_kernel<F><<<(unsigned)pairs, LG_HESS_THREADS, 0, st>>>(n, m, x, d0, d1, r, ncu, nlo, bidx, bval, t, active, lam, G);
         }};
     return &vt;
 }

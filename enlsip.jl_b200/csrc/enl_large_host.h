@@ -19,8 +19,10 @@
 //     surviving side effects;  J*F_A.Q is formed once per factorisation (EF:219, 526, 1249);
 //   * aliasing schedule of Iteration.rx / .cx (SURVEY.md T1) modelled by snapshot-or-live scalars;
 //   * where Julia would throw / loop forever the solve ends with exit code -99 / -98.
-// Newton steps (EF:348-423) do not exist in this regime: `second_derivatives` is forced off when
-// n + m >= 1000 (EF:2658), and the entry point rejects smaller problems (they belong to the batched engine).
+// Newton steps (EF:348-423) follow LargeOptions::second_derivatives, which is the reference's `n + m < 1000` (EF:2658):
+// the entry point turns it on only for row families created with ENLSIPB200_LARGE_MIDSIZE, refuses that flag when
+// n + m >= 1000, and refuses n + m < 1000 without it.  The driver decides the reference's size situations of the Newton
+// step; the Hessian (LargeOps::hessian) and the linear algebra (SmallBackend::newton_direction) belong to the backend.
 #pragma once
 #include <float.h>
 #include <math.h>
@@ -342,6 +344,13 @@ struct LargeOps {
     // on it leave each other alone in the next collective.  Sharded backends return the mean over the ranks (one sum
     // all-reduce of elapsed / nranks).
     virtual double agreed_elapsed(double local_elapsed) { return local_elapsed; }
+    // Newton step: G = sum_i r_i Hess r_i - sum_{a < t} lam[a] Hess c_{active[a]} at x by the reference's central differences
+    // (EF:243-328), n x n column major into G, which lives where the backend keeps its matrices.  Backends without second
+    // derivatives keep this default.
+    virtual int hessian(const double* x, const double* lam, const int* active, int t, double* G) {
+        (void)x; (void)lam; (void)active; (void)t; (void)G;
+        return -1;
+    }
 };
 
 struct LargeOptions {
@@ -349,6 +358,7 @@ struct LargeOptions {
     int scaling = 0;
     double time_limit = 1e3;
     double eps_abs = 1e-10, eps_rel = SQRT_EPS, eps_x = SQRT_EPS, eps_c = SQRT_EPS, eps_rank = SQRT_EPS;
+    bool second_derivatives = false;   // Newton steps (method code 2) are taken, EF:2658
 };
 
 struct IterTraceL {   // one record per executed iteration (mirrors oracle IterTrace)
@@ -448,6 +458,14 @@ struct SmallBackend {
     virtual void products(const Vec& p, int t, Vec& Jp, Vec& Ap, Vec& active_Ap) = 0;
     // EF:2497: ||C.A' C.cx||
     virtual double At_c_norm(int t, const Vec& Ccx) = 0;
+    // EF:348-423 (sizes validated by the driver): p1 from R_A' \ (-c[P]) (t == rankA) or P_L11 [R11 \ (Q_L11' (-c[P]))[1:rankA]]
+    // (t > rankA); E = (Q1' G) Q1 with G = LargeOps::hessian at x, E[P2, P2] when t > rankA; W22 = E22 + J2'J2,
+    // W21 = E21 + J2'J1, d = -W21 p1 - J2' r; the upper Cholesky factor U of (W22 + W22') / 2 (dpotrf); p = Q1 [p1; U \ (U' \ d)].
+    // Returns 0, 1 when the Cholesky factorisation fails (p = 0), or -1 when the backend has no Newton step (this default).
+    virtual int newton_direction(const double* x, const Vec& lam, const int* active, int t, int rankA, const Vec& Ccx, Vec& p) {
+        (void)x; (void)lam; (void)active; (void)t; (void)rankA; (void)Ccx; (void)p;
+        return -1;
+    }
 };
 
 // Host-memory backend: the CPU test path (oracle/hostport/largeport.cpp).  The product never instantiates it.
@@ -1128,8 +1146,28 @@ public:
         return method_code;
     }
 
+    // EF:348-423: the reference's throws depend on sizes and diag(R) only and are decided here; true when the Cholesky
+    // factorisation of the reduced Hessian fails (p = 0)
+    bool newton_search_direction(const Vec& x, const Vec& lam, int rankA, Vec& p) {
+        const int t = W.t;
+        if (t == rankA) {     // LowerTriangular(F_A.R') \ b
+            if (F_A.k < t) throw WouldThrow{"DimensionMismatch in L11 solve"};
+            need_nonzero_diag(F_A, t, "SingularException (lower)");
+        } else {              // R11[1:rankA, 1:rankA] \ b[1:rankA], F_L11.P[1:rankA, 1:rankA]
+            if (rankA > F_L11.k || rankA > F_L11.cols) throw WouldThrow{"BoundsError R11[1:rankA,1:rankA]"};
+            need_nonzero_diag(F_L11, rankA, "SingularException (upper)");
+        }
+        // EF:379-381 returns a bare vector where the caller destructures (p, error)
+        if (rankA == n) throw WouldThrow{"newton_search_direction with rankA == n"};
+        if (t > rankA && F_L11.cols != n) throw WouldThrow{"E[P2, P2] with length(P2) != n"};
+        const int rc = sb->newton_direction(x.data(), lam, W.active.data(), t, rankA, C.cx, p);
+        if (rc < 0) throw std::runtime_error("Newton step: this backend has no second derivatives");
+        return rc == 1;
+    }
+
     // EF:1191-1291
-    int search_direction_analys(const IterL& prev, IterL& cur, int iter_number, double active_cx_sum, const Vec& p_gn) { ProfScope prof_(9);
+    int search_direction_analys(const IterL& prev, IterL& cur, int iter_number, double active_cx_sum, const Vec& p_gn,
+                                const Vec& x) { ProfScope prof_(9);
         double rx_sum = dotv(rx, rx);
         double nrm_b1_gn = norm_range(cur.b_gn, cur.dimA);
         int rankA = cur.rankA;
@@ -1153,7 +1191,14 @@ public:
             choose_subspace_dimensions(rx_sum, active_cx_sum, W.t, rankJ2, rankA, b, prev, restart, dimA, dimJ2);
             sub_search_direction(W.t, rankA, dimA, dimJ2, method_code, p, b, d);
             if (dimA == rankA && dimJ2 == rankJ2) method_code = 1;
-        } else {   // 2: Newton requested, but second derivatives are off in this regime (EF:2658) -> EF:1272-1276
+        } else if (opt.second_derivatives) {   // 2: Newton step, EF:1262-1271
+            const bool failed = newton_search_direction(x, cur.lam, rankA, p);
+            b = cur.b_gn; d = cur.d_gn;
+            dimA = -W.t;
+            dimJ2 = W.t - n;
+            cur.nb_newton_steps += 1;
+            if (failed) error_code = -3;
+        } else {   // 2: Newton requested with second derivatives off (EF:2658) -> EF:1272-1276
             p = p_gn; b = cur.b_gn; d = cur.d_gn;
             dimA = rankA; dimJ2 = rankJ2;
             error_code = -4;
@@ -1807,7 +1852,7 @@ public:
             for (int i = 0; i < W.t; ++i) { double v = cx[W.active[i] - 1]; active_cx_sum += v * v; }
             first.t = W.t;
             IterL prev = copy_iter(first, rx_sum, live_cx_sum());
-            int error_code = search_direction_analys(prev, first, nb_iteration, active_cx_sum, p_gn);
+            int error_code = search_direction_analys(prev, first, nb_iteration, active_cx_sum, p_gn, x);
             Vec w;
             int Psi_error;
             double alpha = compute_steplength(first, prev, x, w, Psi_error);
@@ -1844,7 +1889,7 @@ public:
                 active_cx_sum = 0.0;
                 for (int i = 0; i < W.t; ++i) { double v = cx[W.active[i] - 1]; active_cx_sum += v * v; }
                 it.t = W.t;
-                error_code = search_direction_analys(prev, it, nb_iteration, active_cx_sum, p_gn);
+                error_code = search_direction_analys(prev, it, nb_iteration, active_cx_sum, p_gn, x);
                 Vec xk = x;
                 alpha = compute_steplength(it, prev, xk, w, Psi_error);
                 it.alpha = alpha;

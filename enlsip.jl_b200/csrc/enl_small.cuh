@@ -2135,4 +2135,87 @@ __global__ void build_rt_kernel(const double* __restrict__ FA, int n, int t, int
     Rt[e] = (r <= c) ? FA[(size_t)c * n + r] : 0.0;
 }
 
+// =============================================================================================
+// Newton step (EF:348-423) of the mid-size row families
+// =============================================================================================
+// out (n x n) = in' (both column major, ld = n)
+__global__ void transpose_kernel(const double* __restrict__ in, int n, double* __restrict__ out) {
+    __shared__ double tile[32][33];
+    const int bx = blockIdx.x * 32, by = blockIdx.y * 32;
+    for (int yy = threadIdx.y; yy < 32; yy += blockDim.y) {
+        const int r = bx + threadIdx.x, c = by + yy;
+        if (r < n && c < n) tile[yy][threadIdx.x] = in[(size_t)c * n + r];
+    }
+    __syncthreads();
+    for (int yy = threadIdx.y; yy < 32; yy += blockDim.y) {
+        const int r = by + threadIdx.x, c = bx + yy;
+        if (r < n && c < n) out[(size_t)c * n + r] = tile[threadIdx.x][yy];
+    }
+}
+// Wn (k2 x n, ld = k2; k2 = n - ra): row a = row ra + a of E[P, P] + (J~Q1)' (J~Q1), P = perm (NULL: identity).  Its
+// columns < ra are W21 = E21 + J2'J1, the others W22 = E22 + J2'J2 (J1 / J2 = columns < ra / >= ra of J~Q1, mt rows).
+// One warp per entry, lanes over the rows of J~Q1.
+__global__ void __launch_bounds__(256) newton_assemble_kernel(const double* __restrict__ E, int n, int ra, const int* __restrict__ perm,
+                                                              const double* __restrict__ JQ1, int mt, double* __restrict__ Wn) {
+    const int k2 = n - ra, lane = threadIdx.x & 31;
+    const long long gw = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long e = gw; e < (long long)k2 * n; e += nw) {
+        const int a = (int)(e % k2), c = (int)(e / k2);
+        const double* u = JQ1 + (size_t)(ra + a) * mt;
+        const double* v = JQ1 + (size_t)c * mt;
+        double s = 0.0;
+        for (int r = lane; r < mt; r += 32) s = fma(u[r], v[r], s);
+        s = s_warp_sum(s);
+        if (lane == 0) {
+            const int er = perm ? perm[ra + a] : ra + a, ec = perm ? perm[c] : c;
+            Wn[(size_t)c * k2 + a] = E[(size_t)ec * n + er] + s;
+        }
+    }
+}
+// U (k2 x k2, ld = k2, upper triangle) = (W22 + W22') * 0.5, W22 = columns ra.. of Wn (ld = k2)
+__global__ void newton_sym_kernel(const double* __restrict__ Wn, int k2, int ra, double* __restrict__ U) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= (long long)k2 * k2) return;
+    const int a = (int)(e % k2), c = (int)(e / k2);
+    if (a <= c) U[(size_t)c * k2 + a] = (Wn[(size_t)(ra + c) * k2 + a] + Wn[(size_t)(ra + a) * k2 + c]) * 0.5;
+}
+
+// Upper Cholesky factorisation with LAPACK dpotrf('U') semantics: the upper triangle of a (n x n, column major, ld lda)
+// is overwritten by U with U'U = a; the strict lower triangle is not referenced.  *info = 0, or j + 1 when the pivot of
+// step j is not positive (or NaN) -- the factorisation stops there.  One CTA, right-looking: step j forms row j of U in
+// shared memory (u[c] = a[j, c] / u_jj) and subtracts u[r] u[c] from the trailing upper triangle, one warp per column.
+constexpr int POTRF_THREADS = 1024;
+__global__ void __launch_bounds__(POTRF_THREADS) potrf_upper_kernel(double* __restrict__ a, int lda, int n, int* info) {
+    extern __shared__ double u[];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    for (int j = 0; j < n; ++j) {
+        const double ajj = a[(size_t)j * lda + j];      // final: step j - 1 wrote it before its closing barrier
+        if (!(ajj > 0.0)) {
+            if (threadIdx.x == 0) *info = j + 1;
+            return;
+        }
+        const double ujj = sqrt(ajj);
+        for (int c = j + 1 + threadIdx.x; c < n; c += blockDim.x) {
+            const double v = a[(size_t)c * lda + j] / ujj;
+            u[c] = v;
+            a[(size_t)c * lda + j] = v;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) a[(size_t)j * lda + j] = ujj;
+        for (int c = j + 1 + w; c < n; c += nw) {
+            const double uc = u[c];
+            double* col = a + (size_t)c * lda;
+            for (int r = j + 1 + lane; r <= c; r += 32) col[r] -= u[r] * uc;
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *info = 0;
+}
+inline int potrf_upper(double* a, int lda, int n, int* info, cudaStream_t st) {
+    if (n <= 0 || n > VEC_STAGE_MAX) return -1;
+    potrf_upper_kernel<<<1, POTRF_THREADS, sizeof(double) * (size_t)n, st>>>(a, lda, n, info);
+    return 1;
+}
+
 }  // namespace enl_small

@@ -168,11 +168,12 @@ total_nb_constraints(model::CnlsModel) = model.nb_constraints                   
 const FAMILY_SINGLE_INDEX = Cint(16)
 const FAMILY_LARGE_CHAINED_ROSENBROCK = Cint(17)
 const LARGE_FACTOR_TSQR = Cint(0x100)      # OR-ed into the family of a row family: TSQR of [J | r], row sharding
+const LARGE_MIDSIZE = Cint(0x200)          # OR-ed into the family of a row family with n + m < 1000: Newton steps (EF:2658)
 
 """
     large_compile_family(source; m, nb_eqcons=0, nb_ineqcons=0, has_jacobians=false) -> library handle
 
-User problems of the large regime (n + m >= 1000): `source` defines `enl_user::residual` / `enl_user::constraint` as
+User problems of the large regime (n + m >= 1000, or smaller with m >= n + 1 and Newton steps): `source` defines `enl_user::residual` / `enl_user::constraint` as
 templates over a point accessor (and optionally `jac_residual` / `jac_constraint`), see include/enlsip_b200.h.  Pass the
 handle to `LargeCnlsModel(lib, starting_point; m=..., nb_eqcons=..., nb_ineqcons=..., data=(...))`.
 """
@@ -240,7 +241,9 @@ General row families: the reference's own chained Rosenbrock test (test/problems
 reference runs n = 1000), or a user family compiled by `large_compile_family`.  `data`: up to two Float64 arrays
 handed to the family's functions (copied to the device here; whole on every rank).  `factor=:tsqr` compresses [J | r]
 with the tall-skinny QR (LARGE_FACTOR_TSQR); with it, `shard=(rank, nranks)` gives this process the rows of
-`shard_rows(m, rank, nranks)`, after which every rank calls `join!`.
+`shard_rows(m, rank, nranks)`, after which every rank calls `join!`.  With n + m < 1000 the problem is solved with
+Newton steps, as the reference decides by size (EF:2658; LARGE_MIDSIZE); such a problem takes neither `factor=:tsqr`
+nor `shard`.
 """
 function LargeCnlsModel(family::Symbol, starting_point::Vector{Float64}; x_low=fill(-Inf, length(starting_point)),
                         x_upp=fill(Inf, length(starting_point)), jacobian::Symbol=:analytic, device::Integer=-1,
@@ -269,11 +272,14 @@ function _row_family_model(lib, fam, starting_point, m, q, ni, data, x_low, x_up
     factor in (:householder, :tsqr) || error("factor must be :householder or :tsqr")
     shard === nothing || factor === :tsqr || error("shard=(rank, nranks) needs factor=:tsqr")
     n = length(starting_point)
+    midsize = n + m < 1000      # second_derivatives of the reference (EF:2658)
+    midsize && (factor === :tsqr || shard !== nothing) && error("n + m < 1000 (Newton steps): neither factor=:tsqr nor shard")
     rows = shard === nothing ? m : shard_rows(m, shard...)[2]
+    flag = (factor === :tsqr ? LARGE_FACTOR_TSQR : Cint(0)) | (midsize ? LARGE_MIDSIZE : Cint(0))
     h = Ref{Ptr{Cvoid}}(C_NULL)
     checkl(ccall(fsym(lib, :enlsipb200_large_create), Cint,
                  (Cint, Cint, Clonglong, Clonglong, Cint, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Cint, Ptr{Ptr{Cvoid}}),
-                 factor === :tsqr ? fam | LARGE_FACTOR_TSQR : fam, n, rows, m, 0, 0, C_NULL, x_low, x_upp, Cint(device), h))
+                 fam | flag, n, rows, m, 0, 0, C_NULL, x_low, x_upp, Cint(device), h))
     for (slot, arr) in enumerate(data)      # copied host -> device inside the call: nothing to keep alive
         checkl(ccall(fsym(lib, :enlsipb200_large_set_data), Cint, (Ptr{Cvoid}, Cint, Ptr{Cdouble}, Clonglong, Cint),
                      h[], Cint(slot - 1), arr, length(arr), Cint(0)))

@@ -14,6 +14,8 @@ from its own rows and calls ``model.join(rank, world)`` once (NCCL unique id bro
 Row families (chained Rosenbrock, LargeUserFamily) compress [J | r] by a plain Householder QR of the column-major matrix
 unless ``factor="tsqr"``: then they take the single-index family's tall-skinny QR, and ``shard=(rank, world)`` gives this
 process its slice of the rows (``shard_rows``) before ``join(rank, world)``.  Data slots stay whole on every rank.
+A row family with n + m < 1000 is solved as the reference solves it at that size, with Newton steps (second derivatives
+on, EF:2658; the handle is created with LARGE_MIDSIZE); such a problem is not factored by the TSQR nor sharded.
 There is no CPU execution path.
 """
 from __future__ import annotations
@@ -51,7 +53,8 @@ def shard_rows(m, rank, world):
 
 class LargeUserFamily:
     """A problem of the large regime defined by user CUDA source: the replacement of the reference's closure arguments
-    (residuals, eq_constraints, ineq_constraints, jacobian_*; cnls_model.jl:345-359) when n + m >= 1000.  `source` defines
+    (residuals, eq_constraints, ineq_constraints, jacobian_*; cnls_model.jl:345-359) for one problem with
+    n + m >= 1000, or a smaller one (m >= n + 1) solved with Newton steps as the reference solves it.  `source` defines
     enl_user::residual / constraint as templates over a point accessor and, with has_jacobians, jac_residual /
     jac_constraint (include/enlsip_b200.h, enlsipb200_large_compile_family).  `data`: names of up to two data arrays."""
 
@@ -128,8 +131,14 @@ class LargeCnlsModel:
         self.nb_eqcons = q
         self.nb_constraints = q + ni + int(np.isfinite(self.x_low).sum()) + int(np.isfinite(self.x_upp).sum())
         self.lmax = self.nb_constraints
+        # the reference takes Newton steps below this size (second_derivatives = n + m < 1000, EF:2658)
+        self.midsize = n + m < 1000
+        if self.midsize and (self.factor_mode == "tsqr" or self.shard is not None):
+            raise AssertionError("n + m < 1000 (Newton steps): the [J | r] of a mid-size problem is neither factored by the "
+                                 "TSQR nor sharded; use factor='householder' without shard")
+        flag = self._flag | (capi.LARGE_MIDSIZE if self.midsize else 0)
         h = ctypes.c_void_p()
-        capi.check_large(self._lib.enlsipb200_large_create(fam_id | self._flag, n, self.rows, m, 0, 0, None, self.x_low.ctypes.data,
+        capi.check_large(self._lib.enlsipb200_large_create(fam_id | flag, n, self.rows, m, 0, 0, None, self.x_low.ctypes.data,
                                                             self.x_upp.ctypes.data, device, ctypes.byref(h)), self._lib)
         self._h = h
         for slot, key in enumerate(keys):
@@ -193,10 +202,11 @@ class LargeCnlsModel:
         return R, float(b.value), float(t.value)
 
     def stats(self):
-        v = np.zeros(13)
-        capi.check_large(self._lib.enlsipb200_large_stats(self._h, v.ctypes.data, 13), self._lib)
+        v = np.zeros(15)
+        capi.check_large(self._lib.enlsipb200_large_stats(self._h, v.ctypes.data, 15), self._lib)
         keys = ("points", "build_ms", "tsqr_ms", "linesearch_ms", "solve_wall_ms", "linesearch_evals",
-                "launches", "rows_pad", "device_qrcp", "device_mulq", "small_stage_ms", "factorisations", "ws_growths")
+                "launches", "rows_pad", "device_qrcp", "device_mulq", "small_stage_ms", "factorisations", "ws_growths",
+                "newton_steps", "hessian_ms")
         return dict(zip(keys, [float(a) for a in v]))
 
     def launch_count(self):

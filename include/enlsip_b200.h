@@ -196,6 +196,14 @@ ENLSIPB200_API int enlsipb200_det_exp(const double* x, double* y, long long n, i
  * ignores it. */
 #define ENLSIPB200_LARGE_FACTOR_TSQR 0x100
 
+/* OR-ed into `family` of enlsipb200_large_create: a mid-size problem (n + m_global < 1000) of a row family (built-in or
+ * ENLSIPB200_FAMILY_USER), solved with second derivatives on as the reference does at that size (EF:2658): where the
+ * iteration asks for a Newton step (method code 2) it takes one, with the Hessian of the Lagrangian by central
+ * differences of the family's residuals and constraints on the device.  Refused (ENLSIPB200_EINVAL, before any device
+ * call) for the single-index family, together with ENLSIPB200_LARGE_FACTOR_TSQR, when n + m_global >= 1000 and when
+ * m_global < n + 1; m_local = m_global = m(n).  Without the flag n + m_global < 1000 stays refused. */
+#define ENLSIPB200_LARGE_MIDSIZE 0x200
+
 typedef struct enlsipb200_large_s* enlsipb200_large;
 
 ENLSIPB200_API const char* enlsipb200_large_last_error(void);
@@ -224,7 +232,8 @@ ENLSIPB200_API int enlsipb200_large_factor(enlsipb200_large h, const double* x, 
  * evaluations (host clock around launch..result), kernels launched, padded local rows, device QRCPs, device M*Q products,
  * ms inside the small-stage calls (host clock: kernels + the waits for their results), factorisations of [J | r] (one per
  * point from which the iteration continued), growths of the working-set buffers (a working set of more than
- * min(l, n) + 1 rows)}; `count` may stop short of the last entries */
+ * min(l, n) + 1 rows), Newton steps (ENLSIPB200_LARGE_MIDSIZE), device ms of the Hessian kernel (CUDA events)};
+ * `count` may stop short of the last entries */
 ENLSIPB200_API int enlsipb200_large_stats(enlsipb200_large h, double* out, int count);
 
 /* Known-answer hooks of the small stage's dense kernels (csrc/enl_small.cuh), host buffers, column major:
@@ -249,6 +258,10 @@ ENLSIPB200_API int enlsipb200_dense_vecop(int kind, int frows, int k, const doub
  *       alpha, y0 and beta unused). */
 ENLSIPB200_API int enlsipb200_dense_gemv(int trans, int rows, int cols, const double* A, int lda, const double* x, double alpha,
                                          const double* y0, double beta, double* y, int device);
+/*   enlsipb200_dense_potrf : the Cholesky factorisation of the Newton step (src/enlsip_functions.jl:348-423, LAPACK
+ *       dpotrf('U')).  a [n x n] (n <= 6144): the upper triangle in, U with U'U = a out; info = 0, or j (1-based) when the
+ *       leading minor of order j is not positive definite. */
+ENLSIPB200_API int enlsipb200_dense_potrf(int n, double* a, int* info, int device);
 /* device time (CUDA events around the kernels, transfers excluded) of the last enlsipb200_dense_* call, in ms */
 ENLSIPB200_API float enlsipb200_dense_last_ms(void);
 
