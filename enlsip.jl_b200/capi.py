@@ -15,7 +15,7 @@ HEADERS = [os.path.join(_HERE, "csrc", f) for f in ("enl_base.h", "enl_linalg.h"
 # second translation unit: the large-Jacobian regime (TSQR + host-driven iteration)
 SRC_LARGE = os.path.join(_HERE, "csrc", "enl_large.cu")
 HEADERS_LARGE = [os.path.join(_HERE, "csrc", f) for f in ("enl_base.h", "enl_tsqr.cuh", "enl_small.cuh", "enl_large_host.h",
-                                                          "enl_large_family.h", "enl_large_generic.cuh")] + \
+                                                          "enl_large_family.h", "enl_large_generic.cuh", "enl_small_device.cuh")] + \
                 [os.path.join(os.path.dirname(_HERE), "include", "enlsip_b200.h")]
 OBJ_DIR = os.path.join(_HERE, "lib", "obj")
 FAMILY_SINGLE_INDEX = 16

@@ -9,22 +9,22 @@
 #include <cuda_runtime.h>
 
 #include "enl_large_family.h"
+#include "enl_large_host.h"
 
 namespace enl_large {
 
-constexpr double G_SQRT_EPS = 1.4901161193847656e-08;
-
-__device__ __forceinline__ double g_warp_sum(double v) {
+// the reductions of every m-sized kernel of the large regime (these and enl_large.cu's single-index kernels)
+__device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
 // four sums over the CTA -> part[blockIdx * 4 + k] (fixed order)
-__device__ __forceinline__ void g_block_reduce4(double (&v)[4], double* part) {
+__device__ __forceinline__ void block_reduce4(double (&v)[4], double* part) {
     __shared__ double sh[8][4];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
 #pragma unroll
-    for (int k = 0; k < 4; ++k) v[k] = g_warp_sum(v[k]);
+    for (int k = 0; k < 4; ++k) v[k] = warp_sum(v[k]);
     if (lane == 0)
 #pragma unroll
         for (int k = 0; k < 4; ++k) sh[w][k] = v[k];
@@ -49,7 +49,7 @@ __global__ void __launch_bounds__(256) lg_build_kernel(int n, long long m, const
         for (int j = lane; j < n; j += 32) {
             double v;
             if (fd || !F::HAS_JAC) {
-                const double dj = __dmul_rn(fmax(fabs(x[j]), 1.0), G_SQRT_EPS);
+                const double dj = __dmul_rn(fmax(fabs(x[j]), 1.0), SQRT_EPS);
                 v = __ddiv_rn(__dsub_rn(F::residual(i, n, XPert{x, j, dj}, d0, d1), ri), dj);
             } else {
                 v = F::jac_residual(i, j, n, x, d0, d1);
@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(256) lg_build_rows_kernel(int n, long long m, 
             double v = 0.0;
             if (j < n) {
                 if (fd || !F::HAS_JAC) {
-                    const double dj = __dmul_rn(fmax(fabs(x[j]), 1.0), G_SQRT_EPS);
+                    const double dj = __dmul_rn(fmax(fabs(x[j]), 1.0), SQRT_EPS);
                     v = __ddiv_rn(__dsub_rn(F::residual(gi, n, XPert{x, j, dj}, d0, d1), ri), dj);
                 } else {
                     v = F::jac_residual(gi, j, n, x, d0, d1);
@@ -114,14 +114,14 @@ __global__ void __launch_bounds__(256) lg_dir_rows_kernel(const double* __restri
         const double* jr = J + i * n;
         double acc = 0.0;
         for (int j = lane; j < n; j += 32) acc = fma(jr[j], p[j], acc);
-        const double jp = g_warp_sum(acc);
+        const double jp = warp_sum(acc);
         if (lane == 0) {
             const double ri = r[i];
             Jp[i] = jp;
             sums[0] = fma(ri, ri, sums[0]); sums[1] = fma(ri, jp, sums[1]); sums[2] = fma(jp, jp, sums[2]);
         }
     }
-    g_block_reduce4(sums, part);
+    block_reduce4(sums, part);
 }
 
 // sums {r.r, r.Jp, Jp.Jp, 0} for the direction just set
@@ -132,7 +132,7 @@ __global__ void __launch_bounds__(256) lg_dir_sums_kernel(const double* __restri
         const double ri = r[i], jp = Jp[i];
         sums[0] = fma(ri, ri, sums[0]); sums[1] = fma(ri, jp, sums[1]); sums[2] = fma(jp, jp, sums[2]);
     }
-    g_block_reduce4(sums, part);
+    block_reduce4(sums, part);
 }
 
 // trial point x + alpha p: partial sums {r_a.r_a, r.v2, Jp.v2, v2.v2}, v2 = ((r_a - r)/alpha - Jp)/alpha  (EF:1687)
@@ -152,7 +152,7 @@ __global__ void __launch_bounds__(256) lg_ls_kernel(int n, long long m, long lon
             sums[1] = fma(ri, v2, sums[1]); sums[2] = fma(jp, v2, sums[2]); sums[3] = fma(v2, v2, sums[3]);
         }
     }
-    g_block_reduce4(sums, part);
+    block_reduce4(sums, part);
 }
 
 // the family's own constraints (equalities then inequalities) at x
@@ -172,7 +172,7 @@ __global__ void lg_jac_cons_kernel(int n, int nc, const double* __restrict__ x, 
     const int k = (int)(e / n), j = (int)(e % n);
     double v;
     if (fd || !F::HAS_JAC) {
-        const double dj = __dmul_rn(fmax(fabs(x[j]), 1.0), G_SQRT_EPS);
+        const double dj = __dmul_rn(fmax(fabs(x[j]), 1.0), SQRT_EPS);
         v = __ddiv_rn(__dsub_rn(F::constraint(k, n, XPert{x, j, dj}, d0, d1), c0[k]), dj);
     } else {
         v = F::jac_constraint(k, j, n, x, d0, d1);
@@ -249,8 +249,8 @@ __global__ void __launch_bounds__(LG_HESS_THREADS) lg_hessian_kernel(int n, long
     }
     __shared__ double sh[LG_HESS_THREADS / 32][2];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    sr = g_warp_sum(sr);
-    sc = g_warp_sum(sc);
+    sr = warp_sum(sr);
+    sc = warp_sum(sc);
     if (lane == 0) { sh[w][0] = sr; sh[w][1] = sc; }
     __syncthreads();
     if (threadIdx.x == 0) {

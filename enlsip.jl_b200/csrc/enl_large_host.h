@@ -22,7 +22,7 @@
 // Newton steps (EF:348-423) follow LargeOptions::second_derivatives, which is the reference's `n + m < 1000` (EF:2658):
 // the entry point turns it on only for row families created with ENLSIPB200_LARGE_MIDSIZE, refuses that flag when
 // n + m >= 1000, and refuses n + m < 1000 without it.  The driver decides the reference's size situations of the Newton
-// step; the Hessian (LargeOps::hessian) and the linear algebra (SmallBackend::newton_direction) belong to the backend.
+// step; the Hessian and the linear algebra (SmallBackend::newton_direction) belong to the backend.
 #pragma once
 #include <float.h>
 #include <math.h>
@@ -324,13 +324,6 @@ struct LargeOps {
     int n = 0, l = 0, q = 0;
     long long m = 0;         // true number of residuals (all shards)
     virtual ~LargeOps() {}
-    // evaluate r, J, c, A at x (new_point!, EF:34-52): the m-sized part stays with the backend; returned are
-    // gradf = J'r (n), *rr = r'r, cx (l), A (l x n, column major).  Returns 0 or an API error.
-    // This is all the termination test of the point needs (EF:2838 reads ||J'r||, ||r||^2 and c), so the
-    // factorisation below is only paid for points from which the iteration goes on.
-    virtual int eval_point(const double* x, double* gradf, double* rr, double* cx, double* A) = 0;
-    // compress the point of the last eval_point: Jt ((n+1) x n, column major) = [R_J; 0], rt (n+1) = [z; rho]
-    virtual int compress(double* Jt, double* rt) = 0;
     // fix the direction of the linesearch at the current point: sums = {r.r, r.Jp, Jp.Jp}
     virtual int set_direction(const double* x, const double* p, double sums[3]) = 0;
     // ||r(x + alpha p)||^2
@@ -344,13 +337,6 @@ struct LargeOps {
     // on it leave each other alone in the next collective.  Sharded backends return the mean over the ranks (one sum
     // all-reduce of elapsed / nranks).
     virtual double agreed_elapsed(double local_elapsed) { return local_elapsed; }
-    // Newton step: G = sum_i r_i Hess r_i - sum_{a < t} lam[a] Hess c_{active[a]} at x by the reference's central differences
-    // (EF:243-328), n x n column major into G, which lives where the backend keeps its matrices.  Backends without second
-    // derivatives keep this default.
-    virtual int hessian(const double* x, const double* lam, const int* active, int t, double* G) {
-        (void)x; (void)lam; (void)active; (void)t; (void)G;
-        return -1;
-    }
 };
 
 struct LargeOptions {
@@ -419,8 +405,9 @@ struct ConstraintL {   // structures.jl:145-150 ; the t x n matrix A (row i = gr
 // block C.A (t x n), the compressed Jacobian J~ ((n+1) x n), J~*Q1 and the three pivoted QR factorisations
 // (EF:700 F_A, EF:769 F_L11, EF:223 F_J2).  The driver below keeps the scalar logic, the working set and the
 // O(n) vectors; it hands vectors in and gets vectors / diagonals / permutations back.
-//   HostSmall    (this header): host memory, the CPU test backend;
-//   DeviceSmall  (enl_small.cuh, product): everything resident in HBM, CUDA kernels only.
+//   HostSmall    (this header): host memory, the CPU test backend, over a HostPoint;
+//   DeviceSmall  (enl_small_device.cuh, product): everything resident in HBM, CUDA kernels only, over a DevicePoint
+//                (LargeHandle, enl_large.cu), which also computes the Newton step's Hessian.
 // Size-dependent error situations of the reference (BoundsError, DimensionMismatch, SingularException) are
 // decided by the driver from FactorInfo BEFORE a backend call, so a backend never has to throw.
 // ------------------------------------------------------------------------------------------
@@ -459,7 +446,7 @@ struct SmallBackend {
     // EF:2497: ||C.A' C.cx||
     virtual double At_c_norm(int t, const Vec& Ccx) = 0;
     // EF:348-423 (sizes validated by the driver): p1 from R_A' \ (-c[P]) (t == rankA) or P_L11 [R11 \ (Q_L11' (-c[P]))[1:rankA]]
-    // (t > rankA); E = (Q1' G) Q1 with G = LargeOps::hessian at x, E[P2, P2] when t > rankA; W22 = E22 + J2'J2,
+    // (t > rankA); E = (Q1' G) Q1 with G the Hessian of the Lagrangian at x, E[P2, P2] when t > rankA; W22 = E22 + J2'J2,
     // W21 = E21 + J2'J1, d = -W21 p1 - J2' r; the upper Cholesky factor U of (W22 + W22') / 2 (dpotrf); p = Q1 [p1; U \ (U' \ d)].
     // Returns 0, 1 when the Cholesky factorisation fails (p = 0), or -1 when the backend has no Newton step (this default).
     virtual int newton_direction(const double* x, const Vec& lam, const int* active, int t, int rankA, const Vec& Ccx, Vec& p) {
@@ -468,9 +455,21 @@ struct SmallBackend {
     }
 };
 
+// what HostSmall needs from the m-sized backend: new_point! with A, J~ and r~ as host matrices
+struct HostPoint {
+    virtual ~HostPoint() {}
+    // evaluate r, J, c, A at x (new_point!, EF:34-52): the m-sized part stays with the backend; returned are
+    // gradf = J'r (n), *rr = r'r, cx (l), A (l x n, column major).  Returns 0 or an API error.
+    // This is all the termination test of the point needs (EF:2838 reads ||J'r||, ||r||^2 and c), so the
+    // factorisation below is only paid for points from which the iteration goes on.
+    virtual int eval_point(const double* x, double* gradf, double* rr, double* cx, double* A) = 0;
+    // compress the point of the last eval_point: Jt ((n+1) x n, column major) = [R_J; 0], rt (n+1) = [z; rho]
+    virtual int compress(double* Jt, double* rt) = 0;
+};
+
 // Host-memory backend: the CPU test path (oracle/hostport/largeport.cpp).  The product never instantiates it.
 struct HostSmall : SmallBackend {
-    LargeOps& ops;
+    HostPoint& ops;
     int n, l, mt;
     Mat J;      // mt x n
     Vec rx;     // mt
@@ -480,7 +479,7 @@ struct HostSmall : SmallBackend {
     Mat JQ1;          // J * F_A.Q, formed once per F_A (EF:219, 526, 1249 recompute it)
     bool jq1_valid = false;
 
-    explicit HostSmall(LargeOps& o) : ops(o), n(o.n), l(o.l), mt(o.n + 1) {
+    HostSmall(HostPoint& o, int nn, int ll) : ops(o), n(nn), l(ll), mt(nn + 1) {
         J = Mat(mt, n);
         rx.assign(mt, 0.0);
         A = Mat(l, n);
@@ -699,8 +698,7 @@ public:
     long long m;
 
     // the matrix-sized state lives in the backend; here: vectors and scalars
-    HostSmall* own_small = nullptr;
-    SmallBackend* sb = nullptr;
+    SmallBackend* sb;
     Vec rx;     // r~ (mt)
     Vec cx;     // l
     Vec gradf;
@@ -710,13 +708,9 @@ public:
     FactorInfo F_A, F_L11, F_J2;
     int n_new_point = 0, n_res_eval = 0;
 
-    // backend == nullptr: host memory (CPU tests); the product passes its device backend
-    LargeSolver(LargeOps& o, const LargeOptions& op, SmallBackend* backend = nullptr) : ops(o), opt(op) {
+    LargeSolver(LargeOps& o, const LargeOptions& op, SmallBackend& small) : ops(o), opt(op), sb(&small) {
         n = o.n; l = o.l; q = o.q; m = o.m; mt = n + 1;
-        if (backend) sb = backend;
-        else { own_small = new HostSmall(o); sb = own_small; }
     }
-    ~LargeSolver() { delete own_small; }
     LargeSolver(const LargeSolver&) = delete;
     LargeSolver& operator=(const LargeSolver&) = delete;
 

@@ -26,7 +26,30 @@
 #include <math.h>
 #include <stdlib.h>
 
+#include <memory>
+
 namespace enl_small {
+
+// owning device and pinned host buffers
+struct DeviceFree { void operator()(void* p) const { cudaFree(p); } };
+struct PinnedFree { void operator()(void* p) const { cudaFreeHost(p); } };
+template <class T> using DevBuf = std::unique_ptr<T[], DeviceFree>;
+template <class T> using PinnedBuf = std::unique_ptr<T[], PinnedFree>;
+// (re)allocate `count` elements; a buffer already held is freed first
+template <class T> cudaError_t dev_alloc(DevBuf<T>& b, size_t count) {
+    b.reset();
+    T* p = nullptr;
+    const cudaError_t e = cudaMalloc(&p, sizeof(T) * count);
+    b.reset(p);
+    return e;
+}
+template <class T> cudaError_t pinned_alloc(PinnedBuf<T>& b, size_t count) {
+    b.reset();
+    T* p = nullptr;
+    const cudaError_t e = cudaHostAlloc(&p, sizeof(T) * count, cudaHostAllocDefault);
+    b.reset(p);
+    return e;
+}
 
 constexpr double S_TOL3Z = 1.0536712127723509e-08;   // sqrt(dlamch('Epsilon')) = sqrt(2^-53)
 constexpr int QR_NB = 32;                             // dgeqp3 block size (ilaenv(1, 'DGEQRF') = 32)
@@ -1237,16 +1260,41 @@ constexpr int QR_PSUM_LEN = QP_MAXG * (QR_NB + 1) > QR_MAXPART ? QP_MAXG * (QR_N
 constexpr int QR_PIDX_LEN = QR_MAXPART + QP_MAXG;                                                    // ints in QrWork::pidx
 constexpr int QR_TICKET_LEN = 8 + 8 * QP_MAXG;   // [0] close ticket; from [1]: the grid barrier of the persistent panel (qp_grid_barrier)
 struct QrWork {          // scratch of one factorisation (sized for the largest matrix of the solve)
-    double *vn1 = nullptr, *vn2 = nullptr, *F = nullptr, *auxv = nullptr, *pbest = nullptr, *psum = nullptr;   // psum: QR_PSUM_LEN
-    int *flags = nullptr, *pidx = nullptr;                                                                     // pidx: QR_PIDX_LEN
-    QrState* state = nullptr;
-    unsigned int* ticket = nullptr;                                                                            // QR_TICKET_LEN
+    DevBuf<double> vn1, vn2, F, auxv, pbest, psum;   // per column: vn1, vn2, F (x QR_NB); psum: QR_PSUM_LEN
+    DevBuf<int> flags, pidx;                         // flags: per column; pidx: QR_PIDX_LEN
+    DevBuf<QrState> state;
+    DevBuf<unsigned int> ticket;                     // QR_TICKET_LEN
     int cap_cols = 0;
     QrGraph graphs[6];
     int next_graph = 0;
     bool use_graphs = true;
+    QrWork() = default;
+    QrWork(const QrWork&) = delete;
+    QrWork& operator=(const QrWork&) = delete;
+    ~QrWork() { drop_graphs(); }
     void drop_graphs() {
         for (QrGraph& g : graphs) { if (g.exec) cudaGraphExecDestroy(g.exec); g = QrGraph(); }
+    }
+    // the per-column arrays for `cols` columns (the contents are scratch of one factorisation)
+    cudaError_t alloc_cols(int cols) {
+        cap_cols = 0;
+        cudaError_t e = dev_alloc(vn1, cols);
+        if (e == cudaSuccess) e = dev_alloc(vn2, cols);
+        if (e == cudaSuccess) e = dev_alloc(F, (size_t)cols * QR_NB);
+        if (e == cudaSuccess) e = dev_alloc(flags, cols);
+        if (e == cudaSuccess) cap_cols = cols;
+        return e;
+    }
+    // everything qrcp_device needs for matrices of up to `cols` columns; the ticket is not cleared
+    cudaError_t alloc(int cols) {
+        cudaError_t e = alloc_cols(cols);
+        if (e == cudaSuccess) e = dev_alloc(auxv, QR_NB);
+        if (e == cudaSuccess) e = dev_alloc(pbest, QR_MAXPART);
+        if (e == cudaSuccess) e = dev_alloc(psum, QR_PSUM_LEN);
+        if (e == cudaSuccess) e = dev_alloc(pidx, QR_PIDX_LEN);
+        if (e == cudaSuccess) e = dev_alloc(state, 1);
+        if (e == cudaSuccess) e = dev_alloc(ticket, QR_TICKET_LEN);
+        return e;
     }
 };
 
@@ -1276,14 +1324,14 @@ inline int qp_grid() {
 }
 inline int qr_enqueue_panel_persist(double* f, int rows, int cols, double* tau, int* jpvt, QrWork& wk, int topbmn, int G,
                                     cudaStream_t st) {
-    double *vn1 = wk.vn1, *vn2 = wk.vn2, *F = wk.F, *pbest = wk.pbest, *ppart = wk.psum;
-    int *flags = wk.flags, *pidx = wk.pidx, *pany = wk.pidx + QR_MAXPART;
-    QrState* stt = wk.state;
-    unsigned int* bar = wk.ticket + 1;
+    double *vn1 = wk.vn1.get(), *vn2 = wk.vn2.get(), *F = wk.F.get(), *pbest = wk.pbest.get(), *ppart = wk.psum.get();
+    int *flags = wk.flags.get(), *pidx = wk.pidx.get(), *pany = wk.pidx.get() + QR_MAXPART;
+    QrState* stt = wk.state.get();
+    unsigned int* bar = wk.ticket.get() + 1;
     void* args[] = {&f, &rows, &cols, &vn1, &vn2, &jpvt, &tau, &F, &flags, &stt, &pbest, &pidx, &pany, &ppart, &bar};
     cudaLaunchCooperativeKernel((const void*)qr_panel_persist_kernel, dim3(G), dim3(QP_THREADS), args, qp_smem_bytes(rows, G), st);
-    qr_panel_trail_fma_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F, wk.state);
-    qr_panel_close_kernel<<<148, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, wk.flags, wk.state, topbmn, wk.ticket);
+    qr_panel_trail_fma_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F.get(), wk.state.get());
+    qr_panel_close_kernel<<<148, 256, 0, st>>>(f, rows, cols, wk.vn1.get(), wk.vn2.get(), wk.flags.get(), wk.state.get(), topbmn, wk.ticket.get());
     return 3;
 }
 
@@ -1292,14 +1340,14 @@ inline int qr_enqueue_panel(double* f, int rows, int cols, double* tau, int* jpv
     const int g_gemv = imin_host((cols + QR_GCOLS - 1) / QR_GCOLS + 4, 148 * 8);
     int launches = 0;
     for (int k = 0; k < QR_NB; ++k) {
-        qr_panel_finish_pivot_kernel<<<g_fin, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, jpvt, wk.F, wk.auxv, wk.flags, wk.state, wk.pbest, wk.pidx, k);
-        qr_panel_column_kernel<<<g_col, 256, 0, st>>>(f, rows, cols, tau, wk.F, wk.state, wk.psum, k);
-        qr_panel_gemv_kernel<<<g_gemv, 256, 0, st>>>(f, rows, cols, wk.F, wk.auxv, wk.state, k);
+        qr_panel_finish_pivot_kernel<<<g_fin, 256, 0, st>>>(f, rows, cols, wk.vn1.get(), wk.vn2.get(), jpvt, wk.F.get(), wk.auxv.get(), wk.flags.get(), wk.state.get(), wk.pbest.get(), wk.pidx.get(), k);
+        qr_panel_column_kernel<<<g_col, 256, 0, st>>>(f, rows, cols, tau, wk.F.get(), wk.state.get(), wk.psum.get(), k);
+        qr_panel_gemv_kernel<<<g_gemv, 256, 0, st>>>(f, rows, cols, wk.F.get(), wk.auxv.get(), wk.state.get(), k);
         launches += 3;
     }
-    qr_panel_finish_pivot_kernel<<<g_fin, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, jpvt, wk.F, wk.auxv, wk.flags, wk.state, wk.pbest, wk.pidx, QR_NB);
-    qr_panel_trail_fma_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F, wk.state);
-    qr_panel_close_kernel<<<148, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, wk.flags, wk.state, topbmn, wk.ticket);
+    qr_panel_finish_pivot_kernel<<<g_fin, 256, 0, st>>>(f, rows, cols, wk.vn1.get(), wk.vn2.get(), jpvt, wk.F.get(), wk.auxv.get(), wk.flags.get(), wk.state.get(), wk.pbest.get(), wk.pidx.get(), QR_NB);
+    qr_panel_trail_fma_kernel<<<148 * 4, 256, 0, st>>>(f, rows, cols, wk.F.get(), wk.state.get());
+    qr_panel_close_kernel<<<148, 256, 0, st>>>(f, rows, cols, wk.vn1.get(), wk.vn2.get(), wk.flags.get(), wk.state.get(), topbmn, wk.ticket.get());
     return launches + 3;
 }
 
@@ -1342,9 +1390,9 @@ inline int qrcp_device(double* f, int rows, int cols, double* tau, int* jpvt, Qr
     // dgeqp3: blocked (dlaqps) while j <= topbmn = minmn - nx, if nb < minmn and nx < minmn
     int topbmn = (QR_NB < minmn && QR_NX < minmn) ? (minmn - QR_NX) : 0;
     int launches = 0;
-    cudaMemsetAsync(wk.flags, 0, sizeof(int) * cols, st);
-    cudaMemsetAsync(wk.ticket, 0, sizeof(unsigned int) * QR_TICKET_LEN, st);
-    qr_init_kernel<<<cols, 256, 0, st>>>(f, rows, cols, wk.vn1, wk.vn2, jpvt, wk.state, topbmn, nopivot);
+    cudaMemsetAsync(wk.flags.get(), 0, sizeof(int) * cols, st);
+    cudaMemsetAsync(wk.ticket.get(), 0, sizeof(unsigned int) * QR_TICKET_LEN, st);
+    qr_init_kernel<<<cols, 256, 0, st>>>(f, rows, cols, wk.vn1.get(), wk.vn2.get(), jpvt, wk.state.get(), topbmn, nopivot);
     ++launches;
     if (topbmn > 0) {
         // A panel that stops early (a norm to recompute) re-opens at its next column, so more than ceil(topbmn / nb)
@@ -1383,14 +1431,14 @@ inline int qrcp_device(double* f, int rows, int cols, double* tau, int* jpvt, Qr
                 else launches += qr_enqueue_panel(f, rows, cols, tau, jpvt, wk, topbmn, st);
             }
             QrState h;
-            cudaMemcpyAsync(&h, wk.state, sizeof(QrState), cudaMemcpyDeviceToHost, st);
+            cudaMemcpyAsync(&h, wk.state.get(), sizeof(QrState), cudaMemcpyDeviceToHost, st);
             cudaStreamSynchronize(st);
             if (!h.active) break;
             budget = (topbmn - h.j0 + QR_NB - 1) / QR_NB + 2;
         }
     }
     for (int i = topbmn; i < minmn; ++i) {
-        qr_p2_pivot_house_kernel<<<1, 1024, 0, st>>>(f, rows, cols, i, wk.vn1, wk.vn2, jpvt, tau, nopivot);
+        qr_p2_pivot_house_kernel<<<1, 1024, 0, st>>>(f, rows, cols, i, wk.vn1.get(), wk.vn2.get(), jpvt, tau, nopivot);
         ++launches;
         if (i < cols - 1) {
             const int len = rows - i - 1;
@@ -1398,9 +1446,9 @@ inline int qrcp_device(double* f, int rows, int cols, double* tau, int* jpvt, Qr
             int grid = (ncol + 7) / 8;
             if (grid > 148 * 4) grid = 148 * 4;
             if (len <= VEC_STAGE_MAX)
-                qr_p2_apply_kernel<true><<<grid, 256, sizeof(double) * (size_t)(len > 0 ? len : 1), st>>>(f, rows, cols, i, wk.vn1, wk.vn2, tau);
+                qr_p2_apply_kernel<true><<<grid, 256, sizeof(double) * (size_t)(len > 0 ? len : 1), st>>>(f, rows, cols, i, wk.vn1.get(), wk.vn2.get(), tau);
             else
-                qr_p2_apply_kernel<false><<<grid, 256, 0, st>>>(f, rows, cols, i, wk.vn1, wk.vn2, tau);
+                qr_p2_apply_kernel<false><<<grid, 256, 0, st>>>(f, rows, cols, i, wk.vn1.get(), wk.vn2.get(), tau);
             ++launches;
         }
     }
@@ -1534,7 +1582,19 @@ inline int wy_build_t_all(const double* f, int frows, int k, const double* tau, 
     return launches;
 }
 
-struct WyWork { double *Vb = nullptr, *T = nullptr, *W = nullptr, *W2 = nullptr, *part = nullptr; };   // Vb: frows x 32, T: 32 x 32, W/W2: mr x 32, part: GEMM_MAX_SPLITS x mr x 32
+struct WyWork {           // scratch of mulq_device for Q of up to `frows` rows applied to up to `mr` rows
+    DevBuf<double> Vb, T, W, W2, part;   // Vb: frows x 32, T: 32 x 32, W/W2: mr x 32, part: GEMM_MAX_SPLITS x mr x 32
+    size_t part_len = 0;                 // doubles in part
+    cudaError_t alloc(size_t frows, size_t mr) {
+        part_len = mr * 32 * GEMM_MAX_SPLITS;
+        cudaError_t e = dev_alloc(Vb, frows * 32);
+        if (e == cudaSuccess) e = dev_alloc(T, 32 * 32);
+        if (e == cudaSuccess) e = dev_alloc(W, mr * 32);
+        if (e == cudaSuccess) e = dev_alloc(W2, mr * 32);
+        if (e == cudaSuccess) e = dev_alloc(part, part_len);
+        return e;
+    }
+};
 
 // M: mr x nq column major (ld = mr); f: frows (= nq) x k
 // Tall (optional): the T factors of all panels (wy_build_t_all) -- built here if `build_t`, reusable by reflect_vec_wy
@@ -1542,7 +1602,7 @@ inline int mulq_device(double* M, int mr, int nq, const double* f, int frows, in
                        cudaStream_t st, double* Tall = nullptr, bool build_t = true) {
     int launches = 0;
     if (Tall && build_t) {
-        const int rc = wk.part ? wy_build_t_all(f, frows, k, tau, Tall, wk.part, (size_t)mr * 32 * GEMM_MAX_SPLITS, st) : -1;
+        const int rc = wk.part.get() ? wy_build_t_all(f, frows, k, tau, Tall, wk.part.get(), wk.part_len, st) : -1;
         if (rc < 0) Tall = nullptr; else launches += rc;
     }
     for (int j0 = 0; j0 < k; j0 += 32) {
@@ -1550,27 +1610,27 @@ inline int mulq_device(double* M, int mr, int nq, const double* f, int frows, in
         const int len = frows - j0;
         if (len <= 0) break;
         const long long ne = (long long)len * pw;
-        wy_build_v_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(f, frows, j0, pw, wk.Vb);
-        const double* Tp = wk.T;
+        wy_build_v_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(f, frows, j0, pw, wk.Vb.get());
+        const double* Tp = wk.T.get();
         if (Tall) Tp = Tall + (size_t)(j0 / 32) * 1024;
-        else { wy_build_t_kernel<<<1, 1024, 0, st>>>(wk.Vb, len, pw, tau + j0, wk.T); ++launches; }
+        else { wy_build_t_kernel<<<1, 1024, 0, st>>>(wk.Vb.get(), len, pw, tau + j0, wk.T.get()); ++launches; }
         ++launches;
         // W = M(:, j0:) Vb ; W2 = W T ; M(:, j0:) -= W2 Vb'
         int splits = len / 256;                                   // W = M V: N = 32, K = len
         if (splits > GEMM_MAX_SPLITS) splits = GEMM_MAX_SPLITS;
-        if (splits >= 2 && wk.part) {
+        if (splits >= 2 && wk.part.get()) {
             const int kc = ((len + splits - 1) / splits + 31) / 32 * 32;
             splits = (len + kc - 1) / kc;
             dim3 grid((mr + 63) / 64, splits);
-            gemm_dmma_splitk_kernel<false><<<grid, 256, 0, st>>>(M + (size_t)j0 * mr, mr, wk.Vb, len, wk.part, mr, pw, len, kc);
+            gemm_dmma_splitk_kernel<false><<<grid, 256, 0, st>>>(M + (size_t)j0 * mr, mr, wk.Vb.get(), len, wk.part.get(), mr, pw, len, kc);
             const long long mn = (long long)mr * pw;
-            splitk_reduce_kernel<<<(unsigned)((mn + 255) / 256), 256, 0, st>>>(wk.part, splits, mn, 1.0, 0.0, wk.W, mr, mr);
+            splitk_reduce_kernel<<<(unsigned)((mn + 255) / 256), 256, 0, st>>>(wk.part.get(), splits, mn, 1.0, 0.0, wk.W.get(), mr, mr);
             launches += 2;
         } else {
-            launches += gemm<false>(M + (size_t)j0 * mr, mr, wk.Vb, len, wk.W, mr, mr, pw, len, 1.0, 0.0, st);
+            launches += gemm<false>(M + (size_t)j0 * mr, mr, wk.Vb.get(), len, wk.W.get(), mr, mr, pw, len, 1.0, 0.0, st);
         }
-        launches += gemm<false>(wk.W, mr, Tp, 32, wk.W2, mr, mr, pw, pw, 1.0, 0.0, st);
-        launches += gemm<true>(wk.W2, mr, wk.Vb, len, M + (size_t)j0 * mr, mr, mr, len, pw, -1.0, 1.0, st);
+        launches += gemm<false>(wk.W.get(), mr, Tp, 32, wk.W2.get(), mr, mr, pw, pw, 1.0, 0.0, st);
+        launches += gemm<true>(wk.W2.get(), mr, wk.Vb.get(), len, M + (size_t)j0 * mr, mr, mr, len, pw, -1.0, 1.0, st);
     }
     return launches;
 }

@@ -1,4 +1,4 @@
-// largeport.cpp -- CPU backend of enl_large::LargeOps for the single-index family.
+// largeport.cpp -- CPU backend of enl_large::LargeOps and HostPoint for the single-index family.
 //
 // TEST INFRASTRUCTURE / CPU BASELINE ONLY (same role as hostport.cpp for the batched core):
 //   (1) checks the large-regime ENLSIP driver (enlsip.jl_b200/csrc/enl_large_host.h) against the
@@ -24,7 +24,7 @@ namespace {
 typedef void (*allgather_fn)(const double* send, double* recv, long long count);   // recv: world * count
 typedef void (*allreduce_fn)(double* buf, int count);                              // in-place sum
 
-struct CpuOps : LargeOps {
+struct CpuOps : LargeOps, HostPoint {
     const double* W;    // rows x n row major (this shard's rows)
     const double* y;
     long long rows = 0;  // rows held here (== m when not sharded)
@@ -190,7 +190,8 @@ extern "C" int largeport_solve_sharded(int n, long long m, long long rows, int w
     LargeOptions opt;
     opt.max_iter = max_iter; opt.scaling = scaling;
     opt.eps_rel = rel_tol; opt.eps_x = x_tol; opt.eps_c = c_tol;
-    LargeSolver S(ops, opt);
+    HostSmall small(ops, ops.n, ops.l);
+    LargeSolver S(ops, opt, small);
     LargeResult R = S.solve(x0, trace != nullptr);
     std::memcpy(x, R.x.data(), sizeof(double) * n);
     *f = R.f; *exit_code = R.exit_code; *status = R.status; *iters = R.iterations; *nact = R.nact;
